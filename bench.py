@@ -10,6 +10,7 @@ to step).  `value` is whole-job channel-samples/s with the float32 I/Q planes al
 wire format), copies inside the timed region.
 
   python bench.py [--gpus N --steps K --warmup W]          our CUDA path
+  python bench.py ... --dump-outputs DIR                    also save the audio of each workload's last timed step (DIR/config<N>.npy)
   python bench.py --impl reference ...                      the reference's own CPU update() on all host cores
 Under torchrun every rank drives its own GPU and its own 4 096 channels (weak scaling); there is no data-path
 collective, NCCL only reduces the counters (samples, elapsed time, parity error, status counters).
@@ -55,6 +56,8 @@ WORKLOADS = {
 }
 BYTES_PER_SAMPLE = 12.0     # SURVEY 8d: 8 B in (f32 I + f32 Q) + 4 B out per channel-sample
 HBM_FALLBACK_GBS = 6650.0
+DUMP_BYTES = 32 << 20       # --dump-outputs: the headline step's audio is 512 MB, a fixed sample of its rows is kept
+DUMP_BYTES_SIDE = 8 << 20   # the same for each of configs 3, 4 and 5: 56 MB in all
 
 
 def shard_range(total, rank, world):
@@ -425,6 +428,18 @@ class Workload:
         return dict(value=cnt["samples"] / (cnt["max_ms"] * 1e-3) / 1e6, ms_per_step=cnt["max_ms"] / steps, per_launch_ms=per,
                     launches=int(self.b.launch_count - l0), samples=cnt["samples"])
 
+    def dump(self, path, budget):
+        """The audio plane of the last step, as a caller of process() receives it, saved as path/config<N>.npy (float32
+        [rows, samples]): the same seeded sample of channel rows in every run, at most `budget` bytes, so that two builds can
+        be compared output for output."""
+        import torch
+        n = min(self.nch, max(1, budget // (4 * self.ns)))
+        rows = np.sort(np.random.default_rng(0).choice(self.nch, n, replace=False))
+        torch.cuda.synchronize()
+        audio = self.out[torch.from_numpy(rows).to(self.dev), :budget // (4 * n)].cpu().numpy()
+        os.makedirs(path, exist_ok=True)
+        np.save(os.path.join(path, "config%d.npy" % self.cfg_id), audio)
+
     def free(self):
         import torch
         del self.b, self.I16, self.Q16, self.If, self.Qf, self.out
@@ -435,8 +450,10 @@ def side_workload(cfg_id, args, rank, world, local, dev, barrier, peaks32):
     """One of the non-headline BASELINE configurations: device-resident rate, FP32 roofline with its own flop count, parity."""
     w = Workload(cfg_id, rank, world, local, dev)
     parity, status = w.warm_up(3)
-    steps = max(3, min(args.steps, 5))
+    steps = args.steps
     t = w.timed(steps, barrier)
+    if args.dump_outputs and rank == 0:
+        w.dump(args.dump_outputs, DUMP_BYTES_SIDE)
     launch_s = float(np.mean(t["per_launch_ms"])) * 1e-3
     rec = dict(workload=WORKLOADS[cfg_id]["name"], metric=METRIC, unit=UNIT, value=t["value"], n_gpus=world, scaling=WORKLOADS[cfg_id]["scaling"],
                channels_this_rank=w.nch, blocks_per_step=w.nblk, steps=steps, warmup=3, ms_per_step=t["ms_per_step"], gpu_launches=t["launches"],
@@ -464,7 +481,14 @@ def main():
     ap.add_argument("--variant", default="", help="diagnostics only: comma list of nonb,noagc,noaud,als (changes the workload!)")
     ap.add_argument("--role-profile", action="store_true", help="per-stage busy fractions (adds clock reads; not for headline numbers)")
     ap.add_argument("--contract", action="store_true", help="diagnostics only: the opt-in contracting build (not bit-exact) as the line's workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="save the audio of each workload's last timed step as DIR/config<N>.npy "
+                                                            "(float32, a fixed sample of channel rows: at most 32 MB for the "
+                                                            "line's workload, 8 MB for each of configs 3-5; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs saves what the CUDA path computed: it needs --impl ours")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
         run_reference(args, rank, world)
@@ -501,6 +525,8 @@ def main():
     clk = ClockSampler(local); clk.start()
     T = W.timed(args.steps, barrier)
     clocks = clk.stop()
+    if args.dump_outputs and rank == 0:
+        W.dump(args.dump_outputs, DUMP_BYTES)  # before the sustained and e2e runs below advance the same handle
     launches, per_launch_ms, value = T["launches"], T["per_launch_ms"], T["value"]
     role_profile = b.role_profile() if args.role_profile else None  # before the chunked e2e launches dilute the per-launch average
 
@@ -632,7 +658,8 @@ def main():
     if rank == 0 and world == 1 and not diagnostic and not args.only_headline and not args.no_aux:
         aux_blocks = {}
         try:
-            r = subprocess.run([sys.executable, os.path.join(ROOT, "bench_aux.py"), "--no-cpu-baseline", "--steps", "5", "--warmup", "3", "--e2e-steps", "1"],
+            r = subprocess.run([sys.executable, os.path.join(ROOT, "bench_aux.py"), "--no-cpu-baseline", "--steps", str(args.steps),
+                                "--warmup", str(args.warmup), "--e2e-steps", "1"],
                                capture_output=True, text=True, timeout=240)
             for ln in r.stdout.splitlines():
                 if not ln.startswith("{"):
