@@ -8,9 +8,10 @@ tier can import the package), but constructing an SdrBatch raises unless libsdr_
 CUDA device accepts the sm_100a kernel image.  There is no CPU fallback.
 """
 from .api import (AGC_FAST, AGC_MEDIUM, AGC_OFF, AGC_SLOW, AM, AUDIO_2100, AUDIO_2300, AUDIO_2500, AUDIO_2700,
-                  AUDIO_2900, AUDIO_3100, AUDIO_3300, AUDIO_AM, AUDIO_BYPASS, AUDIO_CW, AUDIO_WSPR, CW_LSB, CW_USB,
-                  FMT_F32, FMT_I16, LSB, SAM, SETTERS, USB, WSPR, ChannelStatus, SdrBatch, SdrError, lib_path,
-                  load_library)
+                  AUDIO_2900, AUDIO_3100, AUDIO_3300, AUDIO_AM, AUDIO_BYPASS, AUDIO_CW, AUDIO_WSPR, BS_AGC_ACTIVE,
+                  BS_AGC_GAIN, BS_AM_CARRIER, BS_FIELDS, BS_NAMES, BS_NB_AVERAGE, BS_NB_DETECTED, BS_SAM_FREQUENCY,
+                  BS_SAM_LOCKED, CW_LSB, CW_USB, FMT_F32, FMT_I16, LSB, SAM, SETTERS, USB, WSPR, ChannelStatus, SdrBatch,
+                  SdrError, block_status_fields, lib_path, load_library)
 from .aux import AuxError, GrabberBatch, IQGeneratorBatch, PreProcessorBatch
 from .build import build_aux_library, build_library
 

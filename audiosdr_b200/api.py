@@ -30,7 +30,26 @@ EXPORTS = ["sdr_batch_create", "sdr_batch_destroy", "sdr_batch_set", "sdr_batch_
            "sdr_batch_process_host", "sdr_batch_get_status", "sdr_batch_get_agc_lookup", "sdr_batch_peek_state",
            "sdr_batch_get_role_profile", "sdr_batch_launch_count", "sdr_batch_last_error", "sdr_batch_version",
            "sdr_batch_process", "sdr_batch_state_bytes", "sdr_batch_export_state", "sdr_batch_import_state",
-           "sdr_batch_submit_host", "sdr_batch_wait_host", "sdr_batch_host_ticket", "sdr_batch_wait_host_ticket"]
+           "sdr_batch_submit_host", "sdr_batch_wait_host", "sdr_batch_host_ticket", "sdr_batch_wait_host_ticket",
+           "sdr_batch_process_device_status", "sdr_batch_process_host_status", "sdr_batch_submit_host_status"]
+
+# per-block status records (include/sdr_batch.h, SDR_BS_*): array [n_blocks, BS_FIELDS, n_channels] of 32-bit words
+(BS_AGC_GAIN, BS_AGC_ACTIVE, BS_AM_CARRIER, BS_SAM_FREQUENCY, BS_SAM_LOCKED, BS_NB_AVERAGE, BS_NB_DETECTED,
+ BS_FIELDS) = range(8)
+BS_NAMES = ["agc_gain", "agc_active", "am_carrier", "sam_frequency", "sam_locked", "nb_average", "nb_detected"]
+_BS_FLAGS = (BS_AGC_ACTIVE, BS_SAM_LOCKED, BS_NB_DETECTED)
+
+
+def block_status_fields(records):
+    """Named views of a per-block status record array [n_blocks, BS_FIELDS, n_channels] (numpy, any 4-byte dtype, or a torch
+    tensor, which is copied to the host): {name: [n_blocks, n_channels]}, float32 for the levels, bool for the three flags
+    (AGCisActive, getSAMphaseLockStatus, NoiseBlankerDetection)."""
+    if hasattr(records, "detach"):
+        records = records.detach().cpu().numpy()
+    r = np.asarray(records)
+    assert r.ndim == 3 and r.shape[1] == BS_FIELDS and r.dtype.itemsize == 4, "expected [n_blocks, %d, n_channels] 32-bit words" % BS_FIELDS
+    return {name: (r[:, f, :].view(np.uint32) != 0) if f in _BS_FLAGS else r[:, f, :].view(np.float32)
+            for f, name in enumerate(BS_NAMES)}
 
 
 class SdrError(RuntimeError):
@@ -88,6 +107,10 @@ def _bind(L):
     L.sdr_batch_launch_count.restype = C.c_uint64
     L.sdr_batch_last_error.restype = C.c_char_p
     L.sdr_batch_version.restype = C.c_char_p
+    if hasattr(L, "sdr_batch_process_device_status"):  # (a build older than the per-block records binds without them)
+        L.sdr_batch_process_device_status.argtypes = L.sdr_batch_process_device.argtypes[:-1] + [C.c_void_p, C.c_void_p]
+        L.sdr_batch_process_host_status.argtypes = L.sdr_batch_process_host.argtypes + [C.c_void_p]
+        L.sdr_batch_submit_host_status.argtypes = L.sdr_batch_process_host_status.argtypes
     return L
 
 
@@ -257,39 +280,68 @@ class SdrBatch:
         return int(self.L.sdr_batch_launch_count(self.h))
 
     # ---- hot path
-    def process(self, I, Q, audio, n_blocks=None, stream=None):
-        """Device tensors (torch, CUDA, 2-D [n_channels, >= 128*n_blocks], contiguous rows); asynchronous."""
+    def _records(self, block_status, n_blocks, on_device):
+        """Address of a per-block status record buffer (None: no records): [n_blocks, BS_FIELDS, n_channels], 4-byte
+        elements, contiguous; a CUDA tensor for process(), a numpy array for the host paths."""
+        if block_status is None:
+            return None
+        want = (n_blocks, BS_FIELDS, self.n_channels)
+        if on_device:
+            assert block_status.is_cuda and block_status.is_contiguous() and block_status.element_size() == 4, \
+                "block_status: a contiguous CUDA tensor of 4-byte elements"
+            assert tuple(block_status.shape) == want, "block_status: shape %r, want %r" % (tuple(block_status.shape), want)
+            return block_status.data_ptr()
+        assert isinstance(block_status, np.ndarray) and block_status.flags.c_contiguous and block_status.itemsize == 4, \
+            "block_status: a C-contiguous numpy array of 4-byte elements"
+        assert block_status.shape == want, "block_status: shape %r, want %r" % (block_status.shape, want)
+        return block_status.ctypes.data
+
+    def process(self, I, Q, audio, n_blocks=None, stream=None, block_status=None):
+        """Device tensors (torch, CUDA, 2-D [n_channels, >= 128*n_blocks], contiguous rows); asynchronous.  `block_status`:
+        optional CUDA tensor [n_blocks, BS_FIELDS, n_channels] (4-byte dtype) that receives the getters after every block
+        (block_status_fields() names them), on the same stream as the audio."""
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
         assert I.shape[0] == self.n_channels and Q.shape == I.shape and audio.shape[0] == self.n_channels
         assert I.stride(1) == 1 and Q.stride(1) == 1 and audio.stride(1) == 1 and I.stride(0) == Q.stride(0)
         sp = C.c_void_p(stream.cuda_stream) if stream is not None else None
-        self._check(self.L.sdr_batch_process_device(self.h, I.data_ptr(), Q.data_ptr(), I.stride(0), _fmt_of(str(I.dtype)),
-                                                    audio.data_ptr(), audio.stride(0), _fmt_of(str(audio.dtype)),
-                                                    n_blocks, sp))
+        args = (self.h, I.data_ptr(), Q.data_ptr(), I.stride(0), _fmt_of(str(I.dtype)), audio.data_ptr(), audio.stride(0),
+                _fmt_of(str(audio.dtype)), n_blocks)
+        if block_status is None:
+            self._check(self.L.sdr_batch_process_device(*args, sp))
+        else:
+            self._check(self.L.sdr_batch_process_device_status(*args, self._records(block_status, n_blocks, True), sp))
 
-    def process_host(self, I, Q, audio=None, out_fmt=FMT_F32, n_blocks=None):
-        """Host numpy arrays [n_channels, S]; copies in, runs, copies out; returns the audio array."""
+    def process_host(self, I, Q, audio=None, out_fmt=FMT_F32, n_blocks=None, block_status=None):
+        """Host numpy arrays [n_channels, S]; copies in, runs, copies out; returns the audio array.  `block_status`: optional
+        numpy array [n_blocks, BS_FIELDS, n_channels] (4-byte dtype) that receives the getters after every block."""
         I = np.ascontiguousarray(I)
         Q = np.ascontiguousarray(Q)
         assert I.shape == Q.shape and I.dtype == Q.dtype and I.shape[0] == self.n_channels
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
         if audio is None:
             audio = np.empty((self.n_channels, n_blocks * N_BLOCK), np.float32 if out_fmt == FMT_F32 else np.int16)
-        self._check(self.L.sdr_batch_process_host(self.h, I.ctypes.data, Q.ctypes.data, I.strides[0] // I.itemsize,
-                                                  _fmt_of(str(I.dtype)), audio.ctypes.data,
-                                                  audio.strides[0] // audio.itemsize, _fmt_of(str(audio.dtype)), n_blocks))
+        args = (self.h, I.ctypes.data, Q.ctypes.data, I.strides[0] // I.itemsize, _fmt_of(str(I.dtype)), audio.ctypes.data,
+                audio.strides[0] // audio.itemsize, _fmt_of(str(audio.dtype)), n_blocks)
+        if block_status is None:
+            self._check(self.L.sdr_batch_process_host(*args))
+        else:
+            self._check(self.L.sdr_batch_process_host_status(*args, self._records(block_status, n_blocks, False)))
         return audio
 
-    def submit_host(self, I, Q, audio, n_blocks=None):
+    def submit_host(self, I, Q, audio, n_blocks=None, block_status=None):
         """Streaming form of process_host: queues the call and returns; `wait_host()` completes everything queued.  The arrays
         must be C-contiguous rows (they are used in place: no copy is made) and should be pinned; I, Q must stay unchanged
-        and `audio` unread until wait_host() returns."""
+        and `audio` (and `block_status`, the optional per-block records as in process_host) unread until wait_host() -- or
+        wait_host(ticket) with the ticket this returns -- has returned."""
         assert I.shape == Q.shape and I.dtype == Q.dtype and I.shape[0] == self.n_channels and audio.shape[0] == self.n_channels
         assert I.strides[1] == I.itemsize and Q.strides == I.strides and audio.strides[1] == audio.itemsize
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
-        self._check(self.L.sdr_batch_submit_host(self.h, I.ctypes.data, Q.ctypes.data, I.strides[0] // I.itemsize,
-                                                 _fmt_of(str(I.dtype)), audio.ctypes.data,
-                                                 audio.strides[0] // audio.itemsize, _fmt_of(str(audio.dtype)), n_blocks))
+        args = (self.h, I.ctypes.data, Q.ctypes.data, I.strides[0] // I.itemsize, _fmt_of(str(I.dtype)), audio.ctypes.data,
+                audio.strides[0] // audio.itemsize, _fmt_of(str(audio.dtype)), n_blocks)
+        if block_status is None:
+            self._check(self.L.sdr_batch_submit_host(*args))
+        else:
+            self._check(self.L.sdr_batch_submit_host_status(*args, self._records(block_status, n_blocks, False)))
         return int(self.L.sdr_batch_host_ticket(self.h))
 
     def wait_host(self, ticket=None):

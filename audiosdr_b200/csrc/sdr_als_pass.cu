@@ -20,7 +20,7 @@ using namespace SDR_NS;
 extern "C" __global__ void __launch_bounds__(32, 8) sdr_als_pass_kernel(const __grid_constant__ SdrLaunch L) {
   extern __shared__ __align__(16) unsigned char smem[];
   Ctx x;
-  x.L = &L; x.Y = &L.lay; x.G = &L.groups[blockIdx.x]; x.smem = smem; x.gidx = (int)blockIdx.x; x.prof = false; x.t0 = 0;
+  x.L = &L; x.Y = &L.lay; x.G = &L.groups[blockIdx.x]; x.smem = smem; x.gidx = (int)blockIdx.x; x.prof = false; x.rec = false; x.t0 = 0;
   const int lane = (int)threadIdx.x;
   reinterpret_cast<int *>(smem + x.o_cid())[lane] = x.G->cid[lane];
   x.k.reset();

@@ -167,6 +167,7 @@ struct sdr_batch {
   /* host-buffer path: two staging sets and three streams so that the H2D copy of chunk k+1, the kernel of chunk k and
    * the D2H copy of chunk k-1 overlap */
   void *d_in_i[2], *d_in_q[2], *d_out[2]; size_t stage_in_bytes, stage_out_bytes;
+  void *d_bs[2]; size_t stage_bs_bytes; /* per-block status records of a chunk, beside d_out (allocated by the first call that asks for records) */
   void *s_h2d, *s_comp, *s_d2h; void *ev_h2d[2], *ev_comp[2], *ev_d2h[2];
   uint64_t host_seq; /* chunks queued by submit_host since create: chunk n uses staging set n & 1 */
   uint64_t host_calls; void *ev_call[SDR_HOST_TICKETS]; /* host calls queued since create (= the ticket of the latest); call t's last copy-out records ev_call[t % SDR_HOST_TICKETS] */
@@ -608,7 +609,7 @@ void sdr_batch_destroy(sdr_batch_t *h) {
   dev_free(h->d_state); dev_free(h->d_cfg); dev_free(h->d_groups); dev_free(h->d_luts); dev_free(h->d_tabs);
   dev_free(h->d_reset_ch); dev_free(h->d_reset_mask); dev_free(h->d_gather); dev_free(h->d_gather_ids); dev_free(h->d_gather_words);
   for (int k = 0; k < 2; k++) {
-    dev_free(h->d_in_i[k]); dev_free(h->d_in_q[k]); dev_free(h->d_out[k]);
+    dev_free(h->d_in_i[k]); dev_free(h->d_in_q[k]); dev_free(h->d_out[k]); dev_free(h->d_bs[k]);
     dev_event_destroy(h->ev_h2d[k]); dev_event_destroy(h->ev_comp[k]); dev_event_destroy(h->ev_d2h[k]);
   }
   dev_stream_destroy(h->s_h2d); dev_stream_destroy(h->s_comp); dev_stream_destroy(h->s_d2h);
@@ -632,8 +633,8 @@ int sdr_batch_create(sdr_batch_t **out, const sdr_batch_desc *desc) {
   h->d_state = nullptr; h->d_cfg = nullptr; h->d_groups = nullptr; h->d_luts = nullptr; h->d_tabs = nullptr;
   h->d_reset_ch = h->d_reset_mask = nullptr; h->reset_cap = h->luts_cap = h->groups_cap = 0;
   h->d_gather = nullptr; h->d_gather_ids = h->d_gather_words = nullptr; h->gather_cap = 0;
-  for (int k = 0; k < 2; k++) { h->d_in_i[k] = h->d_in_q[k] = h->d_out[k] = nullptr; h->ev_h2d[k] = h->ev_comp[k] = h->ev_d2h[k] = nullptr; }
-  h->s_h2d = h->s_comp = h->s_d2h = nullptr; h->stage_in_bytes = h->stage_out_bytes = 0; h->host_seq = 0;
+  for (int k = 0; k < 2; k++) { h->d_in_i[k] = h->d_in_q[k] = h->d_out[k] = h->d_bs[k] = nullptr; h->ev_h2d[k] = h->ev_comp[k] = h->ev_d2h[k] = nullptr; }
+  h->s_h2d = h->s_comp = h->s_d2h = nullptr; h->stage_in_bytes = h->stage_out_bytes = h->stage_bs_bytes = 0; h->host_seq = 0;
   h->host_calls = 0; for (int k = 0; k < SDR_HOST_TICKETS; k++) h->ev_call[k] = nullptr;
   h->n_groups = 0; h->blocks_done = 0; h->launches = 0; h->last_stream = nullptr;
   h->d_prof = nullptr; h->prof_cap = 0; h->prof_launches = 0;
@@ -703,8 +704,14 @@ int sdr_batch_configure(sdr_batch_t *h, const sdr_setter_call *calls, uint32_t n
 
 int sdr_batch_process_device(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
                              size_t out_pitch, int out_fmt, uint32_t n_blocks, void *stream) {
+  return sdr_batch_process_device_status(h, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, nullptr, stream);
+}
+
+int sdr_batch_process_device_status(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
+                                    size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status, void *stream) {
   if (!h) return fail(SDR_ERR_ARG, "null handle");
   if (n_blocks == 0) return fail(SDR_ERR_ARG, "n_blocks == 0");
+  if ((uintptr_t)block_status % 16 != 0) return fail(SDR_ERR_ARG, "block_status: the record buffer must be 16-byte aligned");
   if (h->desc.max_blocks_per_call && n_blocks > h->desc.max_blocks_per_call) return fail(SDR_ERR_ARG, "n_blocks > max_blocks_per_call");
   if (n_blocks > (1u << 24)) return fail(SDR_ERR_ARG, "n_blocks too large (at most 2^24 blocks per call)");
   int rc;
@@ -723,6 +730,7 @@ int sdr_batch_process_device(sdr_batch_t *h, const void *I, const void *Q, size_
   L.blk0_mod3 = (uint32_t)(h->blocks_done % 3);
   L.flags = h->desc.flags & SDR_BATCH_CONTRACT;
   L.cfg = h->d_cfg; L.state = h->d_state; L.ch_stride = h->ch_stride; L.agc_luts = h->d_luts; L.tabs = h->d_tabs;
+  L.bstat = (uint32_t *)block_status; L.bs_stride = h->n_ch; /* every bucket writes the records of its own channels */
   if (h->prof_on) {
     size_t need = (size_t)std::max<uint32_t>(h->n_groups, 1) * SDR_PROF_SLOTS * 8;
     if (need > h->prof_cap) {
@@ -783,6 +791,8 @@ int sdr_batch_process_device(sdr_batch_t *h, const void *I, const void *Q, size_
         M.blk0_mod3 = (uint32_t)((h->blocks_done + b0) % 3);
         M.raw = h->d_raw[k];
         SdrLaunch A = M;
+        A.bstat = nullptr; /* the records come from the chain launch (its AGC stage), the post-pass writes none */
+        if (M.bstat) M.bstat += (size_t)b0 * SDR_BS_FIELDS * h->n_ch;
         M.lay = b.lay_main; M.n_tiles = nb * (uint32_t)b.lay_main.tpb; M.flags |= SDRL_RAW_OUT;
         A.lay = b.lay_als; A.n_tiles = nb * (uint32_t)b.lay_als.tpb;
         A.lay.smem_bytes += env_int("SDR_ALS_PASS_PAD", 0); /* experiment: fewer groups per SM in the post-pass */
@@ -830,24 +840,35 @@ int sdr_batch_wait_host_ticket(sdr_batch_t *h, uint64_t ticket) {
 }
 
 static int host_call(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt,
-                     uint32_t n_blocks, bool streamed);
+                     uint32_t n_blocks, void *block_status, bool streamed);
 
 int sdr_batch_process_host(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
                            size_t out_pitch, int out_fmt, uint32_t n_blocks) {
-  const int rc = host_call(h, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, false);
+  return sdr_batch_process_host_status(h, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, nullptr);
+}
+
+int sdr_batch_process_host_status(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
+                                  size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status) {
+  const int rc = host_call(h, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status, false);
   if (rc) return rc; /* (the streams have been drained) */
   return sdr_batch_wait_host(h);
 }
 
 int sdr_batch_submit_host(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
                           size_t out_pitch, int out_fmt, uint32_t n_blocks) {
-  return host_call(h, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, true);
+  return sdr_batch_submit_host_status(h, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, nullptr);
+}
+
+int sdr_batch_submit_host_status(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
+                                 size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status) {
+  return host_call(h, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status, true);
 }
 
 static int host_call(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt,
-                     uint32_t n_blocks, bool streamed) {
+                     uint32_t n_blocks, void *block_status, bool streamed) {
   if (!h || !I || !Q || !audio) return fail(SDR_ERR_ARG, "process_host: bad arguments");
   if (n_blocks == 0) return fail(SDR_ERR_ARG, "n_blocks == 0");
+  if ((uintptr_t)block_status % 16 != 0) return fail(SDR_ERR_ARG, "block_status: the record buffer must be 16-byte aligned");
   if (in_fmt != SDR_FMT_I16 && in_fmt != SDR_FMT_F32) return fail(SDR_ERR_ARG, "process_host: unknown input format");
   if (out_fmt != SDR_FMT_I16 && out_fmt != SDR_FMT_F32) return fail(SDR_ERR_ARG, "process_host: unknown output format");
   const size_t ns = (size_t)n_blocks * SDR_BLOCK_SAMPLES;
@@ -875,12 +896,18 @@ static int host_call(sdr_batch_t *h, const void *I, const void *Q, size_t in_pit
       if (dev_event_create(&h->ev_h2d[k]) || dev_event_create(&h->ev_comp[k]) || dev_event_create(&h->ev_d2h[k])) return SDR_ERR_CUDA;
     for (int k = 0; k < SDR_HOST_TICKETS; k++) if (dev_event_create(&h->ev_call[k])) return SDR_ERR_CUDA;
   }
-  if (in_bytes > h->stage_in_bytes || out_bytes > h->stage_out_bytes) {
+  const size_t bs_bytes = block_status ? (size_t)chunk * SDR_BS_FIELDS * h->n_ch * 4 : 0;
+  if (in_bytes > h->stage_in_bytes || out_bytes > h->stage_out_bytes || bs_bytes > h->stage_bs_bytes) {
     dev_sync(h->last_stream); dev_sync(h->s_h2d); dev_sync(h->s_comp); dev_sync(h->s_d2h);
-    const bool grow_in = in_bytes > h->stage_in_bytes, grow_out = out_bytes > h->stage_out_bytes;
+    const bool grow_in = in_bytes > h->stage_in_bytes, grow_out = out_bytes > h->stage_out_bytes, grow_bs = bs_bytes > h->stage_bs_bytes;
     if (grow_in) h->stage_in_bytes = 0; /* (an allocation that fails below leaves no stale size behind: the next call allocates again) */
     if (grow_out) h->stage_out_bytes = 0;
+    if (grow_bs) h->stage_bs_bytes = 0;
     for (int k = 0; k < 2; k++) {
+      if (grow_bs) {
+        dev_free(h->d_bs[k]); h->d_bs[k] = nullptr;
+        if (dev_alloc(&h->d_bs[k], bs_bytes)) return SDR_ERR_NOMEM;
+      }
       if (grow_in) {
         dev_free(h->d_in_i[k]); dev_free(h->d_in_q[k]); h->d_in_i[k] = h->d_in_q[k] = nullptr;
         if (dev_alloc(&h->d_in_i[k], in_bytes) || dev_alloc(&h->d_in_q[k], in_bytes)) return SDR_ERR_NOMEM;
@@ -892,6 +919,7 @@ static int host_call(sdr_batch_t *h, const void *I, const void *Q, size_t in_pit
     }
     if (grow_in) h->stage_in_bytes = in_bytes;
     if (grow_out) h->stage_out_bytes = out_bytes;
+    if (grow_bs) h->stage_bs_bytes = bs_bytes;
   }
   /* work queued by an earlier process_device call on another stream must finish before the state is touched here */
   if (h->last_stream != h->s_comp && dev_sync(h->last_stream)) return SDR_ERR_CUDA;
@@ -929,12 +957,17 @@ static int host_call(sdr_batch_t *h, const void *I, const void *Q, size_t in_pit
     /* kernel of chunk k: needs its input, and the D2H of chunk k-2 must have drained output set b */
     SDR_TRY(dev_stream_wait(h->s_comp, h->ev_h2d[b]) ? SDR_ERR_CUDA : 0);
     if (h->host_seq >= 2) { SDR_TRY(dev_stream_wait(h->s_comp, h->ev_d2h[b]) ? SDR_ERR_CUDA : 0); }
-    int rc = sdr_batch_process_device(h, h->d_in_i[b], h->d_in_q[b], cs, in_fmt, h->d_out[b], cs, out_fmt, nb, h->s_comp);
+    int rc = sdr_batch_process_device_status(h, h->d_in_i[b], h->d_in_q[b], cs, in_fmt, h->d_out[b], cs, out_fmt, nb,
+                                             block_status ? h->d_bs[b] : nullptr, h->s_comp);
     SDR_TRY(rc);
     SDR_TRY(dev_event_record(h->ev_comp[b], h->s_comp) ? SDR_ERR_CUDA : 0);
-    /* D2H of chunk k */
+    /* D2H of chunk k: audio, then its records (block-major: the chunk's blocks are one contiguous range of the caller's buffer) */
     SDR_TRY(dev_stream_wait(h->s_d2h, h->ev_comp[b]) ? SDR_ERR_CUDA : 0);
     SDR_TRY(d2h_2d(dst, out_pitch * oes, h->d_out[b], cs * oes, w_out, h->n_ch, h->s_d2h) ? SDR_ERR_CUDA : 0);
+    if (block_status) {
+      const size_t rec = (size_t)SDR_BS_FIELDS * h->n_ch; /* words per block */
+      SDR_TRY(d2h((uint32_t *)block_status + (size_t)done * rec, h->d_bs[b], (size_t)nb * rec * 4, h->s_d2h) ? SDR_ERR_CUDA : 0);
+    }
     SDR_TRY(dev_event_record(h->ev_d2h[b], h->s_d2h) ? SDR_ERR_CUDA : 0);
     done += nb; k++; h->host_seq++;
   }

@@ -258,7 +258,7 @@ __device__ __forceinline__ void run_stage(const Ctx &x, int stage, int lane) {
   }
 }
 
-template <bool PROF>
+template <bool PROF, bool REC>
 __device__ __forceinline__ void pipeline_cta(const SdrLaunch &L, unsigned char *smem) {
   Ctx x;
   x.L = &L;
@@ -267,6 +267,7 @@ __device__ __forceinline__ void pipeline_cta(const SdrLaunch &L, unsigned char *
   x.smem = smem;
   x.gidx = (int)blockIdx.x;
   x.prof = PROF;
+  x.rec = REC;
   x.t0 = PROF ? clock64() : 0;
   const int nthr = (int)blockDim.x;
   for (int i = threadIdx.x; i < 257; i += nthr) x.f(x.o_sine())[i] = L.tabs->sine[i];
@@ -295,18 +296,23 @@ __device__ __forceinline__ void pipeline_cta(const SdrLaunch &L, unsigned char *
   run_stage(x, (int)x.Y->stage_of_warp[phys], lane);
 }
 
-/* The product kernel and its diagnostics twin (per-stage busy / waiting counters, sub-phase timers, stage skipping): the
- * twin is launched only when the handle was created with SDR_ROLE_PROFILE=1.  Keeping the counters out of the product
- * kernel is not cosmetic: its stages are different instruction streams whose loops must share the instruction caches. */
+/* The product kernel, its twin that also writes per-block status records (launched when SdrLaunch::bstat is set), and the
+ * diagnostics twin (per-stage busy / waiting counters, sub-phase timers, stage skipping; no records), launched only when the
+ * handle was created with SDR_ROLE_PROFILE=1.  Keeping the counters and the record stores out of the product kernel is not
+ * cosmetic: its stages are different instruction streams whose loops must share the instruction caches. */
 /* register budget: the 32-sample plans run up to 14 warps, one CTA per SM; the shorter tiles exist for plans of at most 11
  * warps that share an SM two at a time (SDR_LB_THREADS / SDR_LB_BLOCKS are set by the sdr_pipe_t*.cu files) */
 extern "C" __global__ void __launch_bounds__(SDR_LB_THREADS, SDR_LB_BLOCKS) SDR_SYM(sdr_pipeline_kernel)(const __grid_constant__ SdrLaunch L) {
   extern __shared__ __align__(16) unsigned char smem[];
-  pipeline_cta<false>(L, smem);
+  pipeline_cta<false, false>(L, smem);
+}
+extern "C" __global__ void __launch_bounds__(SDR_LB_THREADS, SDR_LB_BLOCKS) SDR_SYM(sdr_pipeline_rec_kernel)(const __grid_constant__ SdrLaunch L) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  pipeline_cta<false, true>(L, smem);
 }
 extern "C" __global__ void __launch_bounds__(SDR_LB_THREADS, 1) SDR_SYM(sdr_pipeline_prof_kernel)(const __grid_constant__ SdrLaunch L) {
   extern __shared__ __align__(16) unsigned char smem[];
-  pipeline_cta<true>(L, smem);
+  pipeline_cta<true, false>(L, smem);
 }
 
 extern "C" int SDR_SYM(sdrk_setup_pipe)(const float *hilbert64) {
@@ -316,10 +322,14 @@ extern "C" int SDR_SYM(sdrk_setup_pipe)(const float *hilbert64) {
   if (e != cudaSuccess) return (int)e;
   e = cudaFuncSetAttribute(SDR_SYM(sdr_pipeline_kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
   if (e != cudaSuccess) return (int)e;
+  e = cudaFuncSetAttribute(SDR_SYM(sdr_pipeline_rec_kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+  if (e != cudaSuccess) return (int)e;
   e = cudaFuncSetAttribute(SDR_SYM(sdr_pipeline_prof_kernel), cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
   if (e != cudaSuccess) return (int)e;
   /* launches that need less than half of an SM's shared memory are meant to share the SM: keep the carve-out at its maximum */
   e = cudaFuncSetAttribute(SDR_SYM(sdr_pipeline_kernel), cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
+  if (e != cudaSuccess) return (int)e;
+  e = cudaFuncSetAttribute(SDR_SYM(sdr_pipeline_rec_kernel), cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
   if (e != cudaSuccess) return (int)e;
   e = cudaFuncSetAttribute(SDR_SYM(sdr_pipeline_prof_kernel), cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
   return (int)e;
@@ -328,6 +338,7 @@ extern "C" int SDR_SYM(sdrk_setup_pipe)(const float *hilbert64) {
 extern "C" int SDR_SYM(sdrk_launch_pipe)(const SdrLaunch *L, void *stream) {
   const int threads = L->lay.n_warps * 32, smem = L->lay.smem_bytes;
   if (L->prof) SDR_SYM(sdr_pipeline_prof_kernel)<<<L->n_groups, threads, smem, (cudaStream_t)stream>>>(*L);
+  else if (L->bstat) SDR_SYM(sdr_pipeline_rec_kernel)<<<L->n_groups, threads, smem, (cudaStream_t)stream>>>(*L);
   else SDR_SYM(sdr_pipeline_kernel)<<<L->n_groups, threads, smem, (cudaStream_t)stream>>>(*L);
   return (int)cudaGetLastError();
 }

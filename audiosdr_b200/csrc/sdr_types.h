@@ -149,6 +149,10 @@ typedef struct {
                             SDRL_RAW_OUT launch, read by the ALS post-pass (sdr_als_pass.cu) */
   uint32_t diag_skip;    /* diagnostics (profiling runs only): bit s set = stage s idles; results are then meaningless */
   unsigned long long *prof; /* optional [n_groups][SDR_PROF_SLOTS] (diagnostics twin): busy and waiting cycles per stage */
+  uint32_t *bstat;       /* optional per-block status records of the launch's blocks (include/sdr_batch.h, SDR_BS_*): word
+                            ((block * SDR_BS_FIELDS + field) * bs_stride + channel); null = no records.  Written at the end of
+                            each block by the stage that owns the field (sdr_pipeline.cuh, Ctx::bs_put) */
+  unsigned long long bs_stride; /* = the handle's channel count */
   SdrLay lay;
 } SdrLaunch;
 

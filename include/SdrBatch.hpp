@@ -136,6 +136,22 @@ class SdrBatch {
                    uint32_t n_blocks) {
     check(sdr_batch_submit_host(h_, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks), "sdr_batch_submit_host");
   }
+  /* ... each of the three with per-block status records: the dynamic getters after every block of the call, block-major
+   * [n_blocks][SDR_BS_FIELDS][channels] 32-bit words (sdr_batch.h, SDR_BS_*), 16-byte aligned; device memory for process(),
+   * host memory for the host forms (they land with the call's audio).  nullptr = the overload without records. */
+  void process(const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt,
+               uint32_t n_blocks, void *block_status, void *cuda_stream) {
+    check(sdr_batch_process_device_status(h_, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status, cuda_stream),
+          "sdr_batch_process_device_status");
+  }
+  void process_host(const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt,
+                    uint32_t n_blocks, void *block_status) {
+    check(sdr_batch_process_host_status(h_, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status), "sdr_batch_process_host_status");
+  }
+  void submit_host(const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt,
+                   uint32_t n_blocks, void *block_status) {
+    check(sdr_batch_submit_host_status(h_, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status), "sdr_batch_submit_host_status");
+  }
   void wait_host() { check(sdr_batch_wait_host(h_), "sdr_batch_wait_host"); }
   uint64_t host_ticket() const { return sdr_batch_host_ticket(h_); } /* names the call submitted last */
   void wait_host(uint64_t ticket) { check(sdr_batch_wait_host_ticket(h_, ticket), "sdr_batch_wait_host_ticket"); }

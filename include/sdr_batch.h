@@ -14,6 +14,7 @@
  *   sdr_batch_process[_*]   AudioStream::update_all() -> AudioSDR::update()     C:39-168
  *                            (receiveWritable(0/1) C:46-47 = the I/Q planes in; transmit(blockI,0/1) C:164-165 = the audio plane out)
  *   sdr_batch_get_status    the getters                                          C:224-230,255-273,295,371-381,495,507-512,568-600,660-665,752-757
+ *   sdr_batch_*_status      process + the dynamic getters polled after every block (per-block status records, SDR_BS_*)
  *   sdr_batch_destroy       (object lifetime)
  *
  * Data layout: channel-major planes.  Sample t of channel c lives at plane[c*pitch + t]; pitch is
@@ -144,6 +145,22 @@ typedef struct {
   uint8_t pad[2];
 } sdr_channel_status;
 
+/* Per-block status records: the dynamic getters after EVERY block of a process call, as the reference's sketch sees them when
+ * it polls between two update() calls.  One 32-bit word per (block, field, channel), block-major:
+ *     status[((size_t)b * SDR_BS_FIELDS + f) * n_channels + c]      b = block of the call, f = SDR_BS_*, c = channel
+ * so that a run of blocks is one contiguous range.  Record (b, c) is what the getters (and _agc_gain / _nb_AvgMag) hold right
+ * after channel c's update() for block b -- for every channel and every block, also fields whose stage does not run for the
+ * channel (they keep their carried-over value).  The last record of a call equals sdr_batch_get_status after the call.
+ * Flags are uint32 0 / 1, the other fields float32.  The buffer must be 16-byte aligned. */
+enum { SDR_BS_AGC_GAIN = 0,     /* _agc_gain                            float */
+       SDR_BS_AGC_ACTIVE,       /* AGCisActive()            C:510-512   uint32 0/1 */
+       SDR_BS_AM_CARRIER,       /* getAMcarrierLevel()      C:495-497   float */
+       SDR_BS_SAM_FREQUENCY,    /* getSAMfrequency()        C:752-754   float */
+       SDR_BS_SAM_LOCKED,       /* getSAMphaseLockStatus()  C:755-757   uint32 0/1 */
+       SDR_BS_NB_AVERAGE,       /* _nb_AvgMag                           float */
+       SDR_BS_NB_DETECTED,      /* NoiseBlankerDetection()  C:663-665   uint32 0/1 */
+       SDR_BS_FIELDS };
+
 int sdr_batch_create(sdr_batch_t **out, const sdr_batch_desc *desc);
 void sdr_batch_destroy(sdr_batch_t *h);
 
@@ -175,6 +192,17 @@ int sdr_batch_process_host(sdr_batch_t *h, const void *I, const void *Q, size_t 
 int sdr_batch_submit_host(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt,
                           void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks);
 int sdr_batch_wait_host(sdr_batch_t *h);
+/* The three calls above with per-block status records (layout above: n_blocks * SDR_BS_FIELDS * n_channels words).
+ * block_status == NULL makes each identical to the call without records.  _device_status: device memory, asynchronous on
+ * the stream like the audio.  _host_status / submit_host_status: host memory (pinned for asynchronous copies); the
+ * records land together with the call's audio, so wait_host_ticket(n) means the records of call n are there too. */
+int sdr_batch_process_device_status(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt,
+                                    void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status,
+                                    void *cuda_stream);
+int sdr_batch_process_host_status(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt,
+                                  void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status);
+int sdr_batch_submit_host_status(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt,
+                                 void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status);
 /* One call at a time: sdr_batch_host_ticket() right after a submit_host (or process_host) names that call (1, 2, ...);
  * wait_host_ticket returns when that call's audio has landed, while later calls stay in flight -- a receiver that keeps
  * two calls queued drains call n while call n + 1 is being copied in and computed.  Calls complete in order. */
@@ -200,7 +228,7 @@ int sdr_batch_import_state(sdr_batch_t *h, const uint32_t *channel_ids, uint32_t
 
 /* Diagnostics: per-stage busy cycles of the pipeline kernel, summed over groups and launches since create.
  * Only recorded when the environment variable SDR_ROLE_PROFILE=1 was set at create (costs two clock reads per
- * stage per tile).  busy[cls*14 + stage] (14 stages per pipeline class), total[cls] = summed CTA cycles,
+ * stage per tile; the kernel timed in that mode writes no per-block status records).  busy[cls*14 + stage] (14 stages per pipeline class), total[cls] = summed CTA cycles,
  * groups[cls] = CTA launches counted. */
 int sdr_batch_get_role_profile(sdr_batch_t *h, uint64_t *busy28, uint64_t *total2, uint64_t *groups2);
 
