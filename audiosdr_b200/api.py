@@ -31,7 +31,8 @@ EXPORTS = ["sdr_batch_create", "sdr_batch_destroy", "sdr_batch_set", "sdr_batch_
            "sdr_batch_get_role_profile", "sdr_batch_launch_count", "sdr_batch_last_error", "sdr_batch_version",
            "sdr_batch_process", "sdr_batch_state_bytes", "sdr_batch_export_state", "sdr_batch_import_state",
            "sdr_batch_submit_host", "sdr_batch_wait_host", "sdr_batch_host_ticket", "sdr_batch_wait_host_ticket",
-           "sdr_batch_process_device_status", "sdr_batch_process_host_status", "sdr_batch_submit_host_status"]
+           "sdr_batch_process_device_status", "sdr_batch_process_host_status", "sdr_batch_submit_host_status",
+           "sdr_batch_process_device_subset", "sdr_batch_process_host_subset", "sdr_batch_submit_host_subset"]
 
 # per-block status records (include/sdr_batch.h, SDR_BS_*): array [n_blocks, BS_FIELDS, n_channels] of 32-bit words
 (BS_AGC_GAIN, BS_AGC_ACTIVE, BS_AM_CARRIER, BS_SAM_FREQUENCY, BS_SAM_LOCKED, BS_NB_AVERAGE, BS_NB_DETECTED,
@@ -111,6 +112,11 @@ def _bind(L):
         L.sdr_batch_process_device_status.argtypes = L.sdr_batch_process_device.argtypes[:-1] + [C.c_void_p, C.c_void_p]
         L.sdr_batch_process_host_status.argtypes = L.sdr_batch_process_host.argtypes + [C.c_void_p]
         L.sdr_batch_submit_host_status.argtypes = L.sdr_batch_process_host_status.argtypes
+    if hasattr(L, "sdr_batch_process_device_subset"):
+        ids = [C.c_void_p, C.c_uint32]
+        L.sdr_batch_process_device_subset.argtypes = [C.c_void_p] + ids + L.sdr_batch_process_device_status.argtypes[1:]
+        L.sdr_batch_process_host_subset.argtypes = [C.c_void_p] + ids + L.sdr_batch_process_host_status.argtypes[1:]
+        L.sdr_batch_submit_host_subset.argtypes = L.sdr_batch_process_host_subset.argtypes
     return L
 
 
@@ -280,12 +286,20 @@ class SdrBatch:
         return int(self.L.sdr_batch_launch_count(self.h))
 
     # ---- hot path
-    def _records(self, block_status, n_blocks, on_device):
-        """Address of a per-block status record buffer (None: no records): [n_blocks, BS_FIELDS, n_channels], 4-byte
-        elements, contiguous; a CUDA tensor for process(), a numpy array for the host paths."""
+    def _rows(self, channels):
+        """(ids array or None, row count) of a call: channels None = every channel; otherwise the ids whose rows the planes
+        hold, in that order (kept alive by the caller until the call returns)."""
+        if channels is None:
+            return None, self.n_channels
+        ids = np.ascontiguousarray(np.atleast_1d(np.asarray(channels)).astype(np.uint32))
+        return ids, ids.size
+
+    def _records(self, block_status, n_blocks, on_device, rows=None):
+        """Address of a per-block status record buffer (None: no records): [n_blocks, BS_FIELDS, rows] (rows: the call's
+        channel count), 4-byte elements, contiguous; a CUDA tensor for process(), a numpy array for the host paths."""
         if block_status is None:
             return None
-        want = (n_blocks, BS_FIELDS, self.n_channels)
+        want = (n_blocks, BS_FIELDS, self.n_channels if rows is None else rows)
         if on_device:
             assert block_status.is_cuda and block_status.is_contiguous() and block_status.element_size() == 4, \
                 "block_status: a contiguous CUDA tensor of 4-byte elements"
@@ -296,49 +310,66 @@ class SdrBatch:
         assert block_status.shape == want, "block_status: shape %r, want %r" % (block_status.shape, want)
         return block_status.ctypes.data
 
-    def process(self, I, Q, audio, n_blocks=None, stream=None, block_status=None):
+    def process(self, I, Q, audio, n_blocks=None, stream=None, block_status=None, channels=None):
         """Device tensors (torch, CUDA, 2-D [n_channels, >= 128*n_blocks], contiguous rows); asynchronous.  `block_status`:
         optional CUDA tensor [n_blocks, BS_FIELDS, n_channels] (4-byte dtype) that receives the getters after every block
-        (block_status_fields() names them), on the same stream as the audio."""
+        (block_status_fields() names them), on the same stream as the audio.  `channels`: run only these channel ids (distinct,
+        any order); the planes then have one row per listed channel, row i for channels[i], and the records
+        [n_blocks, BS_FIELDS, len(channels)]; every other channel skips the call untouched (sdr_batch_process_device_subset)."""
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
-        assert I.shape[0] == self.n_channels and Q.shape == I.shape and audio.shape[0] == self.n_channels
+        ids, rows = self._rows(channels)
+        assert I.shape[0] == rows and Q.shape == I.shape and audio.shape[0] == rows
         assert I.stride(1) == 1 and Q.stride(1) == 1 and audio.stride(1) == 1 and I.stride(0) == Q.stride(0)
         sp = C.c_void_p(stream.cuda_stream) if stream is not None else None
         args = (self.h, I.data_ptr(), Q.data_ptr(), I.stride(0), _fmt_of(str(I.dtype)), audio.data_ptr(), audio.stride(0),
                 _fmt_of(str(audio.dtype)), n_blocks)
-        if block_status is None:
+        if ids is not None:
+            self._check(self.L.sdr_batch_process_device_subset(args[0], ids.ctypes.data, rows, *args[1:],
+                                                               self._records(block_status, n_blocks, True, rows), sp))
+        elif block_status is None:
             self._check(self.L.sdr_batch_process_device(*args, sp))
         else:
             self._check(self.L.sdr_batch_process_device_status(*args, self._records(block_status, n_blocks, True), sp))
 
-    def process_host(self, I, Q, audio=None, out_fmt=FMT_F32, n_blocks=None, block_status=None):
+    def process_host(self, I, Q, audio=None, out_fmt=FMT_F32, n_blocks=None, block_status=None, channels=None):
         """Host numpy arrays [n_channels, S]; copies in, runs, copies out; returns the audio array.  `block_status`: optional
-        numpy array [n_blocks, BS_FIELDS, n_channels] (4-byte dtype) that receives the getters after every block."""
+        numpy array [n_blocks, BS_FIELDS, n_channels] (4-byte dtype) that receives the getters after every block.
+        `channels`: run only these channel ids, as in process() (planes [len(channels), S], records [.., len(channels)])."""
         I = np.ascontiguousarray(I)
         Q = np.ascontiguousarray(Q)
-        assert I.shape == Q.shape and I.dtype == Q.dtype and I.shape[0] == self.n_channels
+        ids, rows = self._rows(channels)
+        assert I.shape == Q.shape and I.dtype == Q.dtype and I.shape[0] == rows
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
         if audio is None:
-            audio = np.empty((self.n_channels, n_blocks * N_BLOCK), np.float32 if out_fmt == FMT_F32 else np.int16)
+            audio = np.empty((rows, n_blocks * N_BLOCK), np.float32 if out_fmt == FMT_F32 else np.int16)
+        assert audio.shape[0] == rows
         args = (self.h, I.ctypes.data, Q.ctypes.data, I.strides[0] // I.itemsize, _fmt_of(str(I.dtype)), audio.ctypes.data,
                 audio.strides[0] // audio.itemsize, _fmt_of(str(audio.dtype)), n_blocks)
-        if block_status is None:
+        if ids is not None:
+            self._check(self.L.sdr_batch_process_host_subset(args[0], ids.ctypes.data, rows, *args[1:],
+                                                             self._records(block_status, n_blocks, False, rows)))
+        elif block_status is None:
             self._check(self.L.sdr_batch_process_host(*args))
         else:
             self._check(self.L.sdr_batch_process_host_status(*args, self._records(block_status, n_blocks, False)))
         return audio
 
-    def submit_host(self, I, Q, audio, n_blocks=None, block_status=None):
+    def submit_host(self, I, Q, audio, n_blocks=None, block_status=None, channels=None):
         """Streaming form of process_host: queues the call and returns; `wait_host()` completes everything queued.  The arrays
         must be C-contiguous rows (they are used in place: no copy is made) and should be pinned; I, Q must stay unchanged
         and `audio` (and `block_status`, the optional per-block records as in process_host) unread until wait_host() -- or
-        wait_host(ticket) with the ticket this returns -- has returned."""
-        assert I.shape == Q.shape and I.dtype == Q.dtype and I.shape[0] == self.n_channels and audio.shape[0] == self.n_channels
+        wait_host(ticket) with the ticket this returns -- has returned.  `channels`: as in process_host (the id list is
+        copied by the library before this returns)."""
+        ids, rows = self._rows(channels)
+        assert I.shape == Q.shape and I.dtype == Q.dtype and I.shape[0] == rows and audio.shape[0] == rows
         assert I.strides[1] == I.itemsize and Q.strides == I.strides and audio.strides[1] == audio.itemsize
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
         args = (self.h, I.ctypes.data, Q.ctypes.data, I.strides[0] // I.itemsize, _fmt_of(str(I.dtype)), audio.ctypes.data,
                 audio.strides[0] // audio.itemsize, _fmt_of(str(audio.dtype)), n_blocks)
-        if block_status is None:
+        if ids is not None:
+            self._check(self.L.sdr_batch_submit_host_subset(args[0], ids.ctypes.data, rows, *args[1:],
+                                                            self._records(block_status, n_blocks, False, rows)))
+        elif block_status is None:
             self._check(self.L.sdr_batch_submit_host(*args))
         else:
             self._check(self.L.sdr_batch_submit_host_status(*args, self._records(block_status, n_blocks, False)))

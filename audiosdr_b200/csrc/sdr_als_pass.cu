@@ -22,7 +22,7 @@ extern "C" __global__ void __launch_bounds__(32, 8) sdr_als_pass_kernel(const __
   Ctx x;
   x.L = &L; x.Y = &L.lay; x.G = &L.groups[blockIdx.x]; x.smem = smem; x.gidx = (int)blockIdx.x; x.prof = false; x.rec = false; x.t0 = 0;
   const int lane = (int)threadIdx.x;
-  reinterpret_cast<int *>(smem + x.o_cid())[lane] = x.G->cid[lane];
+  reinterpret_cast<int *>(smem + x.o_cid())[lane] = x.G->row[lane];
   x.k.reset();
   RoleOut r; r.load(x, lane);
   const uint32_t n = L.n_tiles;

@@ -134,6 +134,17 @@ void build_agc_lut(float thr, float slope, float knee, float *lut) {
   lut[130] = lut[131] = 0.0f;
 }
 
+/* the blanker's mask words and ring planes are indexed by (absolute block index % 3): moving a channel between handles
+ * that have processed different numbers of blocks turns the slots by the difference */
+void rotate_slots(float *w, uint32_t delta) {
+  if (delta % 3 == 0) return;
+  std::vector<float> t(w, w + SDR_STATE_WORDS);
+  for (uint32_t s = 0; s < 3; s++) {
+    const uint32_t d = (s + delta) % 3;
+    memcpy(w + W_NB_MASK + d * 32, &t[W_NB_MASK + s * 32], 32 * sizeof(float));
+    for (uint32_t pl = 0; pl < 3; pl++) memcpy(w + W_NB_RING + pl * 384 + d * 128, &t[W_NB_RING + pl * 384 + s * 128], 128 * sizeof(float));
+  }
+}
 }  // namespace
 
 /* the groups of one pipeline class with one set of optional stages: one kernel launch with its own shared-memory plan */
@@ -142,6 +153,12 @@ struct Bucket {
   /* a bucket with the ALS filter and more groups than SMs runs as two launches (sdr_lay.h, lay_build_als): the chain up to
    * the AGC on the plan the bucket would have without ALS, then the ALS + output post-pass, four groups to an SM */
   bool split; SdrLay lay_main, lay_als;
+};
+
+/* the groups and buckets of one set of channels: every channel of the handle, or the channels of a subset call */
+struct Grouping {
+  std::vector<SdrGroup> groups; std::vector<Bucket> buckets;
+  SdrGroup *d_groups; size_t cap;
 };
 
 enum { SDR_HOST_TICKETS = 8 }; /* host calls whose completion can be waited for one by one (sdr_batch_wait_host_ticket) */
@@ -161,8 +178,8 @@ struct sdr_batch {
   std::vector<float> luts; /* [n][SDR_AGC_LUT_STRIDE] */
   size_t lut_gc_at; /* registry size at which unused tables are looked for next (collect_luts) */
   /* device */
-  float *d_state; SdrChanCfg *d_cfg; SdrGroup *d_groups; float *d_luts; SdrTables *d_tabs;
-  uint32_t *d_reset_ch, *d_reset_mask; size_t reset_cap; size_t luts_cap; size_t groups_cap;
+  float *d_state; SdrChanCfg *d_cfg; float *d_luts; SdrTables *d_tabs;
+  uint32_t *d_reset_ch, *d_reset_mask; size_t reset_cap; size_t luts_cap;
   float *d_gather; uint32_t *d_gather_ids; uint32_t *d_gather_words; size_t gather_cap;
   /* host-buffer path: two staging sets and three streams so that the H2D copy of chunk k+1, the kernel of chunk k and
    * the D2H copy of chunk k-1 overlap */
@@ -171,14 +188,24 @@ struct sdr_batch {
   void *s_h2d, *s_comp, *s_d2h; void *ev_h2d[2], *ev_comp[2], *ev_d2h[2];
   uint64_t host_seq; /* chunks queued by submit_host since create: chunk n uses staging set n & 1 */
   uint64_t host_calls; void *ev_call[SDR_HOST_TICKETS]; /* host calls queued since create (= the ticket of the latest); call t's last copy-out records ev_call[t % SDR_HOST_TICKETS] */
-  uint32_t n_groups;
   float *d_raw[SDR_MAX_BUCKETS]; size_t raw_cap[SDR_MAX_BUCKETS]; /* scratch planes of split ALS buckets (by bucket index), grown on demand */
   unsigned long long *d_prof; size_t prof_cap; bool prof_on; uint64_t prof_launches;
   std::vector<uint64_t> prof_busy, prof_total, prof_groups, prof_extra, prof_load, prof_crit, prof_bar; /* folded per class */
   uint64_t blocks_done, launches;
   void *last_stream;
   std::vector<SdrChanCfg> h_cfg;
-  std::vector<SdrGroup> h_groups;
+  /* every channel (the plain calls), and the last subset call's channels: kept apart, so that alternating the two forms
+   * re-plans neither; the subset grouping is reused while its id list and the configuration stay the same */
+  Grouping all, sub;
+  std::vector<uint32_t> sub_ids; bool sub_valid;
+  int prof_of; /* the grouping the profile rows belong to: 0 all, 1 sub */
+  /* Block clocks.  The blanker slots of a channel are laid out for the handle's block clock after the last call that ran
+   * it (or the import that installed it): max(plain_at, at[c]).  A channel whose layout is behind the clock when a call
+   * lists it again is turned first (SDRK_R_TURN*).  own[c]: the channel's blocks in subset calls (it has also run every
+   * block of the plain calls), the order of a subset's channels inside a bucket. */
+  uint64_t plain_at; bool sub_since_plain;
+  std::vector<uint64_t> at, own;
+  std::vector<uint8_t> id_mark;
 };
 
 namespace {
@@ -381,14 +408,18 @@ int plan_bucket(Bucket &b, int cls, uint32_t feat, int n_sm, uint32_t handle_gro
   return 0;
 }
 
-int build_groups(sdr_batch *h) {
-  h->h_groups.clear(); h->buckets.clear();
+/* Groups and buckets of the channels ids[0..n) (ids == nullptr: every channel), lane rows = the channels' positions in the
+ * list (their ids for every channel), with each group's feature summary and staged AGC tables. */
+int build_groups(sdr_batch *h, Grouping &G, const uint32_t *ids, uint32_t n) {
+  G.groups.clear(); G.buckets.clear();
   /* Channels of one class with the same optional stages share groups (= one bucket, one launch); inside a bucket they are
    * ordered by mode so that the lanes of a warp run the same oscillator frequency and coefficient set (channel results
-   * never depend on the grouping). */
+   * never depend on the grouping).  A subset's channels are also ordered by blocks processed: lanes with the same history
+   * keep one oscillator phase, so RoleNco stays on its one-oscillator table path. */
   static const int order[2][5] = {{SDR_LSB, SDR_USB, SDR_CW_LSB, SDR_CW_USB, SDR_WSPR}, {SDR_AM, SDR_SAM, -1, -1, -1}};
-  std::vector<uint32_t> by_key[2][8][5];
-  for (uint32_t c = 0; c < h->n_ch; c++) {
+  std::vector<uint32_t> by_key[2][8][5]; /* positions in the list */
+  for (uint32_t i = 0; i < n; i++) {
+    const uint32_t c = ids ? ids[i] : i;
     const int m = h->sh[c].mode, cls = (m == SDR_AM || m == SDR_SAM) ? CLS_ENV : CLS_SSB;
     int mi = 0;
     for (int k = 0; k < 5; k++) if (order[cls][k] == m) mi = k;
@@ -396,42 +427,45 @@ int build_groups(sdr_batch *h) {
 #ifndef SDR_HANDOVER
     if (m == SDR_SAM) f |= LF_SAM; /* SAM channels get groups (and a bucket) of their own: no AM lane among them */
 #endif
-    by_key[cls][f][mi].push_back(c);
+    by_key[cls][f][mi].push_back(i);
   }
+  if (ids)
+    for (auto &a : by_key) for (auto &b : a) for (auto &v : b)
+      std::stable_sort(v.begin(), v.end(), [&](uint32_t x, uint32_t y) { return h->own[ids[x]] < h->own[ids[y]]; });
   for (int cls = 0; cls < 2; cls++) {
     for (uint32_t feat = 0; feat < 8; feat++) {
-      Bucket b; b.first = (uint32_t)h->h_groups.size();
+      Bucket b; b.first = (uint32_t)G.groups.size();
       SdrGroup g; int fill = 0;
       auto flush = [&]() {
         if (!fill) return;
-        for (int l = fill; l < SDR_LANES; l++) g.cid[l] = -1;
-        h->h_groups.push_back(g); fill = 0;
+        for (int l = fill; l < SDR_LANES; l++) g.cid[l] = g.row[l] = -1;
+        G.groups.push_back(g); fill = 0;
       };
       for (int mi = 0; mi < 5; mi++) {
-        for (uint32_t c : by_key[cls][feat][mi]) {
+        for (uint32_t i : by_key[cls][feat][mi]) {
           if (!fill) { memset(&g, 0, sizeof g); g.cls = cls; }
-          g.cid[fill++] = (int32_t)c;
+          g.cid[fill] = (int32_t)(ids ? ids[i] : i); g.row[fill] = (int32_t)i; fill++;
           if (fill == SDR_LANES) flush();
         }
         /* SSB class: a group never mixes modes, so that all its lanes share one oscillator (RoleNco's table path) */
         if (cls == CLS_SSB) flush();
       }
       flush();
-      b.count = (uint32_t)h->h_groups.size() - b.first;
+      b.count = (uint32_t)G.groups.size() - b.first;
       if (!b.count) continue;
-      b.lay.cls = cls; b.lay.feat = feat; /* planned below, when the handle's group count is known */
-      h->buckets.push_back(b);
+      b.lay.cls = cls; b.lay.feat = feat; /* planned below, when the grouping's group count is known */
+      G.buckets.push_back(b);
     }
   }
-  h->n_groups = (uint32_t)h->h_groups.size();
-  if (h->buckets.size() > (size_t)SDR_MAX_BUCKETS) return fail(SDR_ERR_UNSUPPORTED, "more buckets than SDR_MAX_BUCKETS (internal)");
-  for (Bucket &b : h->buckets) {
-    if (plan_bucket(b, b.lay.cls, b.lay.feat, 148, h->n_groups)) return fail(SDR_ERR_UNSUPPORTED, "no shared-memory plan for a bucket (internal)");
+  const uint32_t n_groups = (uint32_t)G.groups.size();
+  if (G.buckets.size() > (size_t)SDR_MAX_BUCKETS) return fail(SDR_ERR_UNSUPPORTED, "more buckets than SDR_MAX_BUCKETS (internal)");
+  for (Bucket &b : G.buckets) {
+    if (plan_bucket(b, b.lay.cls, b.lay.feat, 148, n_groups)) return fail(SDR_ERR_UNSUPPORTED, "no shared-memory plan for a bucket (internal)");
     if (b.split) { /* the post-pass keeps as many taps and as much input history as the bucket's channels ask for (C:393-398) */
       int m_max = 0, reach_max = 0;
       for (uint32_t g = b.first; g < b.first + b.count; g++)
         for (int l = 0; l < SDR_LANES; l++) {
-          const int c = h->h_groups[g].cid[l];
+          const int c = G.groups[g].cid[l];
           if (c < 0 || !(h->h_cfg[c].flags & CF_ALS)) continue;
           const SdrChanCfg &k = h->h_cfg[c];
           m_max = std::max(m_max, (int)k.als_m); reach_max = std::max(reach_max, (int)k.als_m + (int)k.als_delay);
@@ -441,6 +475,34 @@ int build_groups(sdr_batch *h) {
       if (env_int("SDR_ALS_NO_MIRROR", 0) && b.lay_als.als_mirror) { b.lay_als.als_mirror = 0; b.lay_als.smem_bytes -= b.lay_als.nc * b.lay_als.tile_f * 4; }
     }
   }
+  for (SdrGroup &g : G.groups) {
+    g.feat = 0;
+    for (int k = 0; k < SDR_LUT_SLOTS; k++) g.lut_ids[k] = -1;
+    for (int l = 0; l < SDR_LANES; l++) {
+      g.lut_slot[l] = 255;
+      if (g.cid[l] < 0) continue;
+      g.feat |= h->h_cfg[g.cid[l]].flags;
+      int id = h->h_cfg[g.cid[l]].agc_lut;
+      for (int k = 0; k < SDR_LUT_SLOTS; k++) {
+        if (g.lut_ids[k] == id) { g.lut_slot[l] = (uint8_t)k; break; }
+        if (g.lut_ids[k] < 0) { g.lut_ids[k] = id; g.lut_slot[l] = (uint8_t)k; break; }
+      }
+      if (g.lut_slot[l] == 255) g.feat |= GF_LUT_GLOBAL;
+    }
+  }
+  return 0;
+}
+
+/* The grouping's groups to the device, in stream order: a launch of an earlier call that reads the buffer was queued on
+ * `stream` or joined into it (a buffer that must grow waits for the handle's last stream before it is freed). */
+int upload_groups(sdr_batch *h, Grouping &G, void *stream) {
+  size_t need = sizeof(SdrGroup) * std::max<size_t>(G.groups.size(), 1);
+  if (need > G.cap) {
+    if (G.d_groups) { if (dev_sync(h->last_stream)) return SDR_ERR_CUDA; dev_free(G.d_groups); G.d_groups = nullptr; G.cap = 0; }
+    if (dev_alloc((void **)&G.d_groups, need)) return SDR_ERR_NOMEM;
+    G.cap = need;
+  }
+  if (!G.groups.empty() && h2d(G.d_groups, G.groups.data(), sizeof(SdrGroup) * G.groups.size(), stream)) return SDR_ERR_CUDA;
   return 0;
 }
 
@@ -508,29 +570,9 @@ int sync_config(sdr_batch *h, void *stream) {
   }
   if (h->groups_dirty) {
     if (h->prof_on && fold_profile(h)) return SDR_ERR_CUDA; /* rows are per group: fold before the grouping changes */
-    { int rc = build_groups(h); if (rc) return rc; }
-    for (SdrGroup &g : h->h_groups) {
-      g.feat = 0;
-      for (int k = 0; k < SDR_LUT_SLOTS; k++) g.lut_ids[k] = -1;
-      for (int l = 0; l < SDR_LANES; l++) {
-        g.lut_slot[l] = 255;
-        if (g.cid[l] < 0) continue;
-        g.feat |= h->h_cfg[g.cid[l]].flags;
-        int id = h->h_cfg[g.cid[l]].agc_lut;
-        for (int k = 0; k < SDR_LUT_SLOTS; k++) {
-          if (g.lut_ids[k] == id) { g.lut_slot[l] = (uint8_t)k; break; }
-          if (g.lut_ids[k] < 0) { g.lut_ids[k] = id; g.lut_slot[l] = (uint8_t)k; break; }
-        }
-        if (g.lut_slot[l] == 255) g.feat |= GF_LUT_GLOBAL;
-      }
-    }
-    size_t need = sizeof(SdrGroup) * std::max<size_t>(h->h_groups.size(), 1);
-    if (need > h->groups_cap) {
-      if (h->d_groups) { if (dev_sync(h->last_stream)) return SDR_ERR_CUDA; dev_free(h->d_groups); }
-      if (dev_alloc((void **)&h->d_groups, need)) return SDR_ERR_NOMEM;
-      h->groups_cap = need;
-    }
-    if (!h->h_groups.empty() && h2d(h->d_groups, h->h_groups.data(), sizeof(SdrGroup) * h->h_groups.size(), stream)) return SDR_ERR_CUDA;
+    { int rc = build_groups(h, h->all, nullptr, h->n_ch); if (rc) return rc; }
+    { int rc = upload_groups(h, h->all, stream); if (rc) return rc; }
+    h->sub_valid = false; /* (built from the same configuration) */
     h->groups_dirty = false;
   }
   /* replay pending state re-initialisations */
@@ -544,6 +586,19 @@ int sync_config(sdr_batch *h, void *stream) {
       if (dev_alloc((void **)&h->d_reset_ch, cap * 4) || dev_alloc((void **)&h->d_reset_mask, cap * 4)) return SDR_ERR_NOMEM;
       h->reset_cap = cap;
     }
+#ifdef SDR_EMU
+    /* the host emulation's reset replays the setter side effects only: a slot turn runs here, on the host copy of the state,
+     * with the permutation export / import use (the CUDA reset kernel turns the same slots on the device) */
+    for (size_t i = 0; i < ch.size(); i++) {
+      if ((mk[i] & (SDRK_R_TURN1 | SDRK_R_TURN2)) && !(mk[i] & SDRK_R_NB)) {
+        std::vector<float> w(SDR_STATE_WORDS);
+        sdrk_launch_gather(h->d_state, h->ch_stride, &ch[i], 1, nullptr, SDR_STATE_WORDS, w.data(), stream);
+        rotate_slots(w.data(), (mk[i] & SDRK_R_TURN1) ? 1u : 2u);
+        sdrk_launch_scatter(h->d_state, h->ch_stride, &ch[i], 1, w.data(), stream);
+      }
+      mk[i] &= ~(uint32_t)(SDRK_R_TURN1 | SDRK_R_TURN2);
+    }
+#endif
     for (size_t o = 0; o < ch.size(); o += 65535) { /* gridDim.y limit */
       uint32_t n = (uint32_t)std::min<size_t>(65535, ch.size() - o);
       if (h2d(h->d_reset_ch + o, ch.data() + o, n * 4, stream) || h2d(h->d_reset_mask + o, mk.data() + o, n * 4, stream)) return SDR_ERR_CUDA;
@@ -560,11 +615,12 @@ int sync_config(sdr_batch *h, void *stream) {
 int fold_profile(sdr_batch *h) {
   if (!h->d_prof || !h->prof_launches) return 0;
   if (dev_sync(h->last_stream)) return SDR_ERR_CUDA;
-  std::vector<unsigned long long> rows((size_t)h->n_groups * SDR_PROF_SLOTS);
+  const std::vector<SdrGroup> &groups = (h->prof_of ? h->sub : h->all).groups;
+  std::vector<unsigned long long> rows(std::min(groups.size(), h->prof_cap / (SDR_PROF_SLOTS * 8)) * SDR_PROF_SLOTS);
   if (rows.empty()) return 0;
   if (d2h(rows.data(), h->d_prof, rows.size() * 8, h->last_stream) || dev_sync(h->last_stream)) return SDR_ERR_CUDA;
-  for (uint32_t g = 0; g < h->n_groups && g < h->h_groups.size(); g++) {
-    int cls = h->h_groups[g].cls;
+  for (uint32_t g = 0; g < rows.size() / SDR_PROF_SLOTS; g++) {
+    int cls = groups[g].cls;
     /* row layout (sdr_kernel.cu pipeline_loop, Probe::flush): [0..13] busy cycles per stage, [14] CTA pipeline cycles, [15] prologue,
      * [16..29] cycles per stage spent waiting for other stages, [30..32] NB sub-phases, [33..35] IN sub-phases */
     for (int w = 0; w < SDR_STAGES; w++) h->prof_busy[cls * SDR_STAGES + w] += rows[(size_t)g * SDR_PROF_SLOTS + w];
@@ -577,6 +633,39 @@ int fold_profile(sdr_batch *h) {
   if (dev_zero(h->d_prof, rows.size() * 8, h->last_stream)) return SDR_ERR_CUDA;
   h->prof_launches = 0;
   return 0;
+}
+
+/* A subset call's id list: ids == nullptr stands for every channel (n_ids == n_channels); otherwise 1 <= n_ids, every id below
+ * n_channels and none twice. */
+int check_ids(sdr_batch *h, const uint32_t *ids, uint32_t n_ids) {
+  if (!ids) return n_ids == h->n_ch ? 0 : fail(SDR_ERR_ARG, "channel_ids == NULL needs n_ids == n_channels");
+  if (n_ids == 0) return fail(SDR_ERR_ARG, "n_ids == 0");
+  uint32_t i = 0;
+  for (; i < n_ids && ids[i] < h->n_ch && !h->id_mark[ids[i]]; i++) h->id_mark[ids[i]] = 1;
+  for (uint32_t k = 0; k < i; k++) h->id_mark[ids[k]] = 0;
+  if (i == n_ids) return 0;
+  return fail(SDR_ERR_ARG, ids[i] >= h->n_ch ? "channel id out of range" : "channel id listed twice");
+}
+
+bool is_every_channel(const sdr_batch *h, const uint32_t *ids, uint32_t n_ids) {
+  if (n_ids != h->n_ch) return false;
+  for (uint32_t i = 0; i < n_ids; i++) if (ids[i] != i) return false;
+  return true;
+}
+
+/* Channels of the call (ids == nullptr: every channel) whose blanker slots are laid out for an earlier block clock get
+ * them turned onto the handle's clock, replayed with the setter side effects before the call's launches. */
+void queue_turns(sdr_batch *h, const uint32_t *ids, uint32_t n_ids) {
+  const uint64_t clk = h->blocks_done;
+  for (uint32_t i = 0; i < n_ids; i++) {
+    const uint32_t c = ids ? ids[i] : i;
+    const uint32_t d = (uint32_t)((clk - std::max(h->plain_at, h->at[c])) % 3);
+    if (d) {
+      if (!h->pend_reset[c]) h->dirty_list.push_back(c);
+      h->pend_reset[c] |= d == 1 ? SDRK_R_TURN1 : SDRK_R_TURN2;
+    }
+    h->at[c] = clk;
+  }
 }
 
 int check_plane(const void *p, size_t pitch, int fmt, uint32_t n_blocks, const char *what) {
@@ -606,7 +695,7 @@ void sdr_batch_destroy(sdr_batch_t *h) {
   if (!h) return;
   dev_select(h->desc.device);
   dev_sync(h->last_stream);
-  dev_free(h->d_state); dev_free(h->d_cfg); dev_free(h->d_groups); dev_free(h->d_luts); dev_free(h->d_tabs);
+  dev_free(h->d_state); dev_free(h->d_cfg); dev_free(h->all.d_groups); dev_free(h->sub.d_groups); dev_free(h->d_luts); dev_free(h->d_tabs);
   dev_free(h->d_reset_ch); dev_free(h->d_reset_mask); dev_free(h->d_gather); dev_free(h->d_gather_ids); dev_free(h->d_gather_words);
   for (int k = 0; k < 2; k++) {
     dev_free(h->d_in_i[k]); dev_free(h->d_in_q[k]); dev_free(h->d_out[k]); dev_free(h->d_bs[k]);
@@ -629,14 +718,17 @@ int sdr_batch_create(sdr_batch_t **out, const sdr_batch_desc *desc) {
   h->desc = *desc; h->n_ch = desc->n_channels;
   h->ch_stride = ((size_t)h->n_ch + 31) / 32 * 32;
   h->sh.resize(h->n_ch); h->pend_reset.assign(h->n_ch, 0); h->h_cfg.resize(h->n_ch); h->cfg_mark.assign(h->n_ch, 0);
+  h->at.assign(h->n_ch, 0); h->own.assign(h->n_ch, 0); h->id_mark.assign(h->n_ch, 0);
+  h->plain_at = 0; h->sub_since_plain = false; h->sub_valid = false; h->prof_of = 0;
+  h->all.d_groups = h->sub.d_groups = nullptr; h->all.cap = h->sub.cap = 0;
   h->cfg_dirty = h->groups_dirty = true; h->luts_dirty = false; h->cfg_all = true; h->lut_gc_at = 64;
-  h->d_state = nullptr; h->d_cfg = nullptr; h->d_groups = nullptr; h->d_luts = nullptr; h->d_tabs = nullptr;
-  h->d_reset_ch = h->d_reset_mask = nullptr; h->reset_cap = h->luts_cap = h->groups_cap = 0;
+  h->d_state = nullptr; h->d_cfg = nullptr; h->d_luts = nullptr; h->d_tabs = nullptr;
+  h->d_reset_ch = h->d_reset_mask = nullptr; h->reset_cap = h->luts_cap = 0;
   h->d_gather = nullptr; h->d_gather_ids = h->d_gather_words = nullptr; h->gather_cap = 0;
   for (int k = 0; k < 2; k++) { h->d_in_i[k] = h->d_in_q[k] = h->d_out[k] = h->d_bs[k] = nullptr; h->ev_h2d[k] = h->ev_comp[k] = h->ev_d2h[k] = nullptr; }
   h->s_h2d = h->s_comp = h->s_d2h = nullptr; h->stage_in_bytes = h->stage_out_bytes = h->stage_bs_bytes = 0; h->host_seq = 0;
   h->host_calls = 0; for (int k = 0; k < SDR_HOST_TICKETS; k++) h->ev_call[k] = nullptr;
-  h->n_groups = 0; h->blocks_done = 0; h->launches = 0; h->last_stream = nullptr;
+  h->blocks_done = 0; h->launches = 0; h->last_stream = nullptr;
   h->d_prof = nullptr; h->prof_cap = 0; h->prof_launches = 0;
   for (int k = 0; k < SDR_MAX_BUCKETS; k++) { h->d_raw[k] = nullptr; h->raw_cap[k] = 0; }
   h->ev_fork = nullptr; for (int k = 0; k < SDR_MAX_BUCKETS; k++) { h->s_aux[k] = nullptr; h->ev_join[k] = nullptr; }
@@ -709,7 +801,16 @@ int sdr_batch_process_device(sdr_batch_t *h, const void *I, const void *Q, size_
 
 int sdr_batch_process_device_status(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
                                     size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status, void *stream) {
+  return sdr_batch_process_device_subset(h, nullptr, h ? h->n_ch : 0, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks,
+                                         block_status, stream);
+}
+
+int sdr_batch_process_device_subset(sdr_batch_t *h, const uint32_t *ids, uint32_t n_ids, const void *I, const void *Q, size_t in_pitch,
+                                    int in_fmt, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status,
+                                    void *stream) {
   if (!h) return fail(SDR_ERR_ARG, "null handle");
+  { const int rc = check_ids(h, ids, n_ids); if (rc) return rc; }
+  if (ids && is_every_channel(h, ids, n_ids)) ids = nullptr; /* the plain call */
   if (n_blocks == 0) return fail(SDR_ERR_ARG, "n_blocks == 0");
   if ((uintptr_t)block_status % 16 != 0) return fail(SDR_ERR_ARG, "block_status: the record buffer must be 16-byte aligned");
   if (h->desc.max_blocks_per_call && n_blocks > h->desc.max_blocks_per_call) return fail(SDR_ERR_ARG, "n_blocks > max_blocks_per_call");
@@ -723,16 +824,28 @@ int sdr_batch_process_device_status(sdr_batch_t *h, const void *I, const void *Q
    * another stream (they share the handle's state and tables) */
   if (h->launches && stream != h->last_stream && dev_sync(h->last_stream)) return SDR_ERR_CUDA;
   if (getenv("SDR_MAP_SEARCH")) h->groups_dirty = true; /* tools/map_search.py: plan (and read the placement variables) at every call */
+  if (ids || h->sub_since_plain) queue_turns(h, ids, n_ids); /* (nothing lags while only plain calls are made) */
   if ((rc = sync_config(h, stream)) != 0) return rc;
+  Grouping &G = ids ? h->sub : h->all;
+  if (ids && (!h->sub_valid || h->sub_ids.size() != n_ids || !std::equal(ids, ids + n_ids, h->sub_ids.begin()))) {
+    if (h->prof_on && h->prof_of == 1 && fold_profile(h)) return SDR_ERR_CUDA; /* rows are per group: fold before the grouping changes */
+    h->sub_valid = false;
+    if ((rc = build_groups(h, h->sub, ids, n_ids)) != 0 || (rc = upload_groups(h, h->sub, stream)) != 0) return rc;
+    h->sub_ids.assign(ids, ids + n_ids); h->sub_valid = true;
+  }
+  if (h->prof_on && h->prof_of != (ids ? 1 : 0)) {
+    if (fold_profile(h)) return SDR_ERR_CUDA;
+    h->prof_of = ids ? 1 : 0;
+  }
   SdrLaunch L;
   memset(&L, 0, sizeof L);
   L.in_i = I; L.in_q = Q; L.out = audio; L.in_pitch = in_pitch; L.out_pitch = out_pitch; L.in_fmt = in_fmt; L.out_fmt = out_fmt;
   L.blk0_mod3 = (uint32_t)(h->blocks_done % 3);
   L.flags = h->desc.flags & SDR_BATCH_CONTRACT;
   L.cfg = h->d_cfg; L.state = h->d_state; L.ch_stride = h->ch_stride; L.agc_luts = h->d_luts; L.tabs = h->d_tabs;
-  L.bstat = (uint32_t *)block_status; L.bs_stride = h->n_ch; /* every bucket writes the records of its own channels */
+  L.bstat = (uint32_t *)block_status; L.bs_stride = n_ids; /* every bucket writes the records of its own channels */
   if (h->prof_on) {
-    size_t need = (size_t)std::max<uint32_t>(h->n_groups, 1) * SDR_PROF_SLOTS * 8;
+    size_t need = std::max<size_t>(G.groups.size(), 1) * SDR_PROF_SLOTS * 8;
     if (need > h->prof_cap) {
       dev_free(h->d_prof); h->d_prof = nullptr;
       if (dev_alloc((void **)&h->d_prof, need) || dev_zero(h->d_prof, need, stream)) return SDR_ERR_NOMEM;
@@ -743,7 +856,7 @@ int sdr_batch_process_device_status(sdr_batch_t *h, const void *I, const void *Q
   }
   /* one launch per bucket; the first on the caller's stream, the others on streams forked from it and joined back, so
    * that the buckets of a mixed handle share the GPU instead of queueing behind each other */
-  const size_t nbk = h->buckets.size();
+  const size_t nbk = G.buckets.size();
   if (nbk > 1) {
     if (!h->ev_fork) {
       if (dev_event_create(&h->ev_fork)) return SDR_ERR_CUDA;
@@ -752,10 +865,10 @@ int sdr_batch_process_device_status(sdr_batch_t *h, const void *I, const void *Q
     if (dev_event_record(h->ev_fork, stream)) return SDR_ERR_CUDA;
   }
   for (size_t k = 0; k < nbk; k++) {
-    const Bucket &b = h->buckets[k];
+    const Bucket &b = G.buckets[k];
     void *s = k == 0 ? stream : h->s_aux[k - 1];
     if (k > 0 && dev_stream_wait(s, h->ev_fork)) return SDR_ERR_CUDA;
-    L.lay = b.lay; L.groups = h->d_groups + b.first; L.n_groups = b.count;
+    L.lay = b.lay; L.groups = G.d_groups + b.first; L.n_groups = b.count;
     L.n_tiles = n_blocks * (uint32_t)b.lay.tpb;
     L.prof = h->prof_on ? h->d_prof + (size_t)b.first * SDR_PROF_SLOTS : nullptr;
     if (getenv("SDR_DEBUG_PLAN")) {
@@ -792,7 +905,7 @@ int sdr_batch_process_device_status(sdr_batch_t *h, const void *I, const void *Q
         M.raw = h->d_raw[k];
         SdrLaunch A = M;
         A.bstat = nullptr; /* the records come from the chain launch (its AGC stage), the post-pass writes none */
-        if (M.bstat) M.bstat += (size_t)b0 * SDR_BS_FIELDS * h->n_ch;
+        if (M.bstat) M.bstat += (size_t)b0 * SDR_BS_FIELDS * n_ids;
         M.lay = b.lay_main; M.n_tiles = nb * (uint32_t)b.lay_main.tpb; M.flags |= SDRL_RAW_OUT;
         A.lay = b.lay_als; A.n_tiles = nb * (uint32_t)b.lay_als.tpb;
         A.lay.smem_bytes += env_int("SDR_ALS_PASS_PAD", 0); /* experiment: fewer groups per SM in the post-pass */
@@ -809,6 +922,12 @@ int sdr_batch_process_device_status(sdr_batch_t *h, const void *I, const void *Q
     if (k > 0 && (dev_event_record(h->ev_join[k - 1], s) || dev_stream_wait(stream, h->ev_join[k - 1]))) return SDR_ERR_CUDA;
   }
   h->blocks_done += n_blocks;
+  if (ids) {
+    for (uint32_t i = 0; i < n_ids; i++) { h->at[ids[i]] = h->blocks_done; h->own[ids[i]] += n_blocks; }
+    h->sub_since_plain = true;
+  } else {
+    h->plain_at = h->blocks_done; h->sub_since_plain = false;
+  }
   h->last_stream = stream;
   return SDR_OK;
 }
@@ -839,8 +958,8 @@ int sdr_batch_wait_host_ticket(sdr_batch_t *h, uint64_t ticket) {
   return dev_event_sync(h->ev_call[t % SDR_HOST_TICKETS]) ? SDR_ERR_CUDA : SDR_OK;
 }
 
-static int host_call(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt,
-                     uint32_t n_blocks, void *block_status, bool streamed);
+static int host_call(sdr_batch_t *h, const uint32_t *ids, uint32_t n_ids, const void *I, const void *Q, size_t in_pitch, int in_fmt,
+                     void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status, bool streamed);
 
 int sdr_batch_process_host(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
                            size_t out_pitch, int out_fmt, uint32_t n_blocks) {
@@ -849,7 +968,12 @@ int sdr_batch_process_host(sdr_batch_t *h, const void *I, const void *Q, size_t 
 
 int sdr_batch_process_host_status(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
                                   size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status) {
-  const int rc = host_call(h, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status, false);
+  return sdr_batch_process_host_subset(h, nullptr, h ? h->n_ch : 0, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status);
+}
+
+int sdr_batch_process_host_subset(sdr_batch_t *h, const uint32_t *ids, uint32_t n_ids, const void *I, const void *Q, size_t in_pitch,
+                                  int in_fmt, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status) {
+  const int rc = host_call(h, ids, n_ids, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status, false);
   if (rc) return rc; /* (the streams have been drained) */
   return sdr_batch_wait_host(h);
 }
@@ -861,12 +985,19 @@ int sdr_batch_submit_host(sdr_batch_t *h, const void *I, const void *Q, size_t i
 
 int sdr_batch_submit_host_status(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
                                  size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status) {
-  return host_call(h, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status, true);
+  return sdr_batch_submit_host_subset(h, nullptr, h ? h->n_ch : 0, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status);
 }
 
-static int host_call(sdr_batch_t *h, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt,
-                     uint32_t n_blocks, void *block_status, bool streamed) {
+int sdr_batch_submit_host_subset(sdr_batch_t *h, const uint32_t *ids, uint32_t n_ids, const void *I, const void *Q, size_t in_pitch,
+                                 int in_fmt, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status) {
+  return host_call(h, ids, n_ids, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status, true);
+}
+
+static int host_call(sdr_batch_t *h, const uint32_t *ids, uint32_t n_ids, const void *I, const void *Q, size_t in_pitch, int in_fmt,
+                     void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status, bool streamed) {
   if (!h || !I || !Q || !audio) return fail(SDR_ERR_ARG, "process_host: bad arguments");
+  { const int rc = check_ids(h, ids, n_ids); if (rc) return rc; }
+  const uint32_t n_rows = n_ids; /* rows of the planes and record columns: one per listed channel */
   if (n_blocks == 0) return fail(SDR_ERR_ARG, "n_blocks == 0");
   if ((uintptr_t)block_status % 16 != 0) return fail(SDR_ERR_ARG, "block_status: the record buffer must be 16-byte aligned");
   if (in_fmt != SDR_FMT_I16 && in_fmt != SDR_FMT_F32) return fail(SDR_ERR_ARG, "process_host: unknown input format");
@@ -889,14 +1020,14 @@ static int host_call(sdr_batch_t *h, const void *I, const void *Q, size_t in_pit
   if (chunk > n_blocks) chunk = n_blocks;
   if (h->desc.max_blocks_per_call && chunk > h->desc.max_blocks_per_call) chunk = h->desc.max_blocks_per_call;
   const size_t cs = (size_t)chunk * SDR_BLOCK_SAMPLES;
-  const size_t in_bytes = cs * ies * h->n_ch, out_bytes = cs * oes * h->n_ch;
+  const size_t in_bytes = cs * ies * n_rows, out_bytes = cs * oes * n_rows;
   if (!h->s_comp) {
     if (dev_stream_create(&h->s_h2d) || dev_stream_create(&h->s_comp) || dev_stream_create(&h->s_d2h)) return SDR_ERR_CUDA;
     for (int k = 0; k < 2; k++)
       if (dev_event_create(&h->ev_h2d[k]) || dev_event_create(&h->ev_comp[k]) || dev_event_create(&h->ev_d2h[k])) return SDR_ERR_CUDA;
     for (int k = 0; k < SDR_HOST_TICKETS; k++) if (dev_event_create(&h->ev_call[k])) return SDR_ERR_CUDA;
   }
-  const size_t bs_bytes = block_status ? (size_t)chunk * SDR_BS_FIELDS * h->n_ch * 4 : 0;
+  const size_t bs_bytes = block_status ? (size_t)chunk * SDR_BS_FIELDS * n_rows * 4 : 0;
   if (in_bytes > h->stage_in_bytes || out_bytes > h->stage_out_bytes || bs_bytes > h->stage_bs_bytes) {
     dev_sync(h->last_stream); dev_sync(h->s_h2d); dev_sync(h->s_comp); dev_sync(h->s_d2h);
     const bool grow_in = in_bytes > h->stage_in_bytes, grow_out = out_bytes > h->stage_out_bytes, grow_bs = bs_bytes > h->stage_bs_bytes;
@@ -951,21 +1082,21 @@ static int host_call(sdr_batch_t *h, const void *I, const void *Q, size_t in_pit
     /* H2D of chunk k into staging set b: the kernel of chunk k-2 (of this call or, with submit_host, of the call before) must
      * be done with it */
     if (h->host_seq >= 2) { SDR_TRY(dev_stream_wait(h->s_h2d, h->ev_comp[b]) ? SDR_ERR_CUDA : 0); }
-    SDR_TRY(h2d_2d(h->d_in_i[b], cs * ies, srcI, in_pitch * ies, w_in, h->n_ch, h->s_h2d) ? SDR_ERR_CUDA : 0);
-    SDR_TRY(h2d_2d(h->d_in_q[b], cs * ies, srcQ, in_pitch * ies, w_in, h->n_ch, h->s_h2d) ? SDR_ERR_CUDA : 0);
+    SDR_TRY(h2d_2d(h->d_in_i[b], cs * ies, srcI, in_pitch * ies, w_in, n_rows, h->s_h2d) ? SDR_ERR_CUDA : 0);
+    SDR_TRY(h2d_2d(h->d_in_q[b], cs * ies, srcQ, in_pitch * ies, w_in, n_rows, h->s_h2d) ? SDR_ERR_CUDA : 0);
     SDR_TRY(dev_event_record(h->ev_h2d[b], h->s_h2d) ? SDR_ERR_CUDA : 0);
     /* kernel of chunk k: needs its input, and the D2H of chunk k-2 must have drained output set b */
     SDR_TRY(dev_stream_wait(h->s_comp, h->ev_h2d[b]) ? SDR_ERR_CUDA : 0);
     if (h->host_seq >= 2) { SDR_TRY(dev_stream_wait(h->s_comp, h->ev_d2h[b]) ? SDR_ERR_CUDA : 0); }
-    int rc = sdr_batch_process_device_status(h, h->d_in_i[b], h->d_in_q[b], cs, in_fmt, h->d_out[b], cs, out_fmt, nb,
+    int rc = sdr_batch_process_device_subset(h, ids, n_ids, h->d_in_i[b], h->d_in_q[b], cs, in_fmt, h->d_out[b], cs, out_fmt, nb,
                                              block_status ? h->d_bs[b] : nullptr, h->s_comp);
     SDR_TRY(rc);
     SDR_TRY(dev_event_record(h->ev_comp[b], h->s_comp) ? SDR_ERR_CUDA : 0);
     /* D2H of chunk k: audio, then its records (block-major: the chunk's blocks are one contiguous range of the caller's buffer) */
     SDR_TRY(dev_stream_wait(h->s_d2h, h->ev_comp[b]) ? SDR_ERR_CUDA : 0);
-    SDR_TRY(d2h_2d(dst, out_pitch * oes, h->d_out[b], cs * oes, w_out, h->n_ch, h->s_d2h) ? SDR_ERR_CUDA : 0);
+    SDR_TRY(d2h_2d(dst, out_pitch * oes, h->d_out[b], cs * oes, w_out, n_rows, h->s_d2h) ? SDR_ERR_CUDA : 0);
     if (block_status) {
-      const size_t rec = (size_t)SDR_BS_FIELDS * h->n_ch; /* words per block */
+      const size_t rec = (size_t)SDR_BS_FIELDS * n_rows; /* words per block */
       SDR_TRY(d2h((uint32_t *)block_status + (size_t)done * rec, h->d_bs[b], (size_t)nb * rec * 4, h->s_d2h) ? SDR_ERR_CUDA : 0);
     }
     SDR_TRY(dev_event_record(h->ev_d2h[b], h->s_d2h) ? SDR_ERR_CUDA : 0);
@@ -1036,17 +1167,6 @@ namespace {
 const uint32_t STATE_MAGIC = 0x53445242u; /* "SDRB" */
 struct StateHeader { uint32_t magic, version, phase, shadow_bytes; };
 size_t state_blob_bytes() { return sizeof(StateHeader) + ((sizeof(Shadow) + 15) / 16) * 16 + sizeof(float) * SDR_STATE_WORDS; }
-/* the blanker's mask words and ring planes are indexed by (absolute block index % 3): moving a channel between handles
- * that have processed different numbers of blocks turns the slots by the difference */
-void rotate_slots(float *w, uint32_t delta) {
-  if (delta % 3 == 0) return;
-  std::vector<float> t(w, w + SDR_STATE_WORDS);
-  for (uint32_t s = 0; s < 3; s++) {
-    const uint32_t d = (s + delta) % 3;
-    memcpy(w + W_NB_MASK + d * 32, &t[W_NB_MASK + s * 32], 32 * sizeof(float));
-    for (uint32_t pl = 0; pl < 3; pl++) memcpy(w + W_NB_RING + pl * 384 + d * 128, &t[W_NB_RING + pl * 384 + s * 128], 128 * sizeof(float));
-  }
-}
 }  // namespace
 
 size_t sdr_batch_state_bytes(void) { return state_blob_bytes(); }
@@ -1074,9 +1194,10 @@ int sdr_batch_export_state(sdr_batch_t *h, const uint32_t *ids, uint32_t n, void
   for (uint32_t i = 0; i < n; i++) {
     char *b = (char *)blobs + (size_t)i * bb;
     memset(b, 0, bb);
-    StateHeader hd = {STATE_MAGIC, 1u, (uint32_t)(h->blocks_done % 3), (uint32_t)sizeof(Shadow)};
+    const uint32_t c = ids ? ids[i] : i;
+    StateHeader hd = {STATE_MAGIC, 1u, (uint32_t)(std::max(h->plain_at, h->at[c]) % 3), (uint32_t)sizeof(Shadow)}; /* the clock its slots are laid out for */
     memcpy(b, &hd, sizeof hd);
-    memcpy(b + so, &h->sh[ids ? ids[i] : i], sizeof(Shadow));
+    memcpy(b + so, &h->sh[c], sizeof(Shadow));
     memcpy(b + wo, &words[(size_t)i * SDR_STATE_WORDS], sizeof(float) * SDR_STATE_WORDS);
   }
   return SDR_OK;
@@ -1104,7 +1225,7 @@ int sdr_batch_import_state(sdr_batch_t *h, const uint32_t *ids, uint32_t n, cons
     cid[i] = c;
     Shadow sh; memcpy(&sh, b + so, sizeof sh);
     sh.lut_id = lut_for(h, sh.thr, sh.slope, sh.knee); /* table ids are local to a handle */
-    h->sh[c] = sh; h->pend_reset[c] = 0;
+    h->sh[c] = sh; h->pend_reset[c] = 0; h->at[c] = h->blocks_done; /* (turned onto this handle's clock below) */
     float *w = &words[(size_t)i * SDR_STATE_WORDS];
     memcpy(w, b + wo, sizeof(float) * SDR_STATE_WORDS);
     rotate_slots(w, (uint32_t)((h->blocks_done % 3) + 3 - hd.phase));

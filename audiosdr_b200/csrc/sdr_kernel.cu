@@ -25,7 +25,8 @@ int sdrk_setup_als_pass(void), sdrk_occupancy_als_pass(const SdrLaunch *); /* sd
 }
 
 /* Zero (or re-seed) state words of listed channels: the side effects of the reference setters that
- * re-initialise filter state / rings (SURVEY 8a13).  One thread per (entry, word). */
+ * re-initialise filter state / rings (SURVEY 8a13), and the turn of a lagging channel's blanker slots.  One thread per
+ * (entry, word). */
 extern "C" __global__ void sdr_reset_kernel(float *state, unsigned long long ch_stride, const uint32_t *chan, const uint32_t *mask,
                                             uint32_t n) {
   const uint32_t e = blockIdx.y;
@@ -44,6 +45,22 @@ extern "C" __global__ void sdr_reset_kernel(float *state, unsigned long long ch_
     float4 *ring = reinterpret_cast<float4 *>(state + (size_t)W_NB_RING * ch_stride);
     for (uint32_t f = blockIdx.x * blockDim.x + threadIdx.x; f < 288; f += gridDim.x * blockDim.x)
       ring[(size_t)f * ch_stride + c] = make_float4(0.f, 0.f, 0.f, 0.f);
+  } else if (m & (SDRK_R_TURN1 | SDRK_R_TURN2)) {
+    /* task j < 32: mask word j of the 3 slots; task 32 + 32 * plane + g: float4 group g of the 3 slots of a ring plane */
+    const uint32_t d = (m & SDRK_R_TURN1) ? 1u : 2u;
+    for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < 128; j += gridDim.x * blockDim.x) {
+      if (j < 32) {
+        float v[3];
+        for (uint32_t s = 0; s < 3; s++) v[s] = state[(size_t)(W_NB_MASK + s * 32 + j) * ch_stride + c];
+        for (uint32_t s = 0; s < 3; s++) state[(size_t)(W_NB_MASK + (s + d) % 3 * 32 + j) * ch_stride + c] = v[s];
+      } else {
+        float4 *ring = reinterpret_cast<float4 *>(state + (size_t)W_NB_RING * ch_stride);
+        const uint32_t pl = (j - 32) >> 5, g = j & 31;
+        float4 v[3];
+        for (uint32_t s = 0; s < 3; s++) v[s] = ring[(size_t)(pl * 96 + s * 32 + g) * ch_stride + c];
+        for (uint32_t s = 0; s < 3; s++) ring[(size_t)(pl * 96 + (s + d) % 3 * 32 + g) * ch_stride + c] = v[s];
+      }
+    }
   }
 }
 

@@ -10,7 +10,12 @@ enum {
   SDRK_R_IMG = 2u, /* ... on the AM image rails                           (init, C:178-179)        */
   SDRK_R_AUD = 4u, /* ... on the audio filter                             (setAudioFilter, C:298-311) */
   SDRK_R_ALS = 8u, /* taps and ring zeroed                                (enableALSfilter, C:384-391) */
-  SDRK_R_NB = 16u  /* initBlanker                                         (C:676-682)              */
+  SDRK_R_NB = 16u, /* initBlanker                                         (C:676-682)              */
+  /* not a setter: a channel that skipped calls of a subset (sdr_batch_process_*_subset) gets its blanker mask and ring block
+   * slots turned onto the handle's block clock before its next block -- slot s moves to (s + 1) % 3 or (s + 2) % 3 (the
+   * permutation of sdr_host.cpp rotate_slots).  Ignored together with SDRK_R_NB, which zeroes those slots anyway. */
+  SDRK_R_TURN1 = 32u,
+  SDRK_R_TURN2 = 64u
 };
 
 #ifdef __cplusplus

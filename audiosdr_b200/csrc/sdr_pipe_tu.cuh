@@ -271,7 +271,7 @@ __device__ __forceinline__ void pipeline_cta(const SdrLaunch &L, unsigned char *
   x.t0 = PROF ? clock64() : 0;
   const int nthr = (int)blockDim.x;
   for (int i = threadIdx.x; i < 257; i += nthr) x.f(x.o_sine())[i] = L.tabs->sine[i];
-  if (threadIdx.x < SDR_LANES) reinterpret_cast<int *>(smem + x.o_cid())[threadIdx.x] = x.G->cid[threadIdx.x];
+  if (threadIdx.x < SDR_LANES) reinterpret_cast<int *>(smem + x.o_cid())[threadIdx.x] = x.G->row[threadIdx.x];
 #ifndef SDR_LOCKSTEP
   {
     const uint32_t bars = (uint32_t)__cvta_generic_to_shared(smem + x.o_bar());
@@ -283,7 +283,7 @@ __device__ __forceinline__ void pipeline_cta(const SdrLaunch &L, unsigned char *
   if (threadIdx.x < 4) bulk_bar_init(smem + x.o_lut() + SDR_INBAR_OFF + 8 * threadIdx.x, SDR_LANES); /* input landing buffers: every lane of stage IN arrives */
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 #endif
-  __syncthreads(); /* stage IN requests its first tile from load(), which needs the channel ids */
+  __syncthreads(); /* stage IN requests its first tile from load(), which needs the plane rows */
   for (int i = threadIdx.x; i < SDR_LUT_SLOTS * SDR_AGC_LUT_STRIDE; i += nthr) { /* the group's AGC tables */
     const int id = x.G->lut_ids[i / SDR_AGC_LUT_STRIDE];
     if (id >= 0) x.f(x.o_lut())[i] = L.agc_luts[(size_t)id * SDR_AGC_LUT_STRIDE + i % SDR_AGC_LUT_STRIDE];

@@ -6,7 +6,7 @@
  *           A warp whose 32 lanes own 32 consecutive channels therefore touches one 128-byte line per
  *           state word.  The state IS the checkpoint: everything a channel carries from block to block.
  * cfg     : one SdrChanCfg per channel (array of structs; read once per launch per role).
- * groups  : one SdrGroup per CTA: 32 channel ids of one pipeline class (-1 = empty lane).
+ * groups  : one SdrGroup per CTA: 32 channel ids of one pipeline class (-1 = empty lane) and their plane rows.
  * planes  : caller-owned I/Q/audio, channel-major (include/sdr_batch.h).
  */
 #ifndef SDR_TYPES_H
@@ -89,6 +89,8 @@ typedef struct {
   int32_t cid[SDR_LANES];        /* channel id per lane, -1 = empty */
   int32_t lut_ids[SDR_LUT_SLOTS];/* up to 4 distinct AGC tables of this group, staged in shared memory (-1 = unused) */
   uint8_t lut_slot[SDR_LANES];   /* per lane: slot in lut_ids, or 255 = read the table from global memory */
+  int32_t row[SDR_LANES];        /* per lane: the channel's row in the call's I/Q/audio planes and record columns (-1 = empty).
+                                    Equal to cid in a call on every channel; the position of cid in the id list of a subset call */
 } SdrGroup;
 
 /* ---- constant tables in device memory ---- */
@@ -150,9 +152,9 @@ typedef struct {
   uint32_t diag_skip;    /* diagnostics (profiling runs only): bit s set = stage s idles; results are then meaningless */
   unsigned long long *prof; /* optional [n_groups][SDR_PROF_SLOTS] (diagnostics twin): busy and waiting cycles per stage */
   uint32_t *bstat;       /* optional per-block status records of the launch's blocks (include/sdr_batch.h, SDR_BS_*): word
-                            ((block * SDR_BS_FIELDS + field) * bs_stride + channel); null = no records.  Written at the end of
+                            ((block * SDR_BS_FIELDS + field) * bs_stride + row); null = no records.  Written at the end of
                             each block by the stage that owns the field (sdr_pipeline.cuh, Ctx::bs_put) */
-  unsigned long long bs_stride; /* = the handle's channel count */
+  unsigned long long bs_stride; /* = the call's row count (the handle's channel count, or the length of a subset call's id list) */
   SdrLay lay;
 } SdrLaunch;
 

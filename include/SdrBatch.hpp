@@ -152,6 +152,23 @@ class SdrBatch {
                    uint32_t n_blocks, void *block_status) {
     check(sdr_batch_submit_host_status(h_, I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt, n_blocks, block_status), "sdr_batch_submit_host_status");
   }
+  /* ... on the channels `ids` only (sdr_batch_process_*_subset): row i of the planes and record column i belong to ids[i];
+   * every other channel skips the call untouched, as update() does without input (AudioSDR.cpp:48-56) */
+  void process(const std::vector<uint32_t> &ids, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
+               size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status = nullptr, void *cuda_stream = nullptr) {
+    check(sdr_batch_process_device_subset(h_, ids.data(), (uint32_t)ids.size(), I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt,
+                                          n_blocks, block_status, cuda_stream), "sdr_batch_process_device_subset");
+  }
+  void process_host(const std::vector<uint32_t> &ids, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
+                    size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status = nullptr) {
+    check(sdr_batch_process_host_subset(h_, ids.data(), (uint32_t)ids.size(), I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt,
+                                        n_blocks, block_status), "sdr_batch_process_host_subset");
+  }
+  void submit_host(const std::vector<uint32_t> &ids, const void *I, const void *Q, size_t in_pitch, int in_fmt, void *audio,
+                   size_t out_pitch, int out_fmt, uint32_t n_blocks, void *block_status = nullptr) {
+    check(sdr_batch_submit_host_subset(h_, ids.data(), (uint32_t)ids.size(), I, Q, in_pitch, in_fmt, audio, out_pitch, out_fmt,
+                                       n_blocks, block_status), "sdr_batch_submit_host_subset");
+  }
   void wait_host() { check(sdr_batch_wait_host(h_), "sdr_batch_wait_host"); }
   uint64_t host_ticket() const { return sdr_batch_host_ticket(h_); } /* names the call submitted last */
   void wait_host(uint64_t ticket) { check(sdr_batch_wait_host_ticket(h_, ticket), "sdr_batch_wait_host_ticket"); }

@@ -15,6 +15,7 @@
  *                            (receiveWritable(0/1) C:46-47 = the I/Q planes in; transmit(blockI,0/1) C:164-165 = the audio plane out)
  *   sdr_batch_get_status    the getters                                          C:224-230,255-273,295,371-381,495,507-512,568-600,660-665,752-757
  *   sdr_batch_*_status      process + the dynamic getters polled after every block (per-block status records, SDR_BS_*)
+ *   sdr_batch_*_subset      process on the listed channels only; the others skip the call as update() does without input C:48-56
  *   sdr_batch_destroy       (object lifetime)
  *
  * Data layout: channel-major planes.  Sample t of channel c lives at plane[c*pitch + t]; pitch is
@@ -170,7 +171,8 @@ int sdr_batch_set(sdr_batch_t *h, const uint32_t *channel_ids, uint32_t n, uint3
 int sdr_batch_configure(sdr_batch_t *h, const sdr_setter_call *calls, uint32_t n_calls);
 
 /* The hot path.  Device pointers; asynchronous on `cuda_stream` (a cudaStream_t, NULL = default stream).
- * in_fmt/out_fmt: SDR_FMT_*; pitches in elements.  Advances every channel by n_blocks blocks.
+ * in_fmt/out_fmt: SDR_FMT_*; pitches in elements.  Advances every channel by n_blocks blocks (the _subset forms below: the
+ * listed channels only).
  * Device memory the handle owns besides the 7.9 KB of state per channel: a handle with more than 148 groups of 32
  * channels (4 736 channels or fewer, by mode mix) keeps a scratch plane for those that use the ALS filter, 4 bytes per ALS
  * channel and sample of the longest call so far, at most SDR_ALS_SCRATCH_MB (environment, default 4096) megabytes per kind
@@ -208,6 +210,32 @@ int sdr_batch_submit_host_status(sdr_batch_t *h, const void *I, const void *Q, s
  * two calls queued drains call n while call n + 1 is being copied in and computed.  Calls complete in order. */
 uint64_t sdr_batch_host_ticket(const sdr_batch_t *h);
 int sdr_batch_wait_host_ticket(sdr_batch_t *h, uint64_t ticket);
+
+/* The same calls on a chosen subset of the channels: the reference's update() returns without touching anything when an
+ * input block is missing (C:48-56), so in a graph some objects skip a block period while others run.  The call advances
+ * the n_ids channels channel_ids[0..n_ids) by n_blocks blocks each, bit for bit as update() would; every other channel is
+ * untouched -- state, getters, no plane row and no record -- and its next processed block continues its own stream.  A
+ * channel's output over any sequence of calls is therefore the reference run on that channel's own blocks, concatenated.
+ *   channel_ids  host memory, read before the call returns; distinct ids below n_channels, n_ids >= 1.  NULL (with
+ *                n_ids == n_channels) is exactly the call on every channel: the entry points above are these calls with NULL.
+ *                Anything else returns SDR_ERR_ARG and queues nothing.
+ *   planes       compact: row i of I, Q and audio belongs to channel channel_ids[i] (n_ids rows, any order of ids).
+ *   block_status compact too: status[((size_t)b * SDR_BS_FIELDS + f) * n_ids + i] (NULL: no records).
+ * Setters are unchanged: a setter on a channel that is not listed takes effect before that channel's next processed block,
+ * as a setter between two ISRs does to an object that got no block.  get_status, export_state and import_state work on any
+ * channel at any time; a blob exported from a channel that has skipped calls continues bit for bit wherever it is imported.
+ * Grouping: the last subset's groups are kept and reused while its id list and the configuration stay the same, apart from
+ * those of the calls on every channel (alternating the two forms re-plans neither). */
+int sdr_batch_process_device_subset(sdr_batch_t *h, const uint32_t *channel_ids, uint32_t n_ids, const void *I, const void *Q,
+                                    size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks,
+                                    void *block_status, void *cuda_stream);
+int sdr_batch_process_host_subset(sdr_batch_t *h, const uint32_t *channel_ids, uint32_t n_ids, const void *I, const void *Q,
+                                  size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks,
+                                  void *block_status);
+/* ticketed like submit_host: sdr_batch_host_ticket() right after it names the call */
+int sdr_batch_submit_host_subset(sdr_batch_t *h, const uint32_t *channel_ids, uint32_t n_ids, const void *I, const void *Q,
+                                 size_t in_pitch, int in_fmt, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks,
+                                 void *block_status);
 
 /* Getters for `n` channels (ids == NULL: channels 0..n-1).  Synchronises the handle's last stream. */
 int sdr_batch_get_status(sdr_batch_t *h, const uint32_t *channel_ids, uint32_t n, sdr_channel_status *out);
