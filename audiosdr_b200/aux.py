@@ -5,7 +5,12 @@ include/sdr_aux.h (audiosdr_b200/libsdr_aux.so; CUDA only, no CPU fallback):
   IQGeneratorBatch   <-  class AudioIQgenerator        (AudioIQgenerator.h:49-107)
   GrabberBatch       <-  class AudioGrabberComplex256  (AudioGrabberComplex256.h:46-64)
 
-Channel selector: None = every channel, an int, or a sequence of ints.  Planes are int16 [n_channels, >= 128*n_blocks]."""
+Channel selector: None = every channel, an int, or a sequence of ints.  Planes are int16 [n_channels, >= 128*n_blocks].
+
+`channels=` on process / process_host advances only the listed channels (the reference's update() returns untouched when
+an input block is missing): the planes then have len(channels) rows, row i belonging to channels[i], and every other
+channel is left as it is (sdr_*_process_*_subset).  export_state / import_state move channels' whole state between
+handles as opaque blobs, uint8 [n, state_bytes]."""
 import ctypes as C
 import os
 
@@ -19,7 +24,11 @@ EXPORTS = ["sdr_preproc_create", "sdr_preproc_destroy", "sdr_preproc_set", "sdr_
            "sdr_iqgen_set_gain_balance", "sdr_iqgen_process_device", "sdr_iqgen_process_host", "sdr_iqgen_launch_count",
            "sdr_grabber_create", "sdr_grabber_destroy", "sdr_grabber_process_device", "sdr_grabber_new_data_available",
            "sdr_grabber_grab", "sdr_grabber_grab_device", "sdr_grabber_spectrum", "sdr_grabber_spectrum_device", "sdr_aux_last_error",
-           "sdr_aux_version"]
+           "sdr_aux_version",
+           "sdr_preproc_process_device_subset", "sdr_preproc_process_host_subset", "sdr_preproc_state_bytes", "sdr_preproc_export_state",
+           "sdr_preproc_import_state", "sdr_iqgen_process_device_subset", "sdr_iqgen_process_host_subset", "sdr_iqgen_state_bytes",
+           "sdr_iqgen_export_state", "sdr_iqgen_import_state", "sdr_grabber_process_device_subset", "sdr_grabber_state_bytes",
+           "sdr_grabber_export_state", "sdr_grabber_import_state"]
 
 
 class AuxError(RuntimeError):
@@ -69,6 +78,17 @@ def load_library(path=None):
     L.sdr_grabber_grab_device.argtypes = [vp, vp, vp]
     L.sdr_grabber_spectrum.argtypes = [vp, vp, u32, vp]
     L.sdr_grabber_spectrum_device.argtypes = [vp, vp, u32, vp, vp]
+    if hasattr(L, "sdr_preproc_process_device_subset"):  # absent from builds older than the subset calls (benchmark comparisons)
+        L.sdr_preproc_process_device_subset.argtypes = [vp, vp, u32, vp, vp, sz, vp, vp, sz, u32, vp]
+        L.sdr_preproc_process_host_subset.argtypes = [vp, vp, u32, vp, vp, sz, vp, vp, sz, u32]
+        L.sdr_iqgen_process_device_subset.argtypes = [vp, vp, u32, vp, sz, vp, vp, sz, u32, vp]
+        L.sdr_iqgen_process_host_subset.argtypes = [vp, vp, u32, vp, sz, vp, vp, sz, u32]
+        L.sdr_grabber_process_device_subset.argtypes = [vp, vp, u32, vp, vp, sz, u32, vp]
+        for k in ("preproc", "iqgen", "grabber"):
+            getattr(L, "sdr_%s_state_bytes" % k).restype = sz
+            getattr(L, "sdr_%s_state_bytes" % k).argtypes = []
+            getattr(L, "sdr_%s_export_state" % k).argtypes = [vp, vp, u32, vp]
+            getattr(L, "sdr_%s_import_state" % k).argtypes = [vp, vp, u32, vp]
     L.sdr_aux_last_error.restype = C.c_char_p
     L.sdr_aux_version.restype = C.c_char_p
     if path is None:
@@ -83,18 +103,50 @@ def _sel(channels):
     return arr.ctypes.data, len(arr), arr
 
 
-def _check_dev(n_channels, *ts):
+def _check_dev(n_rows, *ts):
     for t in ts:
-        assert t.shape[0] == n_channels and t.stride(1) == 1 and str(t.dtype) == "torch.int16" and t.is_cuda
+        assert t.shape[0] == n_rows and t.stride(1) == 1 and str(t.dtype) == "torch.int16" and t.is_cuda
+
+
+def _ids(channels, n_channels):
+    """(pointer, n_ids, keep-alive array, rows) of a subset call's id list; channels=None: every channel (NULL)."""
+    if channels is None:
+        return None, n_channels, None, n_channels
+    arr = np.ascontiguousarray(np.atleast_1d(np.asarray(channels)).astype(np.uint32))
+    return arr.ctypes.data, len(arr), arr, len(arr)
 
 
 class _Base:
+    _kind = None
+
     def _check(self, rc):
         if rc != 0:
             raise AuxError(self.L.sdr_aux_last_error().decode())
 
+    @property
+    def state_bytes(self):
+        return int(getattr(self.L, "sdr_%s_state_bytes" % self._kind)())
+
+    def export_state(self, channels=None):
+        """uint8 [n, state_bytes]: one opaque blob per channel (None: every channel)."""
+        p, n, keep = _sel(channels)
+        cnt = n if channels is not None else self.n_channels
+        out = np.zeros((cnt, self.state_bytes), np.uint8)
+        self._check(getattr(self.L, "sdr_%s_export_state" % self._kind)(self.h, p, cnt, out.ctypes.data))
+        return out
+
+    def import_state(self, channels, blobs):
+        """Loads blobs of export_state (of any handle of this library version) into the channels (None: 0..len(blobs)-1)."""
+        b = np.ascontiguousarray(blobs, np.uint8).reshape(-1, self.state_bytes)
+        p, n, keep = _sel(channels)
+        if channels is not None:
+            assert n == b.shape[0]
+        self._check(getattr(self.L, "sdr_%s_import_state" % self._kind)(self.h, p, b.shape[0], b.ctypes.data))
+
 
 class PreProcessorBatch(_Base):
+    _kind = "preproc"
+
     def __init__(self, n_channels, device=0, _lib=None):
         self.L = _lib or load_library()
         self.n_channels = int(n_channels)
@@ -138,22 +190,30 @@ class PreProcessorBatch(_Base):
         self._check(self.L.sdr_preproc_get_status(self.h, p, n, out))
         return list(out)
 
-    # ---- update() for every channel, n_blocks times
-    def process(self, I, Q, I_out, Q_out, n_blocks=None, stream=None):
+    # ---- update() for every channel (or the listed ones), n_blocks times
+    def process(self, I, Q, I_out, Q_out, n_blocks=None, stream=None, channels=None):
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
-        _check_dev(self.n_channels, I, Q, I_out, Q_out)
+        p, n, keep, rows = _ids(channels, self.n_channels)
+        _check_dev(rows, I, Q, I_out, Q_out)
         assert I.stride(0) == Q.stride(0) and I_out.stride(0) == Q_out.stride(0)
         sp = C.c_void_p(stream.cuda_stream) if stream is not None else None
-        self._check(self.L.sdr_preproc_process_device(self.h, I.data_ptr(), Q.data_ptr(), I.stride(0), I_out.data_ptr(), Q_out.data_ptr(),
-                                                      I_out.stride(0), n_blocks, sp))
+        args = (I.data_ptr(), Q.data_ptr(), I.stride(0), I_out.data_ptr(), Q_out.data_ptr(), I_out.stride(0), n_blocks, sp)
+        if channels is None:
+            self._check(self.L.sdr_preproc_process_device(self.h, *args))
+        else:
+            self._check(self.L.sdr_preproc_process_device_subset(self.h, p, n, *args))
 
-    def process_host(self, I, Q, I_out, Q_out, n_blocks=None):
+    def process_host(self, I, Q, I_out, Q_out, n_blocks=None, channels=None):
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
+        p, n, keep, rows = _ids(channels, self.n_channels)
         for a in (I, Q, I_out, Q_out):
-            assert a.dtype == np.int16 and a.shape[0] == self.n_channels and a.strides[1] == 2
+            assert a.dtype == np.int16 and a.shape[0] == rows and a.strides[1] == 2
         assert I.strides[0] == Q.strides[0] and I_out.strides[0] == Q_out.strides[0]
-        self._check(self.L.sdr_preproc_process_host(self.h, I.ctypes.data, Q.ctypes.data, I.strides[0] // 2, I_out.ctypes.data,
-                                                    Q_out.ctypes.data, I_out.strides[0] // 2, n_blocks))
+        args = (I.ctypes.data, Q.ctypes.data, I.strides[0] // 2, I_out.ctypes.data, Q_out.ctypes.data, I_out.strides[0] // 2, n_blocks)
+        if channels is None:
+            self._check(self.L.sdr_preproc_process_host(self.h, *args))
+        else:
+            self._check(self.L.sdr_preproc_process_host_subset(self.h, p, n, *args))
 
     @property
     def launch_count(self):
@@ -161,6 +221,8 @@ class PreProcessorBatch(_Base):
 
 
 class IQGeneratorBatch(_Base):
+    _kind = "iqgen"
+
     def __init__(self, n_channels, device=0, _lib=None):
         self.L = _lib or load_library()
         self.n_channels = int(n_channels)
@@ -179,21 +241,29 @@ class IQGeneratorBatch(_Base):
         p, n, keep = _sel(channels)
         self._check(self.L.sdr_iqgen_set_gain_balance(self.h, p, n, float(balance)))
 
-    def process(self, X, I_out, Q_out, n_blocks=None, stream=None):
+    def process(self, X, I_out, Q_out, n_blocks=None, stream=None, channels=None):
         n_blocks = int(n_blocks if n_blocks is not None else X.shape[1] // N_BLOCK)
-        _check_dev(self.n_channels, X, I_out, Q_out)
+        p, n, keep, rows = _ids(channels, self.n_channels)
+        _check_dev(rows, X, I_out, Q_out)
         assert I_out.stride(0) == Q_out.stride(0)
         sp = C.c_void_p(stream.cuda_stream) if stream is not None else None
-        self._check(self.L.sdr_iqgen_process_device(self.h, X.data_ptr(), X.stride(0), I_out.data_ptr(), Q_out.data_ptr(), I_out.stride(0),
-                                                    n_blocks, sp))
+        args = (X.data_ptr(), X.stride(0), I_out.data_ptr(), Q_out.data_ptr(), I_out.stride(0), n_blocks, sp)
+        if channels is None:
+            self._check(self.L.sdr_iqgen_process_device(self.h, *args))
+        else:
+            self._check(self.L.sdr_iqgen_process_device_subset(self.h, p, n, *args))
 
-    def process_host(self, X, I_out, Q_out, n_blocks=None):
+    def process_host(self, X, I_out, Q_out, n_blocks=None, channels=None):
         n_blocks = int(n_blocks if n_blocks is not None else X.shape[1] // N_BLOCK)
+        p, n, keep, rows = _ids(channels, self.n_channels)
         for a in (X, I_out, Q_out):
-            assert a.dtype == np.int16 and a.shape[0] == self.n_channels and a.strides[1] == 2
+            assert a.dtype == np.int16 and a.shape[0] == rows and a.strides[1] == 2
         assert I_out.strides[0] == Q_out.strides[0]
-        self._check(self.L.sdr_iqgen_process_host(self.h, X.ctypes.data, X.strides[0] // 2, I_out.ctypes.data, Q_out.ctypes.data,
-                                                  I_out.strides[0] // 2, n_blocks))
+        args = (X.ctypes.data, X.strides[0] // 2, I_out.ctypes.data, Q_out.ctypes.data, I_out.strides[0] // 2, n_blocks)
+        if channels is None:
+            self._check(self.L.sdr_iqgen_process_host(self.h, *args))
+        else:
+            self._check(self.L.sdr_iqgen_process_host_subset(self.h, p, n, *args))
 
     @property
     def launch_count(self):
@@ -201,7 +271,10 @@ class IQGeneratorBatch(_Base):
 
 
 class GrabberBatch(_Base):
-    """AudioGrabberComplex256 for n_channels: process() = update() x n_blocks, grab() = the last complete 256-sample snapshot."""
+    """AudioGrabberComplex256 for n_channels: process() = update() x n_blocks, grab() = the last complete 256-sample snapshot.
+    Each channel is one reference object: after calls on subsets, some channels may have a snapshot while others have none
+    yet; grab() and spectrum() then write only the rows of channels that have one (pass `out=` to keep the other rows)."""
+    _kind = "grabber"
 
     def __init__(self, n_channels, device=0, _lib=None):
         self.L = _lib or load_library()
@@ -216,12 +289,16 @@ class GrabberBatch(_Base):
 
     __del__ = close
 
-    def process(self, I, Q, n_blocks=None, stream=None):
+    def process(self, I, Q, n_blocks=None, stream=None, channels=None):
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
-        _check_dev(self.n_channels, I, Q)
+        p, n, keep, rows = _ids(channels, self.n_channels)
+        _check_dev(rows, I, Q)
         assert I.stride(0) == Q.stride(0)
         sp = C.c_void_p(stream.cuda_stream) if stream is not None else None
-        self._check(self.L.sdr_grabber_process_device(self.h, I.data_ptr(), Q.data_ptr(), I.stride(0), n_blocks, sp))
+        if channels is None:
+            self._check(self.L.sdr_grabber_process_device(self.h, I.data_ptr(), Q.data_ptr(), I.stride(0), n_blocks, sp))
+        else:
+            self._check(self.L.sdr_grabber_process_device_subset(self.h, p, n, I.data_ptr(), Q.data_ptr(), I.stride(0), n_blocks, sp))
 
     def newDataAvailable(self, channel):
         r = self.L.sdr_grabber_new_data_available(self.h, int(channel))
@@ -229,12 +306,15 @@ class GrabberBatch(_Base):
             self._check(r)
         return bool(r)
 
-    def spectrum(self, channels=None):
+    def spectrum(self, channels=None, out=None):
         """float32 [n, 256]: power per bin of the 256-point FFT of each channel's snapshot (natural bin order), or None while
-        no snapshot is valid.  A view of the snapshot: the new-data flags stay as they are."""
+        no listed channel has a snapshot.  Rows of channels without one are not written (zeros, or what `out` held).  A view
+        of the snapshot: the new-data flags stay as they are."""
         p, n, keep = _sel(channels)
         cnt = n if channels is not None else self.n_channels
-        out = np.empty((cnt, 256), np.float32)
+        if out is None:
+            out = np.zeros((cnt, 256), np.float32)
+        assert out.dtype == np.float32 and out.shape == (cnt, 256) and out.flags.c_contiguous
         r = self.L.sdr_grabber_spectrum(self.h, p, n, out.ctypes.data)
         if r < 0:
             self._check(r)
@@ -249,12 +329,15 @@ class GrabberBatch(_Base):
             self._check(r)
         return r > 0
 
-    def grab(self, channels=None):
-        """int16 [n, 512] (re, im interleaved) or None while no pair of blocks has completed (the reference's grab() then
-        leaves the destination untouched)."""
+    def grab(self, channels=None, out=None):
+        """int16 [n, 512] (re, im interleaved) or None while no listed channel has completed a pair of blocks.  The reference's
+        grab() leaves the destination untouched before the first complete pair: rows of such channels are not written
+        (zeros, or what `out` held).  Clears the listed channels' new-data flags."""
         p, n, keep = _sel(channels)
         cnt = n if channels is not None else self.n_channels
-        out = np.empty((cnt, 512), np.int16)
+        if out is None:
+            out = np.zeros((cnt, 512), np.int16)
+        assert out.dtype == np.int16 and out.shape == (cnt, 512) and out.flags.c_contiguous
         r = self.L.sdr_grabber_grab(self.h, p, n, out.ctypes.data)
         if r < 0:
             self._check(r)

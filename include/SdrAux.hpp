@@ -6,12 +6,15 @@
  *
  * Every public method of the reference keeps its name and argument meaning with a channel selector in front
  * (sdr::Channels from SdrBatch.hpp: one id, a vector of ids, or sdr::all); update() becomes process() over int16 planes.
+ * process(ids, ...) advances only the listed channels, on compact planes (row i = channel ids[i]); export_state /
+ * import_state move channels' whole state as opaque blobs of state_bytes() bytes each (sdr_aux.h).
  * Header only; link against audiosdr_b200/libsdr_aux.so.  Errors of the C ABI become std::runtime_error.
  */
 #ifndef SDR_AUX_HPP
 #define SDR_AUX_HPP
 #include <stdexcept>
 #include <string>
+#include <vector>
 
 #include "SdrBatch.hpp"
 #include "sdr_aux.h"
@@ -44,6 +47,27 @@ class PreProcessorBatch {
   void process_host(const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks) {
     check(sdr_preproc_process_host(h_, I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks), "sdr_preproc_process_host");
   }
+  /* the listed channels only; every other channel skips the call untouched */
+  void process(const std::vector<uint32_t> &ids, const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out, int16_t *Q_out,
+               size_t out_pitch, uint32_t n_blocks, void *cuda_stream = nullptr) {
+    check(sdr_preproc_process_device_subset(h_, ids.data(), (uint32_t)ids.size(), I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, cuda_stream),
+          "sdr_preproc_process_device_subset");
+  }
+  void process_host(const std::vector<uint32_t> &ids, const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out, int16_t *Q_out,
+                    size_t out_pitch, uint32_t n_blocks) {
+    check(sdr_preproc_process_host_subset(h_, ids.data(), (uint32_t)ids.size(), I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks),
+          "sdr_preproc_process_host_subset");
+  }
+  static size_t state_bytes() { return sdr_preproc_state_bytes(); }
+  std::vector<uint8_t> export_state(const std::vector<uint32_t> &ids) {
+    std::vector<uint8_t> b(ids.size() * state_bytes());
+    check(sdr_preproc_export_state(h_, ids.data(), (uint32_t)ids.size(), b.data()), "sdr_preproc_export_state");
+    return b;
+  }
+  void import_state(const std::vector<uint32_t> &ids, const std::vector<uint8_t> &blobs) {
+    if (blobs.size() != ids.size() * state_bytes()) throw std::runtime_error("import_state: one blob per channel");
+    check(sdr_preproc_import_state(h_, ids.data(), (uint32_t)ids.size(), blobs.data()), "sdr_preproc_import_state");
+  }
   sdr_preproc_t *handle() { return h_; }
 
  private:
@@ -69,6 +93,26 @@ class IQGeneratorBatch {
   void process_host(const int16_t *X, size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks) {
     check(sdr_iqgen_process_host(h_, X, in_pitch, I_out, Q_out, out_pitch, n_blocks), "sdr_iqgen_process_host");
   }
+  void process(const std::vector<uint32_t> &ids, const int16_t *X, size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch,
+               uint32_t n_blocks, void *cuda_stream = nullptr) {
+    check(sdr_iqgen_process_device_subset(h_, ids.data(), (uint32_t)ids.size(), X, in_pitch, I_out, Q_out, out_pitch, n_blocks, cuda_stream),
+          "sdr_iqgen_process_device_subset");
+  }
+  void process_host(const std::vector<uint32_t> &ids, const int16_t *X, size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch,
+                    uint32_t n_blocks) {
+    check(sdr_iqgen_process_host_subset(h_, ids.data(), (uint32_t)ids.size(), X, in_pitch, I_out, Q_out, out_pitch, n_blocks),
+          "sdr_iqgen_process_host_subset");
+  }
+  static size_t state_bytes() { return sdr_iqgen_state_bytes(); }
+  std::vector<uint8_t> export_state(const std::vector<uint32_t> &ids) {
+    std::vector<uint8_t> b(ids.size() * state_bytes());
+    check(sdr_iqgen_export_state(h_, ids.data(), (uint32_t)ids.size(), b.data()), "sdr_iqgen_export_state");
+    return b;
+  }
+  void import_state(const std::vector<uint32_t> &ids, const std::vector<uint8_t> &blobs) {
+    if (blobs.size() != ids.size() * state_bytes()) throw std::runtime_error("import_state: one blob per channel");
+    check(sdr_iqgen_import_state(h_, ids.data(), (uint32_t)ids.size(), blobs.data()), "sdr_iqgen_import_state");
+  }
   sdr_iqgen_t *handle() { return h_; }
 
  private:
@@ -88,6 +132,19 @@ class GrabberBatch {
   /* update() for every channel, n_blocks blocks each; device planes */
   void process(const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, void *cuda_stream = nullptr) {
     check(sdr_grabber_process_device(h_, I, Q, pitch, n_blocks, cuda_stream), "sdr_grabber_process_device");
+  }
+  void process(const std::vector<uint32_t> &ids, const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, void *cuda_stream = nullptr) {
+    check(sdr_grabber_process_device_subset(h_, ids.data(), (uint32_t)ids.size(), I, Q, pitch, n_blocks, cuda_stream), "sdr_grabber_process_device_subset");
+  }
+  static size_t state_bytes() { return sdr_grabber_state_bytes(); }
+  std::vector<uint8_t> export_state(const std::vector<uint32_t> &ids) {
+    std::vector<uint8_t> b(ids.size() * state_bytes());
+    check(sdr_grabber_export_state(h_, ids.data(), (uint32_t)ids.size(), b.data()), "sdr_grabber_export_state");
+    return b;
+  }
+  void import_state(const std::vector<uint32_t> &ids, const std::vector<uint8_t> &blobs) {
+    if (blobs.size() != ids.size() * state_bytes()) throw std::runtime_error("import_state: one blob per channel");
+    check(sdr_grabber_import_state(h_, ids.data(), (uint32_t)ids.size(), blobs.data()), "sdr_grabber_import_state");
   }
   bool newDataAvailable(uint32_t c) { const int r = sdr_grabber_new_data_available(h_, c); if (r < 0) check(r, "sdr_grabber_new_data_available"); return r != 0; }
   /* grab(destination) of one channel: 512 int16 to host memory; false (destination untouched) before the first complete pair */

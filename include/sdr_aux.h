@@ -9,6 +9,25 @@
  * pitch in elements.  Base pointers must be 16-byte aligned and pitches multiples of 8.  Output planes must not overlap the
  * input planes (the reference works in place on one block; a batched one-sample shift cannot).  Each process call advances
  * every channel by n_blocks blocks of 128 samples; all per-channel state lives in device memory between calls.
+ *
+ * Calls on a subset of the channels (*_subset): each class's update() starts by taking its input block(s) and returns
+ * without touching any member when one is missing, as AudioSDR::update() does (AudioSDR.cpp:48-56).  For these three
+ * classes the cited ranges are those of the whole update() (AudioSDRpreProcessor.cpp:46-138, AudioIQgenerator.cpp:33-87,
+ * AudioGrabberComplex256.cpp:50-72); the exact lines of the early return are unchecked.  So in a graph some objects skip
+ * a block period while others run.  The rules are those of sdr_batch_process_device_subset
+ * (sdr_batch.h), so that one id list drives the whole graph:
+ *   channel_ids  host memory, read before the call returns; distinct ids below n_channels, n_ids >= 1.  NULL (with
+ *                n_ids == n_channels) is the call on every channel: the plain entry points are these calls with NULL.
+ *                Anything else returns SDR_AUX_EINVAL and queues nothing: no state changes, no output is written.
+ *   planes       compact: row i of every plane belongs to channel channel_ids[i] (n_ids rows, ids in any order).
+ * Every unlisted channel is untouched and its next processed block continues its own stream; a channel's output over any
+ * sequence of calls is the reference run on that channel's own blocks, concatenated.  Setters on an unlisted channel take
+ * effect before that channel's next processed block.
+ *
+ * Checkpoint / migration (*_state_bytes, *_export_state, *_import_state): a channel's whole carry-over as one opaque blob
+ * of *_state_bytes() bytes (channel_ids == NULL: channels 0..n-1).  A blob imports into any channel of any handle of the
+ * same block and library version -- another GPU, a handle that has run a different number of blocks -- and the stream
+ * continues bit for bit.  Both calls synchronise the device.
  * All functions return 0 (SDR_AUX_OK) or a negative error; sdr_aux_last_error() gives the text (thread local).
  */
 #ifndef SDR_AUX_H
@@ -52,7 +71,19 @@ int sdr_preproc_process_device(sdr_preproc_t *h, const int16_t *I, const int16_t
 /* ... host planes: copies in, runs, copies out, returns when the outputs are in host memory */
 int sdr_preproc_process_host(sdr_preproc_t *h, const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out,
                              int16_t *Q_out, size_t out_pitch, uint32_t n_blocks);
+/* the same on the n_ids channels channel_ids[0..n_ids) (rules at the top of this file) */
+int sdr_preproc_process_device_subset(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+                                      size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks,
+                                      void *cuda_stream);
+int sdr_preproc_process_host_subset(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+                                    size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks);
 uint64_t sdr_preproc_launch_count(const sdr_preproc_t *h);
+/* Blob: the PP.h:66-72 members (correction, savedSample, both detector counters, swap, detector flag).  Export applies queued
+ * setters first, as get_status does; import replaces the channel's state including setters queued for it, and setters
+ * called after the import apply on top of it. */
+size_t sdr_preproc_state_bytes(void);
+int sdr_preproc_export_state(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n, void *blobs);
+int sdr_preproc_import_state(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n, const void *blobs);
 
 /* ---------------------------------------------------------------- I/Q generator ---- */
 typedef struct sdr_iqgen sdr_iqgen_t;
@@ -66,7 +97,15 @@ int sdr_iqgen_process_device(sdr_iqgen_t *h, const int16_t *X, size_t in_pitch, 
                              size_t out_pitch, uint32_t n_blocks, void *cuda_stream);
 int sdr_iqgen_process_host(sdr_iqgen_t *h, const int16_t *X, size_t in_pitch, int16_t *I_out, int16_t *Q_out,
                            size_t out_pitch, uint32_t n_blocks);
+int sdr_iqgen_process_device_subset(sdr_iqgen_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *X, size_t in_pitch,
+                                    int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks, void *cuda_stream);
+int sdr_iqgen_process_host_subset(sdr_iqgen_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *X, size_t in_pitch,
+                                  int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks);
 uint64_t sdr_iqgen_launch_count(const sdr_iqgen_t *h);
+/* Blob: the last 256 input samples (the filter's history, IQ.cpp:37-38) and (gainI, gainQ) */
+size_t sdr_iqgen_state_bytes(void);
+int sdr_iqgen_export_state(sdr_iqgen_t *h, const uint32_t *channel_ids, uint32_t n, void *blobs);
+int sdr_iqgen_import_state(sdr_iqgen_t *h, const uint32_t *channel_ids, uint32_t n, const void *blobs);
 
 /* ---------------------------------------------------------------- complex snapshot grabber ---- */
 /* replaces class AudioGrabberComplex256 (AudioGrabberComplex256.h:46-64): every update() appends one block of interleaved
@@ -78,21 +117,33 @@ int sdr_grabber_create(sdr_grabber_t **out, uint32_t n_channels, int device);
 void sdr_grabber_destroy(sdr_grabber_t *h);
 /* AudioGrabberComplex256::update() for every channel, n_blocks times; device planes as for the pre-processor */
 int sdr_grabber_process_device(sdr_grabber_t *h, const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, void *cuda_stream);
+/* the same on the n_ids channels channel_ids[0..n_ids).  Each channel keeps its own pair phase, _dataBufferValid and
+ * new-data flag, so after calls on subsets the channels differ in all three. */
+int sdr_grabber_process_device_subset(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+                                      size_t pitch, uint32_t n_blocks, void *cuda_stream);
 /* newDataAvailable() of one channel: 1 / 0, negative on error */
 int sdr_grabber_new_data_available(sdr_grabber_t *h, uint32_t channel);
 /* grab() for the listed channels (NULL: all): 512 int16 per channel = 256 complex samples, to HOST memory
- * dest[i*512 .. i*512+511].  Before the first complete pair nothing is written (the reference's _dataBufferValid), and the
- * call still clears the channels' new-data flags.  Returns the number of channels written, negative on error. */
+ * dest[i*512 .. i*512+511].  A channel before its first complete pair has no snapshot (the reference's _dataBufferValid):
+ * its row is not written.  The call clears every listed channel's new-data flag.  Returns the number of rows written,
+ * negative on error. */
 int sdr_grabber_grab(sdr_grabber_t *h, const uint32_t *channels, uint32_t n, int16_t *dest);
-/* all channels, device to device: dest[n_channels][512]; returns 0 when nothing was valid yet, 1 when written */
+/* all channels, device to device: dest[n_channels][512], rows of channels without a snapshot not written; clears every
+ * new-data flag; returns 1 when some row was written, 0 when none */
 int sdr_grabber_grab_device(sdr_grabber_t *h, int16_t *dest, void *cuda_stream);
+/* Blob: the carried first block of an incomplete pair, the snapshot, the channel's pair phase, _dataBufferValid and the
+ * new-data flag */
+size_t sdr_grabber_state_bytes(void);
+int sdr_grabber_export_state(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n, void *blobs);
+int sdr_grabber_import_state(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n, const void *blobs);
 
 /* Spectrum tap on the snapshots -- what the consumer of grab() does with them (the sketch's panadapter / S-meter; not part
  * of the library classes, SURVEY 8f row 3): the 256-point forward complex FFT of a channel's snapshot, samples taken as
  * floats (re, im) = (float)int16, and the power re^2 + im^2 per bin, natural bin order (bin k = k * 44100/256 Hz, bins 128..255
- * = negative frequencies).  power[i*256 + k] for the i-th listed channel (NULL: all channels).  Returns the number of
- * channels written (host form) / 1 (device form), 0 while no snapshot is valid yet, negative on error; the new-data flags
- * are left alone (a spectrum is a view of the snapshot, not a grab()). */
+ * = negative frequencies).  power[i*256 + k] for the i-th listed channel (NULL: all channels); rows of channels without a
+ * snapshot yet are not written.  Returns the number of rows written (host form) / 1 when some row was written (device
+ * form), 0 when none, negative on error; the new-data flags are left alone (a spectrum is a view of the snapshot, not a
+ * grab()). */
 int sdr_grabber_spectrum(sdr_grabber_t *h, const uint32_t *channels, uint32_t n, float *power);
 int sdr_grabber_spectrum_device(sdr_grabber_t *h, const uint32_t *d_channels, uint32_t n, float *d_power, void *cuda_stream);
 
