@@ -28,7 +28,7 @@ EXPORTS = ["sdr_preproc_create", "sdr_preproc_destroy", "sdr_preproc_set", "sdr_
            "sdr_preproc_process_device_subset", "sdr_preproc_process_host_subset", "sdr_preproc_state_bytes", "sdr_preproc_export_state",
            "sdr_preproc_import_state", "sdr_iqgen_process_device_subset", "sdr_iqgen_process_host_subset", "sdr_iqgen_state_bytes",
            "sdr_iqgen_export_state", "sdr_iqgen_import_state", "sdr_grabber_process_device_subset", "sdr_grabber_state_bytes",
-           "sdr_grabber_export_state", "sdr_grabber_import_state"]
+           "sdr_grabber_export_state", "sdr_grabber_import_state", "sdr_grabber_process_device_snapshots"]
 
 
 class AuxError(RuntimeError):
@@ -89,6 +89,8 @@ def load_library(path=None):
             getattr(L, "sdr_%s_state_bytes" % k).argtypes = []
             getattr(L, "sdr_%s_export_state" % k).argtypes = [vp, vp, u32, vp]
             getattr(L, "sdr_%s_import_state" % k).argtypes = [vp, vp, u32, vp]
+    if hasattr(L, "sdr_grabber_process_device_snapshots"):
+        L.sdr_grabber_process_device_snapshots.argtypes = [vp, vp, u32, vp, vp, sz, u32, vp, vp, vp, vp]
     L.sdr_aux_last_error.restype = C.c_char_p
     L.sdr_aux_version.restype = C.c_char_p
     if path is None:
@@ -289,12 +291,25 @@ class GrabberBatch(_Base):
 
     __del__ = close
 
-    def process(self, I, Q, n_blocks=None, stream=None, channels=None):
+    def process(self, I, Q, n_blocks=None, stream=None, channels=None, snapshots=None, power=None):
+        """update() x n_blocks on every channel (or the listed ones).  snapshots (CUDA int16 [rows, S, 512]) and/or power
+        (CUDA float32 [rows, S, 256]), S = (n_blocks + 1) // 2: every snapshot the call publishes and its spectrum, slot k of
+        row i = the k-th pair the call completes for that row's channel (sdr_grabber_process_device_snapshots).  Then returns
+        counts, numpy uint32 [rows]: the slots written per row."""
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
         p, n, keep, rows = _ids(channels, self.n_channels)
         _check_dev(rows, I, Q)
         assert I.stride(0) == Q.stride(0)
         sp = C.c_void_p(stream.cuda_stream) if stream is not None else None
+        if snapshots is not None or power is not None:
+            S = (n_blocks + 1) // 2
+            for t, dt, w in ((snapshots, "torch.int16", 512), (power, "torch.float32", 256)):
+                assert t is None or (t.is_cuda and str(t.dtype) == dt and tuple(t.shape) == (rows, S, w) and t.is_contiguous())
+            counts = np.zeros(rows, np.uint32)
+            self._check(self.L.sdr_grabber_process_device_snapshots(
+                self.h, p, rows, I.data_ptr(), Q.data_ptr(), I.stride(0), n_blocks, snapshots.data_ptr() if snapshots is not None else None,
+                power.data_ptr() if power is not None else None, counts.ctypes.data, sp))
+            return counts
         if channels is None:
             self._check(self.L.sdr_grabber_process_device(self.h, I.data_ptr(), Q.data_ptr(), I.stride(0), n_blocks, sp))
         else:

@@ -495,6 +495,157 @@ __global__ void __launch_bounds__(GRAB_THREADS) grab_update_kernel(const GrabLau
   }
 }
 
+/* ---- 256-point FFT + power, one warp per snapshot (the per-pair snapshots of a process call and the spectrum tap).
+ * The operation network is the radix-2 decimation-in-frequency one the test suite's checker restates (aux_cfft256_forward), one
+ * rounding per operation (-fmad=false), twiddles from c_fft_tw256, power re*re + im*im in natural bin order: only the data
+ * movement differs.  A lane holds 8 complex points; point index bits b7..b0.  Three register layouts, one per group of
+ * three stages, with a warp-local shared-memory transpose between them:
+ *   L0: lane = b7..b3, register r = b2..b0 (idx = 8 lane + r)      load (16-byte rows), stages 2 and 1, power
+ *   LA: lane = b4..b0, r = b7..b5 (idx = 32 r + lane)               stages 128, 64, 32
+ *   LB: lane = (b7..b5, b1 b0), r = b4..b2                          stages 16, 8, 4
+ * In L0 bin brev8(idx) = brev3(r) * 32 + brev5(lane): each register's power store covers one 128-byte line.
+ * fft_swz: a word address with idx's low 5 bits XORed by G(b7..b5) = (x << 2) | (x >> 1), which makes the 32 lanes of every
+ * layout's access hit 32 distinct banks. */
+#define FFT_WARP_WORDS 512 /* re[256], im[256] */
+__device__ __forceinline__ int fft_swz(int idx) { const int x = idx >> 5; return (idx & 0xE0) | ((idx & 31) ^ ((x << 2) | (x >> 1))); }
+
+struct FftTw { /* the lane's twiddles of stages 128 .. 4 (stages 2 and 1 use warp-uniform entries) */
+  float2 a128[4], a64[2], a32, b16[4], b8[2], b4;
+};
+__device__ __forceinline__ float2 fft_tw(int k) { return make_float2(c_fft_tw256[2 * k], c_fft_tw256[2 * k + 1]); }
+__device__ __forceinline__ void fft_load_tw(FftTw &t, int l) {
+#pragma unroll
+  for (int r = 0; r < 4; r++) t.a128[r] = fft_tw(32 * r + l);     /* j = 32 r + l, step 1 */
+#pragma unroll
+  for (int r = 0; r < 2; r++) t.a64[r] = fft_tw(2 * (32 * r + l)); /* j = 32 (r & 1) + l, step 2 */
+  t.a32 = fft_tw(4 * l);                                            /* j = l, step 4 */
+#pragma unroll
+  for (int r = 0; r < 4; r++) t.b16[r] = fft_tw(8 * (4 * r + (l & 3)));  /* j = 4 r + b1b0, step 8 */
+#pragma unroll
+  for (int r = 0; r < 2; r++) t.b8[r] = fft_tw(16 * (4 * r + (l & 3))); /* j = 4 (r & 1) + b1b0, step 16 */
+  t.b4 = fft_tw(32 * (l & 3));                                            /* j = b1b0, step 32 */
+}
+
+/* aux_cfft256_forward's butterfly: a' = a + b, b' = (a - b) * w, each product and sum rounded on its own */
+__device__ __forceinline__ void fft_bfly(float &ar, float &ai, float &br, float &bi, const float2 w) {
+  const float tr = ar - br, ti = ai - bi;
+  ar = ar + br;
+  ai = ai + bi;
+  const float p0 = tr * w.x, p1 = ti * w.y, p2 = tr * w.y, p3 = ti * w.x;
+  br = p0 - p1;
+  bi = p2 + p3;
+}
+
+/* registers of layout `from` -> shared memory -> registers of the next layout (idx_w(r), idx_r(r): the points written and read) */
+#define FFT_TRANSPOSE(IDX_W, IDX_R)                                                          \
+  do {                                                                                       \
+    __syncwarp();                                                                            \
+    _Pragma("unroll") for (int r = 0; r < 8; r++) { sr[fft_swz(IDX_W)] = xr[r]; si[fft_swz(IDX_W)] = xi[r]; } \
+    __syncwarp();                                                                            \
+    _Pragma("unroll") for (int r = 0; r < 8; r++) { xr[r] = sr[fft_swz(IDX_R)]; xi[r] = si[fft_swz(IDX_R)]; } \
+  } while (0)
+
+/* w[i]: point 8 l + i as (re | im << 16), layout L0.  power[256] of the snapshot (natural bin order) to `out`.  sm: the
+ * warp's FFT_WARP_WORDS words of shared memory. */
+__device__ __forceinline__ void fft256_power(const uint32_t w[8], float *sm, const FftTw &t, int l, float *out) {
+  float *sr = sm, *si = sm + 256;
+  float xr[8], xi[8];
+#pragma unroll
+  for (int r = 0; r < 8; r++) { xr[r] = (float)(int16_t)(w[r] & 0xFFFFu); xi[r] = (float)((int)w[r] >> 16); }
+  FFT_TRANSPOSE(8 * l + r, 32 * r + l); /* L0 -> LA */
+#pragma unroll
+  for (int r = 0; r < 4; r++) fft_bfly(xr[r], xi[r], xr[r + 4], xi[r + 4], t.a128[r]);
+#pragma unroll
+  for (int r = 0; r < 8; r++) if (!(r & 2)) fft_bfly(xr[r], xi[r], xr[r + 2], xi[r + 2], t.a64[r & 1]);
+#pragma unroll
+  for (int r = 0; r < 8; r += 2) fft_bfly(xr[r], xi[r], xr[r + 1], xi[r + 1], t.a32);
+  FFT_TRANSPOSE(32 * r + l, 32 * (l >> 2) + 4 * r + (l & 3)); /* LA -> LB */
+#pragma unroll
+  for (int r = 0; r < 4; r++) fft_bfly(xr[r], xi[r], xr[r + 4], xi[r + 4], t.b16[r]);
+#pragma unroll
+  for (int r = 0; r < 8; r++) if (!(r & 2)) fft_bfly(xr[r], xi[r], xr[r + 2], xi[r + 2], t.b8[r & 1]);
+#pragma unroll
+  for (int r = 0; r < 8; r += 2) fft_bfly(xr[r], xi[r], xr[r + 1], xi[r + 1], t.b4);
+  FFT_TRANSPOSE(32 * (l >> 2) + 4 * r + (l & 3), 8 * l + r); /* LB -> L0 */
+#pragma unroll
+  for (int r = 0; r < 8; r++) if (!(r & 2)) fft_bfly(xr[r], xi[r], xr[r + 2], xi[r + 2], fft_tw(64 * (r & 1))); /* j = b0, step 64 */
+#pragma unroll
+  for (int r = 0; r < 8; r += 2) fft_bfly(xr[r], xi[r], xr[r + 1], xi[r + 1], fft_tw(0));
+  const int col = (int)(__brev((unsigned)l) >> 27);
+#pragma unroll
+  for (int r = 0; r < 8; r++) {
+    const int row = ((r & 1) << 2) | (r & 2) | (r >> 2); /* brev3 */
+    const float a = xr[r] * xr[r], b = xi[r] * xi[r];
+    out[row * 32 + col] = a + b;
+  }
+}
+
+/* 8 samples of each rail (16-byte loads) -> 8 points (re | im << 16) */
+__device__ __forceinline__ void grab_interleave8(const int16_t *I, const int16_t *Q, uint32_t w[8]) {
+  const uint4 a = __ldg(reinterpret_cast<const uint4 *>(I)), b = __ldg(reinterpret_cast<const uint4 *>(Q));
+  const uint32_t ai[4] = {a.x, a.y, a.z, a.w}, bi[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+  for (int i = 0; i < 4; i++) { w[2 * i] = __byte_perm(ai[i], bi[i], 0x5410); w[2 * i + 1] = __byte_perm(ai[i], bi[i], 0x7632); }
+}
+
+#define FFT_THREADS 256
+/* Every snapshot a process call publishes (sdr_grabber_process_device_snapshots), launched before grab_update_kernel on the
+ * call's stream: it only reads the grabber's state (pair phase, carried half).  Item = (row, slot), row-major over
+ * n_rows x S, S = (n_blocks + 1) / 2; one warp per item, grid-stride.  Slot k of a row whose channel has pair phase p is the
+ * pair the call's block e = 2k + 1 - p completes: blocks e - 1 and e, block -1 being the carried half; slots k >=
+ * (p + n_blocks) / 2 do not exist and are not written.  Lane l holds points 8 l .. 8 l + 7: lanes 0-15 the first block, lanes
+ * 16-31 the second. */
+__global__ void __launch_bounds__(FFT_THREADS) grab_snapshots_kernel(const GrabLaunch L, int16_t *snaps, float *power) {
+  __shared__ float sm[FFT_THREADS / 32][FFT_WARP_WORDS];
+  const int l = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  FftTw t;
+  if (power) fft_load_tw(t, l);
+  const uint32_t S = (L.n_blocks + 1) / 2;
+  const unsigned long long items = (unsigned long long)L.n_rows * S, nw = (unsigned long long)gridDim.x * (FFT_THREADS / 32);
+  for (unsigned long long it = (unsigned long long)blockIdx.x * (FFT_THREADS / 32) + wib; it < items; it += nw) {
+    const uint32_t r = (uint32_t)(it / S), k = (uint32_t)(it - (unsigned long long)r * S);
+    const uint32_t ch = L.ids ? __ldg(L.ids + r) : r;
+    const int p = (int)L.phase[ch];
+    if (k >= (p + L.n_blocks) / 2) continue; /* uniform over the warp */
+    const int e = 2 * (int)k + 1 - p, blk = l < 16 ? e - 1 : e, s8 = 8 * (l & 15);
+    uint32_t w[8];
+    if (blk < 0) {
+      const uint4 *c = reinterpret_cast<const uint4 *>(L.half + (size_t)ch * 256 + 2 * s8);
+      const uint4 u = c[0], v = c[1];
+      w[0] = u.x; w[1] = u.y; w[2] = u.z; w[3] = u.w; w[4] = v.x; w[5] = v.y; w[6] = v.z; w[7] = v.w;
+    } else {
+      const size_t off = (size_t)r * L.pitch + (size_t)blk * 128 + s8;
+      grab_interleave8(L.I + off, L.Q + off, w);
+    }
+    if (snaps) {
+      uint4 *d = reinterpret_cast<uint4 *>(snaps + it * 512 + 16 * l);
+      d[0] = make_uint4(w[0], w[1], w[2], w[3]);
+      d[1] = make_uint4(w[4], w[5], w[6], w[7]);
+    }
+    if (power) fft256_power(w, sm[wib], t, l, power + it * 256);
+  }
+}
+
+/* Spectrum tap on the snapshots (SURVEY 8f row 3: the panadapter that consumes grab(); sdr_grabber_spectrum[_device]): power
+ * row i <- the 256-point forward complex FFT of channel channels[i]'s snapshot (NULL: i), (re, im) int16 pairs taken as
+ * floats, power re^2 + im^2 per bin in natural bin order, on the warp core above.  valid != NULL (while some channels have no
+ * snapshot yet): rows of those channels are not written.  One warp per row, grid-stride. */
+__global__ void __launch_bounds__(FFT_THREADS) grab_spectrum_kernel(const int16_t *snap, const uint32_t *channels, const uint8_t *valid,
+                                                                    uint32_t n, float *power) {
+  __shared__ float sm[FFT_THREADS / 32][FFT_WARP_WORDS];
+  const int l = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  FftTw t;
+  fft_load_tw(t, l);
+  for (uint32_t i = blockIdx.x * (FFT_THREADS / 32) + wib; i < n; i += gridDim.x * (FFT_THREADS / 32)) {
+    const uint32_t ch = channels ? __ldg(channels + i) : i;
+    if (valid && !valid[ch]) continue; /* uniform over the warp */
+    const uint4 *s = reinterpret_cast<const uint4 *>(snap + (size_t)ch * 512 + 16 * l);
+    const uint4 u = s[0], v = s[1];
+    const uint32_t w[8] = {u.x, u.y, u.z, u.w, v.x, v.y, v.z, v.w};
+    fft256_power(w, sm[wib], t, l, power + (size_t)i * 256);
+  }
+}
+
 /* ================================================================== host side ==== */
 static thread_local std::string g_err;
 static int fail(int code, const std::string &m) { g_err = m; return code; }
@@ -954,46 +1105,6 @@ extern "C" int sdr_iqgen_import_state(sdr_iqgen_t *h, const uint32_t *channel_id
   return 0;
 }
 
-/* Spectrum tap on the snapshots (SURVEY 8f row 3: the panadapter that consumes grab()): per channel the 256-point forward
- * complex FFT of the snapshot's (re, im) int16 pairs taken as floats, then the power re^2 + im^2 of every bin in natural bin
- * order.  One CTA = one channel, 128 threads = the 128 butterflies of a stage; the operation network is the radix-2
- * decimation-in-frequency one the test suite's checker restates (aux_cfft256_forward), one rounding per operation.
- * valid != NULL (the twin used while some channels have no snapshot yet): the rows of those channels are not written. */
-template <bool SKIP>
-__device__ __forceinline__ void grab_spectrum_body(const int16_t *snap, const uint32_t *channels, const uint8_t *valid, float *power) {
-  __shared__ float2 buf[256];
-  const uint32_t ch = channels ? channels[blockIdx.x] : blockIdx.x;
-  if (SKIP && !valid[ch]) return; /* uniform over the CTA */
-  const int t = threadIdx.x;
-  const int2 raw = reinterpret_cast<const int2 *>(snap + (size_t)ch * 512)[t]; /* samples 2t, 2t+1: (re, im, re, im) */
-  buf[2 * t] = make_float2((float)(int16_t)(raw.x & 0xFFFF), (float)(int16_t)(raw.x >> 16));
-  buf[2 * t + 1] = make_float2((float)(int16_t)(raw.y & 0xFFFF), (float)(int16_t)(raw.y >> 16));
-  __syncthreads();
-#pragma unroll 1
-  for (int half = 128; half >= 1; half >>= 1) {
-    const int step = 128 / half, j = t & (half - 1), ia = ((t / half) * 2 * half) + j, ib = ia + half;
-    const float2 a = buf[ia], b = buf[ib];
-    const float tr = a.x - b.x, ti = a.y - b.y;
-    const float wr = c_fft_tw256[2 * j * step], wi = c_fft_tw256[2 * j * step + 1];
-    const float p0 = tr * wr, p1 = ti * wi, p2 = tr * wi, p3 = ti * wr;
-    buf[ia] = make_float2(a.x + b.x, a.y + b.y);
-    buf[ib] = make_float2(p0 - p1, p2 + p3);
-    __syncthreads();
-  }
-#pragma unroll
-  for (int k = t; k < 256; k += 128) {
-    const float2 v = buf[__brev((unsigned)k) >> 24]; /* 8-bit reversal: natural bin order */
-    const float a = v.x * v.x, b = v.y * v.y;
-    power[(size_t)blockIdx.x * 256 + k] = a + b;
-  }
-}
-__global__ void __launch_bounds__(128) grab_spectrum_kernel(const int16_t *snap, const uint32_t *channels, float *power) {
-  grab_spectrum_body<false>(snap, channels, nullptr, power);
-}
-__global__ void __launch_bounds__(128) grab_spectrum_valid_kernel(const int16_t *snap, const uint32_t *channels, const uint8_t *valid, float *power) {
-  grab_spectrum_body<true>(snap, channels, valid, power);
-}
-
 /* ------------------------------------------------------------------ grabber ---- */
 /* Each channel is one reference object with its own pair phase, _dataBufferValid and _newDataIsAvailable: calls on subsets
  * of the channels leave them in different states.  The device holds phase and validity for the kernels (grab_update_kernel
@@ -1004,6 +1115,7 @@ struct sdr_grabber {
   uint8_t *d_phase = nullptr, *d_valid = nullptr;
   std::vector<uint8_t> phase, valid, fresh; /* blocks processed mod 2, _dataBufferValid, _newDataIsAvailable */
   uint32_t n_valid = 0;
+  int fft_ctas = 1; /* resident CTAs of the warp-FFT kernels on the whole device: their grid */
   IdList ids;
   std::vector<uint8_t> mark;
 };
@@ -1015,6 +1127,12 @@ extern "C" int sdr_grabber_create(sdr_grabber_t **out, uint32_t n_channels, int 
   sdr_grabber *h = new sdr_grabber();
   h->n = n_channels; h->device = device;
   h->phase.assign(n_channels, 0); h->valid.assign(n_channels, 0); h->fresh.assign(n_channels, 0);
+  int sms = 0, per_sm = 0;
+  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, grab_snapshots_kernel, FFT_THREADS, 0) != cudaSuccess) {
+    delete h; return fail(SDR_AUX_ECUDA, "cannot query the device's multiprocessors");
+  }
+  h->fft_ctas = std::max(1, sms * per_sm);
   if (cudaMalloc(&h->half, 512 * (size_t)n_channels) != cudaSuccess || cudaMalloc(&h->outb, 1024 * (size_t)n_channels) != cudaSuccess ||
       cudaMalloc(&h->d_phase, n_channels) != cudaSuccess || cudaMalloc(&h->d_valid, n_channels) != cudaSuccess) {
     sdr_grabber_destroy(h); return fail(SDR_AUX_ENOMEM, "cudaMalloc failed");
@@ -1036,15 +1154,27 @@ extern "C" void sdr_grabber_destroy(sdr_grabber_t *h) {
   delete h;
 }
 
-extern "C" int sdr_grabber_process_device_subset(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
-                                                 size_t pitch, uint32_t n_blocks, void *cuda_stream) {
+/* grid of the warp-FFT kernels: at most one wave of resident CTAs, each warp then strides over the items */
+static unsigned fft_grid(const sdr_grabber *h, unsigned long long items) {
+  const unsigned long long need = (items + FFT_THREADS / 32 - 1) / (FFT_THREADS / 32), cap = (unsigned long long)h->fft_ctas;
+  return (unsigned)std::max(1ull, std::min(need, cap));
+}
+
+extern "C" int sdr_grabber_process_device_snapshots(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I,
+                                                    const int16_t *Q, size_t pitch, uint32_t n_blocks, int16_t *snapshots, float *power,
+                                                    uint32_t *counts, void *cuda_stream) {
   if (!h || !I || !Q || n_blocks == 0) return fail(SDR_AUX_EINVAL, "bad arguments");
   if (int rc = check_ids(channel_ids, n_ids, h->n, h->mark)) return rc;
   if ((pitch & 7) || pitch < (size_t)n_blocks * 128 || (((uintptr_t)I | (uintptr_t)Q) & 15)) return fail(SDR_AUX_EINVAL, "planes must be 16-byte aligned, pitch a multiple of 8 and >= 128*n_blocks");
+  if (((uintptr_t)snapshots | (uintptr_t)power) & 15) return fail(SDR_AUX_EINVAL, "snapshots and power must be 16-byte aligned");
   CK(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
   if (channel_ids) { if (int rc = h->ids.upload(channel_ids, n_ids, st)) return rc; }
   GrabLaunch L = {I, Q, pitch, h->half, h->outb, h->d_phase, h->d_valid, channel_ids ? h->ids.d : nullptr, n_ids, n_blocks};
+  if (snapshots || power) { /* reads the phases and carried halves before grab_update_kernel moves them on */
+    grab_snapshots_kernel<<<fft_grid(h, (unsigned long long)n_ids * ((n_blocks + 1) / 2)), FFT_THREADS, 0, st>>>(L, snapshots, power);
+    CK(cudaGetLastError());
+  }
   const unsigned long long threads = (unsigned long long)n_ids * 64;
   grab_update_kernel<<<(unsigned)((threads + GRAB_THREADS - 1) / GRAB_THREADS), GRAB_THREADS, 0, st>>>(L);
   CK(cudaGetLastError());
@@ -1052,10 +1182,16 @@ extern "C" int sdr_grabber_process_device_subset(sdr_grabber_t *h, const uint32_
   for (uint32_t i = 0; i < n_ids; i++) { /* the host mirror of what the kernel does to phase and valid */
     const uint32_t c = channel_ids ? channel_ids[i] : i;
     const bool completed = h->phase[c] + n_blocks >= 2; /* some block of this call completes a pair */
+    if (counts) counts[i] = (h->phase[c] + n_blocks) / 2;
     h->phase[c] = (uint8_t)((h->phase[c] + n_blocks) & 1);
     if (completed) { h->n_valid += !h->valid[c]; h->valid[c] = 1; h->fresh[c] = 1; }
   }
   return 0;
+}
+
+extern "C" int sdr_grabber_process_device_subset(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+                                                 size_t pitch, uint32_t n_blocks, void *cuda_stream) {
+  return sdr_grabber_process_device_snapshots(h, channel_ids, n_ids, I, Q, pitch, n_blocks, nullptr, nullptr, nullptr, cuda_stream);
 }
 
 extern "C" int sdr_grabber_process_device(sdr_grabber_t *h, const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, void *cuda_stream) {
@@ -1119,13 +1255,10 @@ extern "C" int sdr_grabber_spectrum_device(sdr_grabber_t *h, const uint32_t *d_c
   const uint32_t cnt = d_channels ? n : h->n;
   if (cnt == 0) return 1;
   cudaStream_t st = (cudaStream_t)cuda_stream;
-  if (h->n_valid == h->n) {
-    grab_spectrum_kernel<<<cnt, 128, 0, st>>>(h->outb, d_channels, d_power);
-    CK(cudaGetLastError());
-    return 1;
-  }
-  grab_spectrum_valid_kernel<<<cnt, 128, 0, st>>>(h->outb, d_channels, h->d_valid, d_power);
+  const bool every = h->n_valid == h->n;
+  grab_spectrum_kernel<<<fft_grid(h, cnt), FFT_THREADS, 0, st>>>(h->outb, d_channels, every ? nullptr : h->d_valid, cnt, d_power);
   CK(cudaGetLastError());
+  if (every) return 1;
   if (!d_channels) return 1;
   /* whether a listed channel has a snapshot: the list is in device memory */
   std::vector<uint32_t> ids(cnt);
@@ -1160,7 +1293,7 @@ extern "C" int sdr_grabber_spectrum(sdr_grabber_t *h, const uint32_t *channels, 
       if (cudaMalloc(&d_ch, (size_t)m * 4) != cudaSuccess) { rc = fail(SDR_AUX_ENOMEM, "cudaMalloc failed"); break; }
       if (cudaMemcpy(d_ch, sel.data(), (size_t)m * 4, cudaMemcpyHostToDevice) != cudaSuccess) { rc = fail(SDR_AUX_ECUDA, "copy failed"); break; }
     }
-    grab_spectrum_kernel<<<m, 128>>>(h->outb, d_ch, d_p);
+    grab_spectrum_kernel<<<fft_grid(h, m), FFT_THREADS>>>(h->outb, d_ch, nullptr, m, d_p);
     if (cudaGetLastError() != cudaSuccess) { rc = fail(SDR_AUX_ECUDA, "spectrum kernel failed"); break; }
     if (m == cnt) {
       if (cudaMemcpy(power, d_p, (size_t)m * 1024, cudaMemcpyDeviceToHost) != cudaSuccess) { rc = fail(SDR_AUX_ECUDA, "copy failed"); break; }

@@ -125,7 +125,9 @@ class IQGeneratorBatch {
 /* AudioGrabberComplex256 (AudioGrabberComplex256.h:46-64) for n channels */
 class GrabberBatch {
  public:
-  explicit GrabberBatch(uint32_t n_channels, int device = 0) : h_(nullptr) { check(sdr_grabber_create(&h_, n_channels, device), "sdr_grabber_create"); }
+  explicit GrabberBatch(uint32_t n_channels, int device = 0) : h_(nullptr), n_channels_(n_channels) {
+    check(sdr_grabber_create(&h_, n_channels, device), "sdr_grabber_create");
+  }
   ~GrabberBatch() { sdr_grabber_destroy(h_); }
   GrabberBatch(const GrabberBatch &) = delete;
   GrabberBatch &operator=(const GrabberBatch &) = delete;
@@ -135,6 +137,19 @@ class GrabberBatch {
   }
   void process(const std::vector<uint32_t> &ids, const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, void *cuda_stream = nullptr) {
     check(sdr_grabber_process_device_subset(h_, ids.data(), (uint32_t)ids.size(), I, Q, pitch, n_blocks, cuda_stream), "sdr_grabber_process_device_subset");
+  }
+  /* ... also every snapshot the call publishes and/or its power spectrum (device [rows][(n_blocks+1)/2][512] int16 and
+   * [rows][(n_blocks+1)/2][256] float, either may be null) and the slots written per row (host, rows entries, may be null);
+   * sdr_grabber_process_device_snapshots */
+  void process(const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, int16_t *snapshots, float *power, uint32_t *counts,
+               void *cuda_stream = nullptr) {
+    check(sdr_grabber_process_device_snapshots(h_, nullptr, n_channels_, I, Q, pitch, n_blocks, snapshots, power, counts, cuda_stream),
+          "sdr_grabber_process_device_snapshots");
+  }
+  void process(const std::vector<uint32_t> &ids, const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, int16_t *snapshots,
+               float *power, uint32_t *counts, void *cuda_stream = nullptr) {
+    check(sdr_grabber_process_device_snapshots(h_, ids.data(), (uint32_t)ids.size(), I, Q, pitch, n_blocks, snapshots, power, counts, cuda_stream),
+          "sdr_grabber_process_device_snapshots");
   }
   static size_t state_bytes() { return sdr_grabber_state_bytes(); }
   std::vector<uint8_t> export_state(const std::vector<uint32_t> &ids) {
@@ -157,6 +172,7 @@ class GrabberBatch {
     if (rc != SDR_AUX_OK) throw std::runtime_error(std::string(what) + ": " + sdr_aux_last_error());
   }
   sdr_grabber_t *h_;
+  uint32_t n_channels_;
 };
 
 }  // namespace sdr

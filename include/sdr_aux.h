@@ -121,6 +121,23 @@ int sdr_grabber_process_device(sdr_grabber_t *h, const int16_t *I, const int16_t
  * new-data flag, so after calls on subsets the channels differ in all three. */
 int sdr_grabber_process_device_subset(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
                                       size_t pitch, uint32_t n_blocks, void *cuda_stream);
+/* The same call, also returning every snapshot it publishes and/or its power spectrum: what a sketch polling
+ * newDataAvailable() / grab() after every update() sees, one line per completed pair (a panadapter or waterfall per channel).
+ * Ids, planes and checks are those of sdr_grabber_process_device_subset, and the state it leaves is the same.
+ *   S = (n_blocks + 1) / 2 slots per row.  With p = the row's channel's pair phase before the call (its own blocks processed,
+ *   mod 2), the row publishes counts[i] = (p + n_blocks) / 2 snapshots, in slots 0 .. counts[i]-1: slot k is the pair the
+ *   call's block 2k + 1 - p (0-based) completes, the block after which the reference's newDataAvailable() turns true.  When
+ *   p == 1, slot 0 starts with the block carried over from the channel's previous call (or from an imported blob).  Slots
+ *   past counts[i] are not written (only when n_blocks is odd and p == 0).
+ *   snapshots  device, int16 [n_ids][S][512] or NULL: each slot as grab() would have written it right after that block.
+ *   power      device, float [n_ids][S][256] or NULL: each slot's spectrum, the same bins, order and bits as
+ *              sdr_grabber_spectrum.
+ *   counts     host, uint32 [n_ids] or NULL: filled before the call returns, without synchronising.
+ * snapshots and power must be 16-byte aligned (SDR_AUX_EINVAL otherwise, nothing queued).  With all three NULL this is
+ * sdr_grabber_process_device_subset.  Channel-major layout: a channel's waterfall for the call is one contiguous [S][256]. */
+int sdr_grabber_process_device_snapshots(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+                                         size_t pitch, uint32_t n_blocks, int16_t *snapshots, float *power, uint32_t *counts,
+                                         void *cuda_stream);
 /* newDataAvailable() of one channel: 1 / 0, negative on error */
 int sdr_grabber_new_data_available(sdr_grabber_t *h, uint32_t channel);
 /* grab() for the listed channels (NULL: all): 512 int16 per channel = 256 complex samples, to HOST memory
