@@ -8,8 +8,11 @@
  * restates the published transform (X[k] = sum x[n] exp(-2 pi i n k / 128), natural-order output) as a radix-2
  * decimation-in-frequency network in float32 with one rounding per operation; any correct float32 FFT agrees with
  * it to a few ulp of the largest line.  Everything the reference computes FROM the spectrum (AudioSDRpreProcessor.cpp:
- * 91-118) consumes it only through threshold compares, and tests/test_preproc.py checks the decisions against a
- * float64 DFT as well.  The CUDA kernel evaluates the identical operation network, so CUDA == this file bit for bit.
+ * 91-118) consumes it only through threshold compares, and
+ * tests/test_aux_oracle.py::test_detector_decisions_do_not_hinge_on_fft_rounding checks the decisions against a float64
+ * DFT as well.  The CUDA kernel evaluates the identical operation network, so CUDA == this file bit for bit.
+ * tests/test_emu_pp_edges.py and tests/test_gpu_pp_edges.py pin the kernel to this network on purpose, with blocks one
+ * rounding away from each decision, while parity with CMSIS stays unpinned.
  *
  * Used by oracle/sdr_aux_oracle.c (the restatement) and by oracle/shim/arm_math.h (so that the host-compiled
  * reference in oracle/_ref/refaux calls the same transform).

@@ -72,7 +72,9 @@ def test_kernel_lane_source_matches_oracle_on_host(tmp_path):
 def test_detector_decisions_do_not_hinge_on_fft_rounding():
     """PARITY UNPINNED piece (oracle/aux_fft128.h): the FFT is a restatement of CMSIS-DSP.  Its float32 power spectrum must
     agree with a float64 DFT to float32 accuracy, and the quantities the detector thresholds (strongest line vs 10 x mean,
-    line vs image vs 10) must sit far from their thresholds on the test signals, so any correct float32 FFT decides alike."""
+    line vs image vs 10) must sit far from their thresholds on the test signals, so any correct float32 FFT decides alike.
+    test_emu_pp_edges.py and test_gpu_pp_edges.py pin the CUDA kernel to this network on purpose, with blocks one rounding
+    away from each decision, while parity with CMSIS stays unpinned."""
     I, Q = S.pp_case(8, 40, seed=3)
     worst, margins = 0.0, []
     for c in range(8):
