@@ -10,6 +10,8 @@
  *    a feed-forward copy, 8 bytes moved per sample, HBM bound (pp_static_kernel).  Channels whose detector is running are
  *    compacted into a list and handled block by block by pp_detect_kernel (lane = channel, 128-point FFT per block in
  *    shared memory), because their correction may change from one block to the next.
+ *  Both blocks serve calls on every channel and on subsets (compact planes, row r = channel ids[r]) with one kernel template
+ *  per job; the two forms differ only in where a row's channel comes from (see kList below).
  */
 #include <cuda_runtime.h>
 
@@ -26,6 +28,11 @@
 __constant__ float c_iq_h[64];
 __constant__ float c_fft_tw[128];
 __constant__ float c_fft_tw256[256];
+
+/* The pre-processor and I/Q generator kernels are templates on kList, one source per job.  kList = true serves the *_subset
+ * entry points: the planes are compact, row r belonging to channel ids[r] (device copy of the call's id list), and
+ * L.n_channels counts rows.  Plane addresses use r; state (history, gains, PpState) uses ch = kList ? ids[r] : r.
+ * kList = false is the call on every channel (row = channel, ids unused). */
 
 /* ================================================================== I/Q generator ==== */
 #define IQ_SEG 4096
@@ -49,62 +56,10 @@ __device__ __forceinline__ void iq_unpack8(const int4 v, float *f) {
   }
 }
 
-__global__ void __launch_bounds__(IQ_THREADS) iq_generate_kernel(const IqLaunch L) {
+template <bool kList>
+__global__ void __launch_bounds__(IQ_THREADS) iq_generate_kernel(const IqLaunch L, const uint32_t *ids) {
   __shared__ float xs[IQ_XS_WORDS];
-  const uint32_t ch = blockIdx.x / L.segs, seg = blockIdx.x % L.segs;
-  const long base = (long)seg * IQ_SEG;
-  const int16_t *row = L.x + (size_t)ch * L.in_pitch;
-  /* the span [base-256, base+SEG) as floats at padded positions; 8 samples (16 bytes) per thread and pass */
-  for (int t = threadIdx.x; t < (IQ_SEG + 256) / 8; t += IQ_THREADS) {
-    const long n = base - 256 + 8 * t;
-    int4 v = make_int4(0, 0, 0, 0);
-    if (n < 0) v = *reinterpret_cast<const int4 *>(L.hist_in + (size_t)ch * 256 + (256 + n));
-    else if (n < (long)L.n_samples) v = __ldg(reinterpret_cast<const int4 *>(row + n));
-    float f[8];
-    iq_unpack8(v, f);
-    float *dst = xs + 8 * t + ((8 * t) >> 4);
-#pragma unroll
-    for (int i = 0; i < 8; i++) dst[i] = f[i];
-  }
-  __syncthreads();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long n0 = base + 512 * warp + 16 * lane;
-  if (n0 >= (long)L.n_samples) return;
-  const int q0 = 256 + 512 * warp + 16 * lane;
-  float acc[16];
-  iq_lane_fir(xs, q0, c_iq_h, acc);
-  const float2 g = L.gains[ch];
-  uint32_t wi[8], wq[8];
-  if (g.x == 1.0f && g.y == 1.0f) { /* the constructor's balance (IQ.h:72-73): uniform over the CTA, no FP64, no range test */
-#pragma unroll
-    for (int c = 0; c < 16; c += 2) {
-      const int i0 = aux_to_pcm_unit(iq_lane_delayed(xs, q0, c)), i1 = aux_to_pcm_unit(iq_lane_delayed(xs, q0, c + 1));
-      const int q0v = aux_to_pcm_unit(acc[c]), q1v = aux_to_pcm_unit(acc[c + 1]);
-      wi[c >> 1] = ((uint32_t)i0 & 0xFFFFu) | ((uint32_t)i1 << 16);
-      wq[c >> 1] = ((uint32_t)q0v & 0xFFFFu) | ((uint32_t)q1v << 16);
-    }
-  } else {
-#pragma unroll
-    for (int c = 0; c < 16; c += 2) {
-      const int i0 = aux_to_pcm(iq_lane_delayed(xs, q0, c), g.x), i1 = aux_to_pcm(iq_lane_delayed(xs, q0, c + 1), g.x);
-      const int q0v = aux_to_pcm(acc[c], g.y), q1v = aux_to_pcm(acc[c + 1], g.y);
-      wi[c >> 1] = ((uint32_t)i0 & 0xFFFFu) | ((uint32_t)i1 << 16);
-      wq[c >> 1] = ((uint32_t)q0v & 0xFFFFu) | ((uint32_t)q1v << 16);
-    }
-  }
-  uint4 *di = reinterpret_cast<uint4 *>(L.oi + (size_t)ch * L.out_pitch + n0);
-  uint4 *dq = reinterpret_cast<uint4 *>(L.oq + (size_t)ch * L.out_pitch + n0);
-  di[0] = make_uint4(wi[0], wi[1], wi[2], wi[3]); di[1] = make_uint4(wi[4], wi[5], wi[6], wi[7]);
-  dq[0] = make_uint4(wq[0], wq[1], wq[2], wq[3]); dq[1] = make_uint4(wq[4], wq[5], wq[6], wq[7]);
-}
-
-/* Subset twins (the *_subset entry points): the planes are compact, row r belonging to channel ids[r] (device copy of the
- * call's id list); plane addresses use r, state (history, gains, PpState) uses ids[r], and L.n_channels counts rows.  The
- * kernels above are kept as they are, so that calls on every channel run the same code as before.
- * iq_generate_subset_kernel: grid n_ids x segs. */
-__global__ void __launch_bounds__(IQ_THREADS) iq_generate_subset_kernel(const IqLaunch L, const uint32_t *ids) {
-  __shared__ float xs[IQ_XS_WORDS];
-  const uint32_t r = blockIdx.x / L.segs, seg = blockIdx.x % L.segs, ch = __ldg(ids + r);
+  const uint32_t r = blockIdx.x / L.segs, seg = blockIdx.x % L.segs, ch = kList ? __ldg(ids + r) : r;
   const long base = (long)seg * IQ_SEG;
   const int16_t *row = L.x + (size_t)r * L.in_pitch;
   /* the span [base-256, base+SEG) as floats at padded positions; 8 samples (16 bytes) per thread and pass */
@@ -151,31 +106,21 @@ __global__ void __launch_bounds__(IQ_THREADS) iq_generate_subset_kernel(const Iq
   dq[0] = make_uint4(wq[0], wq[1], wq[2], wq[3]); dq[1] = make_uint4(wq[4], wq[5], wq[6], wq[7]);
 }
 
-/* the last 256 inputs of every channel become the next call's history (other buffer: no ordering hazard) */
-__global__ void iq_history_kernel(const IqLaunch L) {
-  const uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x;
-  const uint32_t ch = idx >> 5, j = idx & 31;
-  if (ch >= L.n_channels) return;
-  const long n = (long)L.n_samples - 256 + 8 * (long)j;
-  int4 v;
-  if (n < 0) v = *reinterpret_cast<const int4 *>(L.hist_in + (size_t)ch * 256 + (256 + n));
-  else v = __ldg(reinterpret_cast<const int4 *>(L.x + (size_t)ch * L.in_pitch + n));
-  *reinterpret_cast<int4 *>(L.hist_out + (size_t)ch * 256 + 8 * j) = v;
-}
-
-/* subset twin: the history is rewritten IN PLACE (hist_out == hist_in), because the channels that skip the call keep
- * theirs in the same buffer.  One warp = one listed channel: with fewer than 256 new samples lane j reads the old slot that
- * lane j + n_samples/8 overwrites, so every lane loads before any lane stores. */
-__global__ void iq_history_subset_kernel(const IqLaunch L, const uint32_t *ids) {
+/* the last 256 inputs of every listed channel become the next call's history.  Calls on every channel write the other
+ * buffer (no ordering hazard).  Subset calls rewrite it IN PLACE (hist_out == hist_in), because the channels that skip the
+ * call keep theirs in the same buffer: one warp = one row, and with fewer than 256 new samples lane j reads the old slot
+ * that lane j + n_samples/8 overwrites, so every lane loads before any lane stores. */
+template <bool kList>
+__global__ void iq_history_kernel(const IqLaunch L, const uint32_t *ids) {
   const uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x;
   const uint32_t r = idx >> 5, j = idx & 31;
   if (r >= L.n_channels) return; /* whole warps */
-  const uint32_t ch = __ldg(ids + r);
+  const uint32_t ch = kList ? __ldg(ids + r) : r;
   const long n = (long)L.n_samples - 256 + 8 * (long)j;
   int4 v;
   if (n < 0) v = *reinterpret_cast<const int4 *>(L.hist_in + (size_t)ch * 256 + (256 + n));
   else v = __ldg(reinterpret_cast<const int4 *>(L.x + (size_t)r * L.in_pitch + n));
-  __syncwarp();
+  if (kList) __syncwarp();
   *reinterpret_cast<int4 *>(L.hist_out + (size_t)ch * 256 + 8 * j) = v;
 }
 
@@ -199,15 +144,12 @@ __global__ void pp_apply_kernel(PpState *st, uint32_t n_channels, const PpSetter
   st[ch] = s;
 }
 
-__global__ void pp_list_kernel(const PpLaunch L) {
-  const uint32_t ch = blockIdx.x * blockDim.x + threadIdx.x;
-  if (ch >= L.n_channels) return;
-  if (L.state[ch].autod) L.auto_list[atomicAdd(L.auto_count, 1u)] = ch;
-}
-__global__ void pp_list_subset_kernel(const PpLaunch L, const uint32_t *ids) {
+/* the rows whose detector is running */
+template <bool kList>
+__global__ void pp_list_kernel(const PpLaunch L, const uint32_t *ids) {
   const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= L.n_channels) return;
-  if (L.state[__ldg(ids + r)].autod) L.auto_list[atomicAdd(L.auto_count, 1u)] = r;
+  if (L.state[kList ? __ldg(ids + r) : r].autod) L.auto_list[atomicAdd(L.auto_count, 1u)] = r;
 }
 
 __device__ __forceinline__ void unpack_i16x8(const int4 v, int16_t *o) {
@@ -223,35 +165,13 @@ __device__ __forceinline__ int4 pack_i16x8(const int16_t *o) {
 }
 
 /* detector off: one thread = one 16-byte chunk of both rails.  8 bytes in + 8 bytes out per 2 samples... i.e. 8 B/sample. */
-__global__ void __launch_bounds__(256) pp_static_kernel(const PpLaunch L) {
-  const uint32_t chunks = L.n_blocks * 16; /* per channel */
-  const unsigned long long idx = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
-  const uint32_t ch = (uint32_t)(idx / chunks), j = (uint32_t)(idx % chunks);
-  if (ch >= L.n_channels) return;
-  const PpState s = L.state[ch];
-  if (s.autod) return; /* pp_detect_kernel owns this channel for the call */
-  const int16_t *ri = L.I + (size_t)ch * L.in_pitch, *rq = L.Q + (size_t)ch * L.in_pitch;
-  const size_t n = (size_t)j * 8;
-  const int4 a = __ldg(reinterpret_cast<const int4 *>(ri + n)), b = __ldg(reinterpret_cast<const int4 *>(rq + n));
-  int4 oa = a, ob = b;
-  if (s.corr != 0) {
-    int16_t vi[8], vq[8], oi[8], oq[8];
-    unpack_i16x8(a, vi); unpack_i16x8(b, vq);
-    int16_t pi = (int16_t)s.saved, pq = (int16_t)s.saved;
-    if (j) { if (s.corr == 1) pi = ri[n - 1]; else pq = rq[n - 1]; }
-    pp_static_chunk(vi, vq, pi, pq, (j & 15) == 0, s.corr, 0, oi, oq);
-    oa = pack_i16x8(oi); ob = pack_i16x8(oq);
-  }
-  int4 *di = reinterpret_cast<int4 *>(L.oi + (size_t)ch * L.out_pitch + n), *dq = reinterpret_cast<int4 *>(L.oq + (size_t)ch * L.out_pitch + n);
-  *di = s.swap ? ob : oa;
-  *dq = s.swap ? oa : ob;
-}
-__global__ void __launch_bounds__(256) pp_static_subset_kernel(const PpLaunch L, const uint32_t *ids) {
+template <bool kList>
+__global__ void __launch_bounds__(256) pp_static_kernel(const PpLaunch L, const uint32_t *ids) {
   const uint32_t chunks = L.n_blocks * 16; /* per channel */
   const unsigned long long idx = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   const uint32_t r = (uint32_t)(idx / chunks), j = (uint32_t)(idx % chunks);
   if (r >= L.n_channels) return;
-  const PpState s = L.state[__ldg(ids + r)];
+  const PpState s = L.state[kList ? __ldg(ids + r) : r];
   if (s.autod) return; /* pp_detect_kernel owns this channel for the call */
   const int16_t *ri = L.I + (size_t)r * L.in_pitch, *rq = L.Q + (size_t)r * L.in_pitch;
   const size_t n = (size_t)j * 8;
@@ -271,25 +191,18 @@ __global__ void __launch_bounds__(256) pp_static_subset_kernel(const PpLaunch L,
 }
 
 /* detector off: savedSample after the call = the delayed rail's last input sample (PP.cpp:62-65 / 67-70) */
-__global__ void pp_finish_kernel(const PpLaunch L) {
-  const uint32_t ch = blockIdx.x * blockDim.x + threadIdx.x;
-  if (ch >= L.n_channels) return;
-  const PpState s = L.state[ch];
-  if (s.autod || s.corr == 0) return;
-  const size_t last = (size_t)L.n_blocks * 128 - 1;
-  L.state[ch].saved = (s.corr == 1 ? L.I : L.Q)[(size_t)ch * L.in_pitch + last];
-}
-__global__ void pp_finish_subset_kernel(const PpLaunch L, const uint32_t *ids) {
+template <bool kList>
+__global__ void pp_finish_kernel(const PpLaunch L, const uint32_t *ids) {
   const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= L.n_channels) return;
-  const uint32_t ch = __ldg(ids + r);
+  const uint32_t ch = kList ? __ldg(ids + r) : r;
   const PpState s = L.state[ch];
   if (s.autod || s.corr == 0) return;
   const size_t last = (size_t)L.n_blocks * 128 - 1;
   L.state[ch].saved = (s.corr == 1 ? L.I : L.Q)[(size_t)r * L.in_pitch + last];
 }
 
-/* detector running: one CTA = 32 listed channels (lane = channel) x PP_W warps that share each channel's work, block
+/* detector running: one CTA = 32 listed rows (lane = row) x PP_W warps that share each channel's work, block
  * after block.  Rows are staged through shared memory with whole-row (coalesced) transfers; a lane's row is 65 words from
  * its neighbour's (odd: no bank conflicts); the FFT buffer is [256][32] floats, lane-interleaved.  Warp 0 owns the
  * per-channel state (correction, counters); the butterflies of a stage, the conversions and the rows are split over
@@ -297,78 +210,8 @@ __global__ void pp_finish_subset_kernel(const PpLaunch L, const uint32_t *ids) {
 #define PP_W 8
 #define PP_ROW_WORDS 65
 #define PP_DETECT_SMEM (256 * 32 * 4 + 2 * 32 * PP_ROW_WORDS * 4 + 2 * 32 * 4)
-__global__ void __launch_bounds__(32 * PP_W) pp_detect_kernel(const PpLaunch L) {
-  extern __shared__ __align__(16) unsigned char sm[];
-  float *fft = reinterpret_cast<float *>(sm);
-  uint32_t *rowI = reinterpret_cast<uint32_t *>(sm + 256 * 32 * 4), *rowQ = rowI + 32 * PP_ROW_WORDS;
-  int *sh_det = reinterpret_cast<int *>(rowQ + 32 * PP_ROW_WORDS), *sh_swap = sh_det + 32;
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-  const uint32_t n_auto = *L.auto_count, first = blockIdx.x * 32;
-  if (first >= n_auto) return;
-  const int ch = first + lane < n_auto ? (int)L.auto_list[first + lane] : -1;
-  PpState s;
-  s.corr = s.saved = s.fail = s.succ = s.swap = s.autod = s.pad0 = s.pad1 = 0;
-  if (ch >= 0) s = L.state[ch]; /* every warp reads it; only warp 0's copy evolves and is written back */
-  float *mine = fft + lane;
-  for (uint32_t b = 0; b < L.n_blocks; b++) {
-    for (int r = w; r < 32; r += PP_W) {
-      const int chr = __shfl_sync(0xFFFFFFFFu, ch, r);
-      if (chr >= 0) {
-        const uint32_t *si = reinterpret_cast<const uint32_t *>(L.I + (size_t)chr * L.in_pitch + (size_t)b * 128);
-        const uint32_t *sq = reinterpret_cast<const uint32_t *>(L.Q + (size_t)chr * L.in_pitch + (size_t)b * 128);
-        rowI[r * PP_ROW_WORDS + lane] = __ldg(si + lane); rowI[r * PP_ROW_WORDS + 32 + lane] = __ldg(si + 32 + lane);
-        rowQ[r * PP_ROW_WORDS + lane] = __ldg(sq + lane); rowQ[r * PP_ROW_WORDS + 32 + lane] = __ldg(sq + 32 + lane);
-      }
-    }
-    __syncthreads();
-    int16_t *ri = reinterpret_cast<int16_t *>(rowI + lane * PP_ROW_WORDS), *rq = reinterpret_cast<int16_t *>(rowQ + lane * PP_ROW_WORDS);
-    if (w == 0) {
-      if (ch >= 0) pp_correct_block(ri, rq, s);
-      sh_det[lane] = ch >= 0 && s.autod;
-      sh_swap[lane] = s.swap;
-    }
-    __syncthreads();
-    const bool det = sh_det[lane] != 0;
-    if (__any_sync(0xFFFFFFFFu, det)) { /* same lanes, same flags in every warp: uniform over the CTA */
-      if (det) {
-        for (int i = w; i < 128; i += PP_W) {
-          mine[(2 * i) * 32] = aux_q15_to_float(ri[i]);
-          mine[(2 * i + 1) * 32] = aux_q15_to_float(rq[i]);
-        }
-      }
-      __syncthreads();
-      for (int st = 0; st < 7; st++) {
-        if (det) pp_fft128_stage(mine, 32, c_fft_tw, st, w, PP_W);
-        __syncthreads();
-      }
-      float pw[128 / PP_W];
-      if (det) {
-#pragma unroll
-        for (int k = 0; k < 128 / PP_W; k++) pw[k] = pp_power(mine, 32, w + k * PP_W);
-      }
-      __syncthreads();
-      if (det) {
-#pragma unroll
-        for (int k = 0; k < 128 / PP_W; k++) mine[(w + k * PP_W) * 32] = pw[k];
-      }
-      __syncthreads();
-      if (w == 0 && det) pp_decide(mine, 32, s);
-    }
-    for (int r = w; r < 32; r += PP_W) {
-      const int chr = __shfl_sync(0xFFFFFFFFu, ch, r), sw = sh_swap[r];
-      if (chr >= 0) {
-        const uint32_t *a = (sw ? rowQ : rowI) + r * PP_ROW_WORDS, *c = (sw ? rowI : rowQ) + r * PP_ROW_WORDS;
-        uint32_t *di = reinterpret_cast<uint32_t *>(L.oi + (size_t)chr * L.out_pitch + (size_t)b * 128);
-        uint32_t *dq = reinterpret_cast<uint32_t *>(L.oq + (size_t)chr * L.out_pitch + (size_t)b * 128);
-        di[lane] = a[lane]; di[32 + lane] = a[32 + lane];
-        dq[lane] = c[lane]; dq[32 + lane] = c[32 + lane];
-      }
-    }
-    __syncthreads();
-  }
-  if (w == 0 && ch >= 0) L.state[ch] = s;
-}
-__global__ void __launch_bounds__(32 * PP_W) pp_detect_subset_kernel(const PpLaunch L, const uint32_t *ids) {
+template <bool kList>
+__global__ void __launch_bounds__(32 * PP_W) pp_detect_kernel(const PpLaunch L, const uint32_t *ids) {
   extern __shared__ __align__(16) unsigned char sm[];
   float *fft = reinterpret_cast<float *>(sm);
   uint32_t *rowI = reinterpret_cast<uint32_t *>(sm + 256 * 32 * 4), *rowQ = rowI + 32 * PP_ROW_WORDS;
@@ -377,17 +220,17 @@ __global__ void __launch_bounds__(32 * PP_W) pp_detect_subset_kernel(const PpLau
   const uint32_t n_auto = *L.auto_count, first = blockIdx.x * 32;
   if (first >= n_auto) return;
   const int row = first + lane < n_auto ? (int)L.auto_list[first + lane] : -1; /* the list holds plane rows */
-  const int ch = row >= 0 ? (int)__ldg(ids + row) : row;
+  const int ch = kList && row >= 0 ? (int)__ldg(ids + row) : row;
   PpState s;
   s.corr = s.saved = s.fail = s.succ = s.swap = s.autod = s.pad0 = s.pad1 = 0;
   if (ch >= 0) s = L.state[ch]; /* every warp reads it; only warp 0's copy evolves and is written back */
   float *mine = fft + lane;
   for (uint32_t b = 0; b < L.n_blocks; b++) {
     for (int r = w; r < 32; r += PP_W) {
-      const int chr = __shfl_sync(0xFFFFFFFFu, row, r);
-      if (chr >= 0) {
-        const uint32_t *si = reinterpret_cast<const uint32_t *>(L.I + (size_t)chr * L.in_pitch + (size_t)b * 128);
-        const uint32_t *sq = reinterpret_cast<const uint32_t *>(L.Q + (size_t)chr * L.in_pitch + (size_t)b * 128);
+      const int rr = __shfl_sync(0xFFFFFFFFu, row, r);
+      if (rr >= 0) {
+        const uint32_t *si = reinterpret_cast<const uint32_t *>(L.I + (size_t)rr * L.in_pitch + (size_t)b * 128);
+        const uint32_t *sq = reinterpret_cast<const uint32_t *>(L.Q + (size_t)rr * L.in_pitch + (size_t)b * 128);
         rowI[r * PP_ROW_WORDS + lane] = __ldg(si + lane); rowI[r * PP_ROW_WORDS + 32 + lane] = __ldg(si + 32 + lane);
         rowQ[r * PP_ROW_WORDS + lane] = __ldg(sq + lane); rowQ[r * PP_ROW_WORDS + 32 + lane] = __ldg(sq + 32 + lane);
       }
@@ -427,11 +270,11 @@ __global__ void __launch_bounds__(32 * PP_W) pp_detect_subset_kernel(const PpLau
       if (w == 0 && det) pp_decide(mine, 32, s);
     }
     for (int r = w; r < 32; r += PP_W) {
-      const int chr = __shfl_sync(0xFFFFFFFFu, row, r), sw = sh_swap[r];
-      if (chr >= 0) {
+      const int rr = __shfl_sync(0xFFFFFFFFu, row, r), sw = sh_swap[r];
+      if (rr >= 0) {
         const uint32_t *a = (sw ? rowQ : rowI) + r * PP_ROW_WORDS, *c = (sw ? rowI : rowQ) + r * PP_ROW_WORDS;
-        uint32_t *di = reinterpret_cast<uint32_t *>(L.oi + (size_t)chr * L.out_pitch + (size_t)b * 128);
-        uint32_t *dq = reinterpret_cast<uint32_t *>(L.oq + (size_t)chr * L.out_pitch + (size_t)b * 128);
+        uint32_t *di = reinterpret_cast<uint32_t *>(L.oi + (size_t)rr * L.out_pitch + (size_t)b * 128);
+        uint32_t *dq = reinterpret_cast<uint32_t *>(L.oq + (size_t)rr * L.out_pitch + (size_t)b * 128);
         di[lane] = a[lane]; di[32 + lane] = a[32 + lane];
         dq[lane] = c[lane]; dq[32 + lane] = c[32 + lane];
       }
@@ -771,8 +614,8 @@ extern "C" int sdr_preproc_create(sdr_preproc_t **out, uint32_t n_channels, int 
   if (!out || n_channels == 0) return fail(SDR_AUX_EINVAL, "sdr_preproc_create: bad arguments");
   CK(cudaSetDevice(device));
   if (int rc = upload_tables()) return rc;
-  CK(cudaFuncSetAttribute(pp_detect_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
-  CK(cudaFuncSetAttribute(pp_detect_subset_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
+  CK(cudaFuncSetAttribute(pp_detect_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
+  CK(cudaFuncSetAttribute(pp_detect_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
   sdr_preproc *h = new sdr_preproc();
   h->n = n_channels; h->device = device;
   if (cudaMalloc(&h->state, sizeof(PpState) * n_channels) != cudaSuccess || cudaMalloc(&h->list, 4 * (size_t)n_channels) != cudaSuccess ||
@@ -837,6 +680,27 @@ extern "C" int sdr_preproc_get_status(sdr_preproc_t *h, const uint32_t *channels
   return 0;
 }
 
+/* a process call's launches; ids: the device id list of a subset call (kList), else unused */
+template <bool kList>
+static int pp_launch(sdr_preproc *h, const PpLaunch &L, const uint32_t *ids, cudaStream_t st) {
+  const uint32_t n = L.n_channels, tb = (n + 255) / 256;
+  const unsigned long long threads = (unsigned long long)n * L.n_blocks * 16;
+  const unsigned sb = (unsigned)((threads + 255) / 256);
+  if (h->auto_possible) {
+    CK(cudaMemsetAsync(h->count, 0, 4, st));
+    pp_list_kernel<kList><<<tb, 256, 0, st>>>(L, ids);
+    h->launches++;
+  }
+  pp_static_kernel<kList><<<sb, 256, 0, st>>>(L, ids);
+  pp_finish_kernel<kList><<<tb, 256, 0, st>>>(L, ids);
+  h->launches += 2;
+  if (h->auto_possible) {
+    pp_detect_kernel<kList><<<(n + 31) / 32, 32 * PP_W, PP_DETECT_SMEM, st>>>(L, ids);
+    h->launches++;
+  }
+  return 0;
+}
+
 extern "C" int sdr_preproc_process_device_subset(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
                                                  size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks,
                                                  void *cuda_stream) {
@@ -848,38 +712,12 @@ extern "C" int sdr_preproc_process_device_subset(sdr_preproc_t *h, const uint32_
   cudaStream_t st = (cudaStream_t)cuda_stream;
   if (int rc = pp_flush(h, st)) return rc; /* setters of every channel, listed or not, in call order */
   PpLaunch L = {I, Q, I_out, Q_out, in_pitch, out_pitch, h->state, n_ids, n_blocks, h->list, h->count};
-  const uint32_t tb = (n_ids + 255) / 256;
-  const unsigned long long threads = (unsigned long long)n_ids * n_blocks * 16;
-  const unsigned sb = (unsigned)((threads + 255) / 256);
-  if (!channel_ids) {
-    if (h->auto_possible) {
-      CK(cudaMemsetAsync(h->count, 0, 4, st));
-      pp_list_kernel<<<tb, 256, 0, st>>>(L);
-      h->launches++;
-    }
-    pp_static_kernel<<<sb, 256, 0, st>>>(L);
-    pp_finish_kernel<<<tb, 256, 0, st>>>(L);
-    h->launches += 2;
-    if (h->auto_possible) {
-      pp_detect_kernel<<<(n_ids + 31) / 32, 32 * PP_W, PP_DETECT_SMEM, st>>>(L);
-      h->launches++;
-    }
-  } else {
+  if (channel_ids) {
     if (int rc = h->ids.upload(channel_ids, n_ids, st)) return rc;
-    const uint32_t *d = h->ids.d;
-    if (h->auto_possible) {
-      CK(cudaMemsetAsync(h->count, 0, 4, st));
-      pp_list_subset_kernel<<<tb, 256, 0, st>>>(L, d);
-      h->launches++;
-    }
-    pp_static_subset_kernel<<<sb, 256, 0, st>>>(L, d);
-    pp_finish_subset_kernel<<<tb, 256, 0, st>>>(L, d);
-    h->launches += 2;
-    if (h->auto_possible) {
-      pp_detect_subset_kernel<<<(n_ids + 31) / 32, 32 * PP_W, PP_DETECT_SMEM, st>>>(L, d);
-      h->launches++;
-    }
+    if (int rc = pp_launch<true>(h, L, h->ids.d, st)) return rc;
     if (int rc = h->ids.done(st)) return rc;
+  } else if (int rc = pp_launch<false>(h, L, nullptr, st)) {
+    return rc;
   }
   CK(cudaGetLastError());
   return 0;
@@ -1002,6 +840,12 @@ extern "C" int sdr_iqgen_set_gain_balance(sdr_iqgen_t *h, const uint32_t *channe
   return 0;
 }
 
+template <bool kList>
+static void iq_launch(const IqLaunch &L, const uint32_t *ids, unsigned grid, cudaStream_t st) {
+  iq_generate_kernel<kList><<<grid, IQ_THREADS, 0, st>>>(L, ids);
+  iq_history_kernel<kList><<<(L.n_channels * 32 + 255) / 256, 256, 0, st>>>(L, ids);
+}
+
 extern "C" int sdr_iqgen_process_device_subset(sdr_iqgen_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *X, size_t in_pitch,
                                                int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks, void *cuda_stream) {
   if (!h) return fail(SDR_AUX_EINVAL, "null handle");
@@ -1019,20 +863,18 @@ extern "C" int sdr_iqgen_process_device_subset(sdr_iqgen_t *h, const uint32_t *c
   }
   IqLaunch L;
   L.x = X; L.oi = I_out; L.oq = Q_out; L.in_pitch = in_pitch; L.out_pitch = out_pitch;
-  L.hist_in = h->hist[h->cur]; L.hist_out = h->hist[h->cur ^ 1]; L.gains = h->gains;
+  /* a call on every channel writes the new history to the other buffer and flips cur.  A subset call writes it in place:
+   * the skipped channels' history stays in hist[cur].  Segment 0 of iq_generate_kernel, the only reader of the old
+   * history, runs before the history kernel. */
+  L.hist_in = h->hist[h->cur]; L.hist_out = h->hist[channel_ids ? h->cur : h->cur ^ 1]; L.gains = h->gains;
   L.n_samples = n_blocks * 128; L.n_channels = n_ids; L.segs = segs;
-  if (!channel_ids) {
-    iq_generate_kernel<<<(unsigned)grid, IQ_THREADS, 0, st>>>(L);
-    iq_history_kernel<<<(n_ids * 32 + 255) / 256, 256, 0, st>>>(L);
-    h->cur ^= 1;
-  } else {
-    /* the skipped channels' history stays in hist[cur], so the listed channels' new history goes there too (in place);
-     * segment 0 of iq_generate_subset_kernel, the only reader of the old history, runs before the history kernel */
-    L.hist_out = h->hist[h->cur];
+  if (channel_ids) {
     if (int rc = h->ids.upload(channel_ids, n_ids, st)) return rc;
-    iq_generate_subset_kernel<<<(unsigned)grid, IQ_THREADS, 0, st>>>(L, h->ids.d);
-    iq_history_subset_kernel<<<(n_ids * 32 + 255) / 256, 256, 0, st>>>(L, h->ids.d);
+    iq_launch<true>(L, h->ids.d, (unsigned)grid, st);
     if (int rc = h->ids.done(st)) return rc;
+  } else {
+    iq_launch<false>(L, nullptr, (unsigned)grid, st);
+    h->cur ^= 1;
   }
   CK(cudaGetLastError());
   h->launches += 2;

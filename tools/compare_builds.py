@@ -1,9 +1,12 @@
 #!/usr/bin/env python3
-"""tools/compare_builds.py OLD_LIB NEW_LIB OLD_PTXAS_LOG NEW_PTXAS_LOG [OUT] -- registers, spills and SASS instruction counts of
-every kernel of two builds of libsdr_batch.so side by side (no GPU needed).
+"""tools/compare_builds.py OLD_LIB NEW_LIB OLD_PTXAS_LOG NEW_PTXAS_LOG [OUT] [OLD_KERNEL=NEW_KERNEL ...] -- registers, spills
+and SASS of every kernel of two builds of a library side by side (no GPU needed).
 
-The logs are the `-Xptxas -v` output of `python -m audiosdr_b200.build --force` for each build; the instruction counts come from
-`cuobjdump -sass` of the libraries.  Prints (and writes to OUT) one line per kernel and the list of kernels that differ."""
+The logs are the `-Xptxas -v` output of `python -m audiosdr_b200.build --force` for each build; the SASS comes from
+`cuobjdump -sass` of the libraries.  Kernels are matched by mangled name; an OLD_KERNEL=NEW_KERNEL pair matches a kernel that
+was renamed (for example a twin that became a template instantiation).  A matched kernel is the same when its registers and
+spills are, and when its instructions are, each compared as text and encoding (control bits included) with the address
+removed.  Prints (and writes to OUT) one line per kernel and the list of kernels that differ."""
 import collections
 import re
 import subprocess
@@ -27,38 +30,56 @@ def ptxas(log):
     return out
 
 
-def sass_counts(lib):
+def sass(lib):
+    """kernel -> list of its instructions, each `text ; /* encoding */ /* encoding */` with the address stripped"""
     txt = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
     n, fn = collections.OrderedDict(), None
     for line in txt.splitlines():
         m = re.search(r"Function : (\S+)", line)
         if m:
             fn = m.group(1)
-            n[fn] = 0
+            n[fn] = []
             continue
-        if fn and re.match(r"\s+/\*[0-9a-f]+\*/\s+\S", line):
-            n[fn] += 1
+        if not fn:
+            continue
+        m = re.match(r"\s+/\*[0-9a-f]+\*/\s+(\S.*)", line)
+        if m:
+            n[fn].append(" ".join(m.group(1).split()))
+        elif n[fn] and re.match(r"\s+/\* 0x[0-9a-f]+ \*/\s*$", line):  # second encoding word of the instruction above
+            n[fn][-1] += " " + line.strip()
     return n
 
 
 def main():
-    old_lib, new_lib, old_log, new_log = sys.argv[1:5]
-    po, pn, so, sn = ptxas(old_log), ptxas(new_log), sass_counts(old_lib), sass_counts(new_lib)
+    args = sys.argv[1:]
+    old_lib, new_lib, old_log, new_log = args[:4]
+    rest = args[4:]
+    pairs = dict(a.split("=", 1) for a in rest if "=" in a)
+    out = [a for a in rest if "=" not in a]
+    po, pn, so, sn = ptxas(old_log), ptxas(new_log), sass(old_lib), sass(new_lib)
+    renamed = set(pairs.values())
+    rows = [(o, pairs.get(o, o)) for o in so] + [(None, n) for n in sn if n not in renamed and n not in so]
     lines, differ = [], []
-    lines.append("%-44s %14s %14s %18s" % ("kernel", "regs old/new", "spill old/new", "SASS instr old/new"))
-    for fn in sorted(set(so) | set(sn)):
-        a, b = po.get(fn, {}), pn.get(fn, {})
-        row = (fn, "%s/%s" % (a.get("regs"), b.get("regs")), "%s|%s" % (a.get("spill"), b.get("spill")), "%s/%s" % (so.get(fn), sn.get(fn)))
-        same = a == b and so.get(fn) == sn.get(fn)
-        lines.append("%-44s %14s %14s %18s%s" % (row + ("" if same else "   DIFFERS",)))
+    lines.append("%-44s %14s %14s %18s %10s" % ("kernel", "regs old/new", "spill old/new", "SASS instr old/new", "SASS code"))
+    for o, n in sorted(rows, key=lambda r: r[1]):
+        a, b = po.get(o, {}), pn.get(n, {})
+        io, inew = so.get(o), sn.get(n)
+        text = "-" if io is None or inew is None else ("same" if io == inew else "differs")
+        row = (n, "%s/%s" % (a.get("regs"), b.get("regs")), "%s|%s" % (a.get("spill"), b.get("spill")),
+               "%s/%s" % (io and len(io), inew and len(inew)), text)
+        same = a == b and text == "same"
+        line = "%-44s %14s %14s %18s %10s" % row
+        if o is not None and o != n:
+            line += "   (old: %s)" % o
+        lines.append(line + ("" if same else "   DIFFERS"))
         if not same:
-            differ.append(fn)
+            differ.append(n if inew is not None else o)
     lines.append("")
     lines.append("kernels that differ: %s" % (", ".join(differ) if differ else "none"))
     text = "\n".join(lines) + "\n"
     sys.stdout.write(text)
-    if len(sys.argv) > 5:
-        with open(sys.argv[5], "w") as f:
+    if out:
+        with open(out[0], "w") as f:
             f.write(text)
 
 
