@@ -9,7 +9,8 @@ Channel selector: None = every channel, an int, or a sequence of ints.  Planes a
 
 `channels=` on process / process_host advances only the listed channels (the reference's update() returns untouched when
 an input block is missing): the planes then have len(channels) rows, row i belonging to channels[i], and every other
-channel is left as it is (sdr_*_process_*_subset).  export_state / import_state move channels' whole state between
+channel is left as it is (sdr_*_process_*_subset).  `block_status=` on PreProcessorBatch.process / process_host receives the
+getters after every block, int32 [n_blocks, PP_BS_FIELDS, rows] (sdr_preproc_process_*_status).  export_state / import_state move channels' whole state between
 handles as opaque blobs, uint8 [n, state_bytes]."""
 import ctypes as C
 import os
@@ -28,7 +29,12 @@ EXPORTS = ["sdr_preproc_create", "sdr_preproc_destroy", "sdr_preproc_set", "sdr_
            "sdr_preproc_process_device_subset", "sdr_preproc_process_host_subset", "sdr_preproc_state_bytes", "sdr_preproc_export_state",
            "sdr_preproc_import_state", "sdr_iqgen_process_device_subset", "sdr_iqgen_process_host_subset", "sdr_iqgen_state_bytes",
            "sdr_iqgen_export_state", "sdr_iqgen_import_state", "sdr_grabber_process_device_subset", "sdr_grabber_state_bytes",
-           "sdr_grabber_export_state", "sdr_grabber_import_state", "sdr_grabber_process_device_snapshots"]
+           "sdr_grabber_export_state", "sdr_grabber_import_state", "sdr_grabber_process_device_snapshots",
+           "sdr_preproc_process_device_status", "sdr_preproc_process_host_status"]
+# per-block status records of the pre-processor (include/sdr_aux.h, SDR_PP_BS_*): int32 [n_blocks, PP_BS_FIELDS, rows], the
+# fields in the order of sdr_preproc_status
+(PP_BS_AUTO_DETECT, PP_BS_CORRECTION, PP_BS_FAILURE_COUNT, PP_BS_SUCCESS_COUNT, PP_BS_SAVED_SAMPLE, PP_BS_SWAP,
+ PP_BS_FIELDS) = range(7)
 
 
 class AuxError(RuntimeError):
@@ -91,6 +97,9 @@ def load_library(path=None):
             getattr(L, "sdr_%s_import_state" % k).argtypes = [vp, vp, u32, vp]
     if hasattr(L, "sdr_grabber_process_device_snapshots"):
         L.sdr_grabber_process_device_snapshots.argtypes = [vp, vp, u32, vp, vp, sz, u32, vp, vp, vp, vp]
+    if hasattr(L, "sdr_preproc_process_device_status"):
+        L.sdr_preproc_process_device_status.argtypes = [vp, vp, u32, vp, vp, sz, vp, vp, sz, u32, vp, vp]
+        L.sdr_preproc_process_host_status.argtypes = [vp, vp, u32, vp, vp, sz, vp, vp, sz, u32, vp]
     L.sdr_aux_last_error.restype = C.c_char_p
     L.sdr_aux_version.restype = C.c_char_p
     if path is None:
@@ -193,26 +202,40 @@ class PreProcessorBatch(_Base):
         return list(out)
 
     # ---- update() for every channel (or the listed ones), n_blocks times
-    def process(self, I, Q, I_out, Q_out, n_blocks=None, stream=None, channels=None):
+    def process(self, I, Q, I_out, Q_out, n_blocks=None, stream=None, channels=None, block_status=None):
+        """`block_status`: optional CUDA int32 tensor [n_blocks, PP_BS_FIELDS, rows], contiguous, that receives the getters
+        after every block on the same stream as the planes (sdr_preproc_process_device_status)."""
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
         p, n, keep, rows = _ids(channels, self.n_channels)
         _check_dev(rows, I, Q, I_out, Q_out)
         assert I.stride(0) == Q.stride(0) and I_out.stride(0) == Q_out.stride(0)
         sp = C.c_void_p(stream.cuda_stream) if stream is not None else None
-        args = (I.data_ptr(), Q.data_ptr(), I.stride(0), I_out.data_ptr(), Q_out.data_ptr(), I_out.stride(0), n_blocks, sp)
-        if channels is None:
-            self._check(self.L.sdr_preproc_process_device(self.h, *args))
+        args = (I.data_ptr(), Q.data_ptr(), I.stride(0), I_out.data_ptr(), Q_out.data_ptr(), I_out.stride(0), n_blocks)
+        if block_status is not None:
+            t = block_status
+            assert t.is_cuda and str(t.dtype) == "torch.int32" and t.is_contiguous() and tuple(t.shape) == (n_blocks, PP_BS_FIELDS, rows), \
+                "block_status: a contiguous CUDA int32 tensor [%d, %d, %d]" % (n_blocks, PP_BS_FIELDS, rows)
+            self._check(self.L.sdr_preproc_process_device_status(self.h, p, n, *args, t.data_ptr(), sp))
+        elif channels is None:
+            self._check(self.L.sdr_preproc_process_device(self.h, *args, sp))
         else:
-            self._check(self.L.sdr_preproc_process_device_subset(self.h, p, n, *args))
+            self._check(self.L.sdr_preproc_process_device_subset(self.h, p, n, *args, sp))
 
-    def process_host(self, I, Q, I_out, Q_out, n_blocks=None, channels=None):
+    def process_host(self, I, Q, I_out, Q_out, n_blocks=None, channels=None, block_status=None):
+        """`block_status`: optional numpy int32 array [n_blocks, PP_BS_FIELDS, rows], C-contiguous, filled before the call
+        returns (sdr_preproc_process_host_status)."""
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
         p, n, keep, rows = _ids(channels, self.n_channels)
         for a in (I, Q, I_out, Q_out):
             assert a.dtype == np.int16 and a.shape[0] == rows and a.strides[1] == 2
         assert I.strides[0] == Q.strides[0] and I_out.strides[0] == Q_out.strides[0]
         args = (I.ctypes.data, Q.ctypes.data, I.strides[0] // 2, I_out.ctypes.data, Q_out.ctypes.data, I_out.strides[0] // 2, n_blocks)
-        if channels is None:
+        if block_status is not None:
+            t = block_status
+            assert isinstance(t, np.ndarray) and t.dtype == np.int32 and t.flags.c_contiguous and t.shape == (n_blocks, PP_BS_FIELDS, rows), \
+                "block_status: a C-contiguous numpy int32 array [%d, %d, %d]" % (n_blocks, PP_BS_FIELDS, rows)
+            self._check(self.L.sdr_preproc_process_host_status(self.h, p, n, *args, t.ctypes.data))
+        elif channels is None:
             self._check(self.L.sdr_preproc_process_host(self.h, *args))
         else:
             self._check(self.L.sdr_preproc_process_host_subset(self.h, p, n, *args))

@@ -190,9 +190,31 @@ __global__ void __launch_bounds__(256) pp_static_kernel(const PpLaunch L, const 
   *dq = s.swap ? oa : ob;
 }
 
-/* detector off: savedSample after the call = the delayed rail's last input sample (PP.cpp:62-65 / 67-70) */
-template <bool kList>
-__global__ void pp_finish_kernel(const PpLaunch L, const uint32_t *ids) {
+/* detector off: savedSample after the call = the delayed rail's last input sample (PP.cpp:62-65 / 67-70).
+ * kRec: the per-block records of these rows instead (sdr_preproc_process_device_status), one thread per (block, row), rows
+ * fastest, so that each word's stores are coalesced across rows and the blocks of a row run in parallel (one thread per row
+ * looping over the blocks measured 2.1x the plain call's time on the feed-forward path, DESIGN section 10).  Only the saved
+ * sample moves: after block b it is the delayed rail's sample 128 b + 127, unchanged when the correction is 0; the thread of
+ * the last block stores it in the state.  Rows with the detector on belong to pp_detect_kernel, which runs after this kernel
+ * and changes their state. */
+template <bool kList, bool kRec>
+__global__ void pp_finish_kernel(const PpLaunch L, const uint32_t *ids, int32_t *rec) {
+  if (kRec) {
+    const unsigned long long idx = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const uint32_t n = L.n_channels, r = (uint32_t)(idx % n), b = (uint32_t)(idx / n);
+    if (b >= L.n_blocks) return;
+    const uint32_t ch = kList ? __ldg(ids + r) : r;
+    const PpState s = L.state[ch]; /* the saved sample read here is used only when the correction is 0: never written then */
+    if (s.autod) return;
+    const size_t at = (size_t)r * L.in_pitch + (size_t)b * 128 + 127;
+    const int32_t saved = s.corr == 1 ? (int32_t)L.I[at] : s.corr == -1 ? (int32_t)L.Q[at] : s.saved;
+    int32_t *o = rec + (size_t)b * SDR_PP_BS_FIELDS * n + r;
+    o[SDR_PP_BS_AUTO_DETECT * (size_t)n] = 0; o[SDR_PP_BS_CORRECTION * (size_t)n] = s.corr;
+    o[SDR_PP_BS_FAILURE_COUNT * (size_t)n] = s.fail; o[SDR_PP_BS_SUCCESS_COUNT * (size_t)n] = s.succ;
+    o[SDR_PP_BS_SAVED_SAMPLE * (size_t)n] = saved; o[SDR_PP_BS_SWAP * (size_t)n] = s.swap;
+    if (b == L.n_blocks - 1 && s.corr != 0) L.state[ch].saved = saved;
+    return;
+  }
   const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= L.n_channels) return;
   const uint32_t ch = kList ? __ldg(ids + r) : r;
@@ -206,12 +228,13 @@ __global__ void pp_finish_kernel(const PpLaunch L, const uint32_t *ids) {
  * after block.  Rows are staged through shared memory with whole-row (coalesced) transfers; a lane's row is 65 words from
  * its neighbour's (odd: no bank conflicts); the FFT buffer is [256][32] floats, lane-interleaved.  Warp 0 owns the
  * per-channel state (correction, counters); the butterflies of a stage, the conversions and the rows are split over
- * the warps with a CTA barrier between dependent phases. */
+ * the warps with a CTA barrier between dependent phases.  kRec: warp 0 also stores each lane's state after every block
+ * (sdr_preproc_process_device_status), column = the lane's plane row; padding lanes store nothing. */
 #define PP_W 8
 #define PP_ROW_WORDS 65
 #define PP_DETECT_SMEM (256 * 32 * 4 + 2 * 32 * PP_ROW_WORDS * 4 + 2 * 32 * 4)
-template <bool kList>
-__global__ void __launch_bounds__(32 * PP_W) pp_detect_kernel(const PpLaunch L, const uint32_t *ids) {
+template <bool kList, bool kRec>
+__global__ void __launch_bounds__(32 * PP_W) pp_detect_kernel(const PpLaunch L, const uint32_t *ids, int32_t *rec) {
   extern __shared__ __align__(16) unsigned char sm[];
   float *fft = reinterpret_cast<float *>(sm);
   uint32_t *rowI = reinterpret_cast<uint32_t *>(sm + 256 * 32 * 4), *rowQ = rowI + 32 * PP_ROW_WORDS;
@@ -268,6 +291,12 @@ __global__ void __launch_bounds__(32 * PP_W) pp_detect_kernel(const PpLaunch L, 
       }
       __syncthreads();
       if (w == 0 && det) pp_decide(mine, 32, s);
+    }
+    if (kRec && w == 0 && ch >= 0) { /* after pp_decide when detection ran in this block, after pp_correct_block otherwise */
+      const size_t n = L.n_channels;
+      int32_t *o = rec + (size_t)b * SDR_PP_BS_FIELDS * n + row;
+      o[SDR_PP_BS_AUTO_DETECT * n] = s.autod; o[SDR_PP_BS_CORRECTION * n] = s.corr; o[SDR_PP_BS_FAILURE_COUNT * n] = s.fail;
+      o[SDR_PP_BS_SUCCESS_COUNT * n] = s.succ; o[SDR_PP_BS_SAVED_SAMPLE * n] = s.saved; o[SDR_PP_BS_SWAP * n] = s.swap;
     }
     for (int r = w; r < 32; r += PP_W) {
       const int rr = __shfl_sync(0xFFFFFFFFu, row, r), sw = sh_swap[r];
@@ -606,6 +635,7 @@ struct sdr_preproc {
   bool auto_possible = false; /* some channel may have its detector on */
   uint64_t launches = 0;
   Staging stg;
+  int32_t *rec = nullptr; size_t rec_bytes = 0; /* device staging of the host form's block_status */
   IdList ids;
   std::vector<uint8_t> mark;
 };
@@ -614,8 +644,10 @@ extern "C" int sdr_preproc_create(sdr_preproc_t **out, uint32_t n_channels, int 
   if (!out || n_channels == 0) return fail(SDR_AUX_EINVAL, "sdr_preproc_create: bad arguments");
   CK(cudaSetDevice(device));
   if (int rc = upload_tables()) return rc;
-  CK(cudaFuncSetAttribute(pp_detect_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
-  CK(cudaFuncSetAttribute(pp_detect_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
+  CK(cudaFuncSetAttribute(pp_detect_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
+  CK(cudaFuncSetAttribute(pp_detect_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
+  CK(cudaFuncSetAttribute(pp_detect_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
+  CK(cudaFuncSetAttribute(pp_detect_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PP_DETECT_SMEM));
   sdr_preproc *h = new sdr_preproc();
   h->n = n_channels; h->device = device;
   if (cudaMalloc(&h->state, sizeof(PpState) * n_channels) != cudaSuccess || cudaMalloc(&h->list, 4 * (size_t)n_channels) != cudaSuccess ||
@@ -629,7 +661,7 @@ extern "C" int sdr_preproc_create(sdr_preproc_t **out, uint32_t n_channels, int 
 extern "C" void sdr_preproc_destroy(sdr_preproc_t *h) {
   if (!h) return;
   cudaSetDevice(h->device);
-  cudaFree(h->state); cudaFree(h->list); cudaFree(h->count); cudaFree(h->d_calls);
+  cudaFree(h->state); cudaFree(h->list); cudaFree(h->count); cudaFree(h->d_calls); cudaFree(h->rec);
   h->stg.release();
   h->ids.release();
   delete h;
@@ -680,9 +712,10 @@ extern "C" int sdr_preproc_get_status(sdr_preproc_t *h, const uint32_t *channels
   return 0;
 }
 
-/* a process call's launches; ids: the device id list of a subset call (kList), else unused */
+/* a process call's launches; ids: the device id list of a subset call (kList), else unused; rec: the call's per-block
+ * records (device, NULL: none), written by the records instantiations of the finish and detect kernels */
 template <bool kList>
-static int pp_launch(sdr_preproc *h, const PpLaunch &L, const uint32_t *ids, cudaStream_t st) {
+static int pp_launch(sdr_preproc *h, const PpLaunch &L, const uint32_t *ids, int32_t *rec, cudaStream_t st) {
   const uint32_t n = L.n_channels, tb = (n + 255) / 256;
   const unsigned long long threads = (unsigned long long)n * L.n_blocks * 16;
   const unsigned sb = (unsigned)((threads + 255) / 256);
@@ -692,64 +725,93 @@ static int pp_launch(sdr_preproc *h, const PpLaunch &L, const uint32_t *ids, cud
     h->launches++;
   }
   pp_static_kernel<kList><<<sb, 256, 0, st>>>(L, ids);
-  pp_finish_kernel<kList><<<tb, 256, 0, st>>>(L, ids);
+  if (rec) pp_finish_kernel<kList, true><<<(unsigned)(((unsigned long long)n * L.n_blocks + 255) / 256), 256, 0, st>>>(L, ids, rec);
+  else pp_finish_kernel<kList, false><<<tb, 256, 0, st>>>(L, ids, nullptr);
   h->launches += 2;
   if (h->auto_possible) {
-    pp_detect_kernel<kList><<<(n + 31) / 32, 32 * PP_W, PP_DETECT_SMEM, st>>>(L, ids);
+    if (rec) pp_detect_kernel<kList, true><<<(n + 31) / 32, 32 * PP_W, PP_DETECT_SMEM, st>>>(L, ids, rec);
+    else pp_detect_kernel<kList, false><<<(n + 31) / 32, 32 * PP_W, PP_DETECT_SMEM, st>>>(L, ids, nullptr);
     h->launches++;
   }
   return 0;
 }
 
-extern "C" int sdr_preproc_process_device_subset(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+static int check_block_status(const int32_t *block_status) {
+  if ((uintptr_t)block_status & 15) return fail(SDR_AUX_EINVAL, "block_status must be 16-byte aligned");
+  return 0;
+}
+
+extern "C" int sdr_preproc_process_device_status(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
                                                  size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks,
-                                                 void *cuda_stream) {
+                                                 int32_t *block_status, void *cuda_stream) {
   if (!h) return fail(SDR_AUX_EINVAL, "null handle");
   if (int rc = check_ids(channel_ids, n_ids, h->n, h->mark)) return rc;
   if (!Q) return fail(SDR_AUX_EINVAL, "null plane");
   if (int rc = check_planes(I, Q, I_out, Q_out, in_pitch, out_pitch, n_blocks)) return rc;
+  if (int rc = check_block_status(block_status)) return rc;
   CK(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)cuda_stream;
   if (int rc = pp_flush(h, st)) return rc; /* setters of every channel, listed or not, in call order */
   PpLaunch L = {I, Q, I_out, Q_out, in_pitch, out_pitch, h->state, n_ids, n_blocks, h->list, h->count};
   if (channel_ids) {
     if (int rc = h->ids.upload(channel_ids, n_ids, st)) return rc;
-    if (int rc = pp_launch<true>(h, L, h->ids.d, st)) return rc;
+    if (int rc = pp_launch<true>(h, L, h->ids.d, block_status, st)) return rc;
     if (int rc = h->ids.done(st)) return rc;
-  } else if (int rc = pp_launch<false>(h, L, nullptr, st)) {
+  } else if (int rc = pp_launch<false>(h, L, nullptr, block_status, st)) {
     return rc;
   }
   CK(cudaGetLastError());
   return 0;
 }
 
+extern "C" int sdr_preproc_process_device_subset(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+                                                 size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks,
+                                                 void *cuda_stream) {
+  return sdr_preproc_process_device_status(h, channel_ids, n_ids, I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, nullptr, cuda_stream);
+}
+
 extern "C" int sdr_preproc_process_device(sdr_preproc_t *h, const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out,
                                           int16_t *Q_out, size_t out_pitch, uint32_t n_blocks, void *cuda_stream) {
   if (!h) return fail(SDR_AUX_EINVAL, "null handle");
-  return sdr_preproc_process_device_subset(h, nullptr, h->n, I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, cuda_stream);
+  return sdr_preproc_process_device_status(h, nullptr, h->n, I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, nullptr, cuda_stream);
+}
+
+/* host block_status: the records are staged in h->rec on the device and copied out before the call returns */
+extern "C" int sdr_preproc_process_host_status(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+                                               size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks,
+                                               int32_t *block_status) {
+  if (!h || !I || !Q || !I_out || !Q_out || n_blocks == 0) return fail(SDR_AUX_EINVAL, "bad arguments");
+  if (int rc = check_ids(channel_ids, n_ids, h->n, h->mark)) return rc;
+  if (int rc = check_block_status(block_status)) return rc;
+  CK(cudaSetDevice(h->device));
+  if (int rc = h->stg.ensure(h->n, n_blocks, 4)) return rc;
+  const size_t rec_bytes = block_status ? (size_t)n_blocks * SDR_PP_BS_FIELDS * n_ids * sizeof(int32_t) : 0;
+  if (rec_bytes > h->rec_bytes) {
+    cudaFree(h->rec); h->rec = nullptr; h->rec_bytes = 0;
+    if (cudaMalloc(&h->rec, rec_bytes) != cudaSuccess) { h->rec = nullptr; return fail(SDR_AUX_ENOMEM, "cudaMalloc(block_status staging) failed"); }
+    h->rec_bytes = rec_bytes;
+  }
+  const size_t w = (size_t)n_blocks * 128 * 2, dp = h->stg.pitch * 2;
+  CK(cudaMemcpy2DAsync(h->stg.p[0], dp, I, in_pitch * 2, w, n_ids, cudaMemcpyHostToDevice, 0));
+  CK(cudaMemcpy2DAsync(h->stg.p[1], dp, Q, in_pitch * 2, w, n_ids, cudaMemcpyHostToDevice, 0));
+  if (int rc = sdr_preproc_process_device_status(h, channel_ids, n_ids, h->stg.p[0], h->stg.p[1], h->stg.pitch, h->stg.p[2], h->stg.p[3],
+                                                 h->stg.pitch, n_blocks, block_status ? h->rec : nullptr, nullptr)) return rc;
+  CK(cudaMemcpy2DAsync(I_out, out_pitch * 2, h->stg.p[2], dp, w, n_ids, cudaMemcpyDeviceToHost, 0));
+  CK(cudaMemcpy2DAsync(Q_out, out_pitch * 2, h->stg.p[3], dp, w, n_ids, cudaMemcpyDeviceToHost, 0));
+  if (block_status) CK(cudaMemcpyAsync(block_status, h->rec, rec_bytes, cudaMemcpyDeviceToHost, 0));
+  CK(cudaStreamSynchronize(0));
+  return 0;
 }
 
 extern "C" int sdr_preproc_process_host_subset(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
                                                size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks) {
-  if (!h || !I || !Q || !I_out || !Q_out || n_blocks == 0) return fail(SDR_AUX_EINVAL, "bad arguments");
-  if (int rc = check_ids(channel_ids, n_ids, h->n, h->mark)) return rc;
-  CK(cudaSetDevice(h->device));
-  if (int rc = h->stg.ensure(h->n, n_blocks, 4)) return rc;
-  const size_t w = (size_t)n_blocks * 128 * 2, dp = h->stg.pitch * 2;
-  CK(cudaMemcpy2DAsync(h->stg.p[0], dp, I, in_pitch * 2, w, n_ids, cudaMemcpyHostToDevice, 0));
-  CK(cudaMemcpy2DAsync(h->stg.p[1], dp, Q, in_pitch * 2, w, n_ids, cudaMemcpyHostToDevice, 0));
-  if (int rc = sdr_preproc_process_device_subset(h, channel_ids, n_ids, h->stg.p[0], h->stg.p[1], h->stg.pitch, h->stg.p[2], h->stg.p[3],
-                                                 h->stg.pitch, n_blocks, nullptr)) return rc;
-  CK(cudaMemcpy2DAsync(I_out, out_pitch * 2, h->stg.p[2], dp, w, n_ids, cudaMemcpyDeviceToHost, 0));
-  CK(cudaMemcpy2DAsync(Q_out, out_pitch * 2, h->stg.p[3], dp, w, n_ids, cudaMemcpyDeviceToHost, 0));
-  CK(cudaStreamSynchronize(0));
-  return 0;
+  return sdr_preproc_process_host_status(h, channel_ids, n_ids, I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, nullptr);
 }
 
 extern "C" int sdr_preproc_process_host(sdr_preproc_t *h, const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out,
                                         int16_t *Q_out, size_t out_pitch, uint32_t n_blocks) {
   if (!h) return fail(SDR_AUX_EINVAL, "bad arguments");
-  return sdr_preproc_process_host_subset(h, nullptr, h->n, I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks);
+  return sdr_preproc_process_host_status(h, nullptr, h->n, I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, nullptr);
 }
 
 extern "C" uint64_t sdr_preproc_launch_count(const sdr_preproc_t *h) { return h ? h->launches : 0; }

@@ -23,7 +23,9 @@ namespace sdr {
 
 class PreProcessorBatch {
  public:
-  explicit PreProcessorBatch(uint32_t n_channels, int device = 0) : h_(nullptr) { check(sdr_preproc_create(&h_, n_channels, device), "sdr_preproc_create"); }
+  explicit PreProcessorBatch(uint32_t n_channels, int device = 0) : h_(nullptr), n_channels_(n_channels) {
+    check(sdr_preproc_create(&h_, n_channels, device), "sdr_preproc_create");
+  }
   ~PreProcessorBatch() { sdr_preproc_destroy(h_); }
   PreProcessorBatch(const PreProcessorBatch &) = delete;
   PreProcessorBatch &operator=(const PreProcessorBatch &) = delete;
@@ -58,6 +60,29 @@ class PreProcessorBatch {
     check(sdr_preproc_process_host_subset(h_, ids.data(), (uint32_t)ids.size(), I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks),
           "sdr_preproc_process_host_subset");
   }
+  /* ... also the getters after every block: block_status int32 [n_blocks][SDR_PP_BS_FIELDS][rows], 16-byte aligned, device
+   * memory for process and host memory for process_host (sdr_preproc_process_*_status) */
+  void process(const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks,
+               int32_t *block_status, void *cuda_stream) {
+    check(sdr_preproc_process_device_status(h_, nullptr, n_channels_, I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, block_status, cuda_stream),
+          "sdr_preproc_process_device_status");
+  }
+  void process_host(const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks,
+                    int32_t *block_status) {
+    check(sdr_preproc_process_host_status(h_, nullptr, n_channels_, I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, block_status),
+          "sdr_preproc_process_host_status");
+  }
+  void process(const std::vector<uint32_t> &ids, const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out, int16_t *Q_out,
+               size_t out_pitch, uint32_t n_blocks, int32_t *block_status, void *cuda_stream) {
+    check(sdr_preproc_process_device_status(h_, ids.data(), (uint32_t)ids.size(), I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, block_status,
+                                            cuda_stream),
+          "sdr_preproc_process_device_status");
+  }
+  void process_host(const std::vector<uint32_t> &ids, const int16_t *I, const int16_t *Q, size_t in_pitch, int16_t *I_out, int16_t *Q_out,
+                    size_t out_pitch, uint32_t n_blocks, int32_t *block_status) {
+    check(sdr_preproc_process_host_status(h_, ids.data(), (uint32_t)ids.size(), I, Q, in_pitch, I_out, Q_out, out_pitch, n_blocks, block_status),
+          "sdr_preproc_process_host_status");
+  }
   static size_t state_bytes() { return sdr_preproc_state_bytes(); }
   std::vector<uint8_t> export_state(const std::vector<uint32_t> &ids) {
     std::vector<uint8_t> b(ids.size() * state_bytes());
@@ -76,6 +101,7 @@ class PreProcessorBatch {
     if (rc != SDR_AUX_OK) throw std::runtime_error(std::string(what) + ": " + sdr_aux_last_error());
   }
   sdr_preproc_t *h_;
+  uint32_t n_channels_;
 };
 
 class IQGeneratorBatch {

@@ -77,6 +77,31 @@ int sdr_preproc_process_device_subset(sdr_preproc_t *h, const uint32_t *channel_
                                       void *cuda_stream);
 int sdr_preproc_process_host_subset(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
                                     size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks);
+/* The same call, also returning the getters after every block: what a sketch polling getI2SerrorCompensation() and
+ * getAutoI2SerrorDetectionStatus() after each update() sees, and so which output blocks were made under which correction and
+ * at which block the detector stopped.  Ids, planes and checks are those of the *_subset calls, and the state the call
+ * leaves is the same.
+ *   block_status  int32 words, one per (block, field, row), block-major:
+ *                 block_status[((size_t)b * SDR_PP_BS_FIELDS + f) * n_ids + i] = field f of row i's channel right after its
+ *                 update() for block b, i.e. what sdr_preproc_get_status would return then (setters queued before the call
+ *                 apply before block 0; the last block's record equals get_status after the call).  Fields in the order of
+ *                 sdr_preproc_status; flags are 0 or 1, the saved sample is the int16 value sign-extended.  Every word of
+ *                 [n_blocks][SDR_PP_BS_FIELDS][n_ids] is written, rows with the detector off included (their fields are
+ *                 constant over the call except the saved sample, when the correction is +1 or -1).
+ *                 Device memory for the device form.  Host memory (pageable or pinned) for the host form: the records are
+ *                 staged on the device and copied out before the call returns.  Must be 16-byte aligned (SDR_AUX_EINVAL
+ *                 otherwise, nothing queued).  NULL: the call without records (the four process entry points above are
+ *                 these calls with NULL). */
+enum { /* 0 .. 5, then the count */
+  SDR_PP_BS_AUTO_DETECT, SDR_PP_BS_CORRECTION, SDR_PP_BS_FAILURE_COUNT, SDR_PP_BS_SUCCESS_COUNT, SDR_PP_BS_SAVED_SAMPLE, SDR_PP_BS_SWAP,
+  SDR_PP_BS_FIELDS
+};
+int sdr_preproc_process_device_status(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+                                      size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks,
+                                      int32_t *block_status, void *cuda_stream);
+int sdr_preproc_process_host_status(sdr_preproc_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q,
+                                    size_t in_pitch, int16_t *I_out, int16_t *Q_out, size_t out_pitch, uint32_t n_blocks,
+                                    int32_t *block_status);
 uint64_t sdr_preproc_launch_count(const sdr_preproc_t *h);
 /* Blob: the PP.h:66-72 members (correction, savedSample, both detector counters, swap, detector flag).  Export applies queued
  * setters first, as get_status does; import replaces the channel's state including setters queued for it, and setters

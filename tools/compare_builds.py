@@ -6,7 +6,8 @@ The logs are the `-Xptxas -v` output of `python -m audiosdr_b200.build --force` 
 `cuobjdump -sass` of the libraries.  Kernels are matched by mangled name; an OLD_KERNEL=NEW_KERNEL pair matches a kernel that
 was renamed (for example a twin that became a template instantiation).  A matched kernel is the same when its registers and
 spills are, and when its instructions are, each compared as text and encoding (control bits included) with the address
-removed.  Prints (and writes to OUT) one line per kernel and the list of kernels that differ."""
+removed.  Prints (and writes to OUT) one line per kernel, the list of kernels that differ and the list of kernels only the
+new build has."""
 import collections
 import re
 import subprocess
@@ -59,7 +60,7 @@ def main():
     po, pn, so, sn = ptxas(old_log), ptxas(new_log), sass(old_lib), sass(new_lib)
     renamed = set(pairs.values())
     rows = [(o, pairs.get(o, o)) for o in so] + [(None, n) for n in sn if n not in renamed and n not in so]
-    lines, differ = [], []
+    lines, differ, added = [], [], []
     lines.append("%-44s %14s %14s %18s %10s" % ("kernel", "regs old/new", "spill old/new", "SASS instr old/new", "SASS code"))
     for o, n in sorted(rows, key=lambda r: r[1]):
         a, b = po.get(o, {}), pn.get(n, {})
@@ -71,11 +72,16 @@ def main():
         line = "%-44s %14s %14s %18s %10s" % row
         if o is not None and o != n:
             line += "   (old: %s)" % o
+        if o is None:
+            lines.append(line + "   NEW")
+            added.append(n)
+            continue
         lines.append(line + ("" if same else "   DIFFERS"))
         if not same:
             differ.append(n if inew is not None else o)
     lines.append("")
     lines.append("kernels that differ: %s" % (", ".join(differ) if differ else "none"))
+    lines.append("kernels only in the new build: %s" % (", ".join(added) if added else "none"))
     text = "\n".join(lines) + "\n"
     sys.stdout.write(text)
     if out:
