@@ -3,7 +3,8 @@
 The hot path `AudioSDR::update()` (reference SRC/AudioSDRlib/AudioSDR.cpp:39-168) is implemented behind the C ABI of
 include/sdr_batch.h; the blocks either side of it (SURVEY 8f: AudioSDRpreProcessor, AudioIQgenerator) behind
 include/sdr_aux.h (`PreProcessorBatch`, `IQGeneratorBatch`).  `SdrBatch` mirrors the reference class's setter names with a
-channel selector.  The CUDA library is mandatory: importing works without it (so that the CPU-only test
+channel selector.  `GraphBatch` (include/sdr_graph.h) streams the sketch's whole graph -- front, grabber tap, receiver --
+from host memory in one ticketed call.  The CUDA library is mandatory: importing works without it (so that the CPU-only test
 tier can import the package), but constructing an SdrBatch raises unless libsdr_batch.so loads and a
 CUDA device accepts the sm_100a kernel image.  There is no CPU fallback.
 """
@@ -13,6 +14,7 @@ from .api import (AGC_FAST, AGC_MEDIUM, AGC_OFF, AGC_SLOW, AM, AUDIO_2100, AUDIO
                   BS_SAM_LOCKED, CW_LSB, CW_USB, FMT_F32, FMT_I16, LSB, SAM, SETTERS, USB, WSPR, ChannelStatus, SdrBatch,
                   SdrError, block_status_fields, lib_path, load_library)
 from .aux import AuxError, GrabberBatch, IQGeneratorBatch, PreProcessorBatch
-from .build import build_aux_library, build_library
+from .build import build_aux_library, build_graph_library, build_library
+from .graph import GraphBatch, GraphError
 
 __all__ = [n for n in dir() if not n.startswith("_")]

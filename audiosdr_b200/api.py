@@ -32,7 +32,8 @@ EXPORTS = ["sdr_batch_create", "sdr_batch_destroy", "sdr_batch_set", "sdr_batch_
            "sdr_batch_process", "sdr_batch_state_bytes", "sdr_batch_export_state", "sdr_batch_import_state",
            "sdr_batch_submit_host", "sdr_batch_wait_host", "sdr_batch_host_ticket", "sdr_batch_wait_host_ticket",
            "sdr_batch_process_device_status", "sdr_batch_process_host_status", "sdr_batch_submit_host_status",
-           "sdr_batch_process_device_subset", "sdr_batch_process_host_subset", "sdr_batch_submit_host_subset"]
+           "sdr_batch_process_device_subset", "sdr_batch_process_host_subset", "sdr_batch_submit_host_subset",
+           "sdr_batch_get_desc", "sdr_batch_release_stream"]
 
 # per-block status records (include/sdr_batch.h, SDR_BS_*): array [n_blocks, BS_FIELDS, n_channels] of 32-bit words
 (BS_AGC_GAIN, BS_AGC_ACTIVE, BS_AM_CARRIER, BS_SAM_FREQUENCY, BS_SAM_LOCKED, BS_NB_AVERAGE, BS_NB_DETECTED,

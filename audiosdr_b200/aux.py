@@ -30,7 +30,8 @@ EXPORTS = ["sdr_preproc_create", "sdr_preproc_destroy", "sdr_preproc_set", "sdr_
            "sdr_preproc_import_state", "sdr_iqgen_process_device_subset", "sdr_iqgen_process_host_subset", "sdr_iqgen_state_bytes",
            "sdr_iqgen_export_state", "sdr_iqgen_import_state", "sdr_grabber_process_device_subset", "sdr_grabber_state_bytes",
            "sdr_grabber_export_state", "sdr_grabber_import_state", "sdr_grabber_process_device_snapshots",
-           "sdr_preproc_process_device_status", "sdr_preproc_process_host_status"]
+           "sdr_preproc_process_device_status", "sdr_preproc_process_host_status",
+           "sdr_preproc_get_info", "sdr_iqgen_get_info", "sdr_grabber_get_info"]
 # per-block status records of the pre-processor (include/sdr_aux.h, SDR_PP_BS_*): int32 [n_blocks, PP_BS_FIELDS, rows], the
 # fields in the order of sdr_preproc_status
 (PP_BS_AUTO_DETECT, PP_BS_CORRECTION, PP_BS_FAILURE_COUNT, PP_BS_SUCCESS_COUNT, PP_BS_SAVED_SAMPLE, PP_BS_SWAP,

@@ -67,7 +67,34 @@ def build_aux_library(force=False, verbose=False):
     return AUX_LIB
 
 
+GRAPH_LIB = os.path.join(HERE, "libsdr_graph.so")
+GRAPH_DEPS = ["sdr_graph.cpp"] + [os.path.join("..", "..", "include", h) for h in ("sdr_graph.h", "sdr_batch.h", "sdr_aux.h")]
+
+
+def needs_graph_build():
+    if not os.path.exists(GRAPH_LIB):
+        return True
+    t = os.path.getmtime(GRAPH_LIB)
+    return any(os.path.getmtime(os.path.join(CSRC, d)) > t for d in GRAPH_DEPS) or any(os.path.getmtime(p) > t for p in (LIB, AUX_LIB))
+
+
+def build_graph_library(force=False, verbose=False):
+    """Builds audiosdr_b200/libsdr_graph.so (include/sdr_graph.h) after the two libraries it links; returns its path."""
+    build_library()
+    build_aux_library()
+    if not force and not needs_graph_build():
+        return GRAPH_LIB
+    # host code only (it drives the other two libraries' device entry points); $ORIGIN: they are found beside it
+    cmd = [_nvcc()] + NVCC_FLAGS + [os.path.join(CSRC, "sdr_graph.cpp"), "-o", GRAPH_LIB, "-L" + HERE, "-lsdr_batch", "-lsdr_aux",
+                                    "-Xlinker", "-rpath,$ORIGIN"]
+    r = subprocess.run(cmd, capture_output=True, text=True)
+    if r.returncode != 0:
+        raise RuntimeError("nvcc failed:\n" + " ".join(cmd) + "\n" + r.stdout + r.stderr)
+    return GRAPH_LIB
+
+
 if __name__ == "__main__":
     import sys
     print(build_library(force="--force" in sys.argv, verbose=True))
     print(build_aux_library(force="--force" in sys.argv, verbose=True))
+    print(build_graph_library(force="--force" in sys.argv))

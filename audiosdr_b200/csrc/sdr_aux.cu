@@ -1253,5 +1253,15 @@ extern "C" int sdr_grabber_import_state(sdr_grabber_t *h, const uint32_t *channe
   return 0;
 }
 
+template <class H>
+static int get_info(const H *h, uint32_t *n_channels, int *device) {
+  if (!h || !n_channels || !device) return fail(SDR_AUX_EINVAL, "get_info: bad arguments");
+  *n_channels = h->n; *device = h->device;
+  return 0;
+}
+extern "C" int sdr_preproc_get_info(const sdr_preproc_t *h, uint32_t *n_channels, int *device) { return get_info(h, n_channels, device); }
+extern "C" int sdr_iqgen_get_info(const sdr_iqgen_t *h, uint32_t *n_channels, int *device) { return get_info(h, n_channels, device); }
+extern "C" int sdr_grabber_get_info(const sdr_grabber_t *h, uint32_t *n_channels, int *device) { return get_info(h, n_channels, device); }
+
 extern "C" const char *sdr_aux_last_error(void) { return g_err.c_str(); }
 extern "C" const char *sdr_aux_version(void) { return "audiosdr_b200 aux 0.1 (sm_100a)"; }

@@ -947,6 +947,20 @@ int sdr_batch_wait_host(sdr_batch_t *h) {
 
 uint64_t sdr_batch_host_ticket(const sdr_batch_t *h) { return h ? h->host_calls : 0; }
 
+int sdr_batch_get_desc(const sdr_batch_t *h, sdr_batch_desc *out) {
+  if (!h || !out) return fail(SDR_ERR_ARG, "get_desc: bad arguments");
+  *out = h->desc;
+  return SDR_OK;
+}
+
+int sdr_batch_release_stream(sdr_batch_t *h, void *stream) {
+  if (!h) return fail(SDR_ERR_ARG, "release_stream: null handle");
+  if (h->last_stream != stream) return SDR_OK;
+  if (dev_select(h->desc.device) || dev_sync(stream)) return SDR_ERR_CUDA;
+  h->last_stream = nullptr;
+  return SDR_OK;
+}
+
 int sdr_batch_wait_host_ticket(sdr_batch_t *h, uint64_t ticket) {
   if (!h) return fail(SDR_ERR_ARG, "wait_host_ticket: bad arguments");
   if (ticket > h->host_calls) return fail(SDR_ERR_ARG, "wait_host_ticket: no such call yet");

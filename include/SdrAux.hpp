@@ -192,6 +192,7 @@ class GrabberBatch {
   bool grab(uint32_t c, int16_t *destination) { const int r = sdr_grabber_grab(h_, &c, 1, destination); if (r < 0) check(r, "sdr_grabber_grab"); return r > 0; }
   /* spectrum tap: power[256] of the 256-point FFT of channel c's snapshot (natural bin order); false before the first complete pair */
   bool spectrum(uint32_t c, float *power) { const int r = sdr_grabber_spectrum(h_, &c, 1, power); if (r < 0) check(r, "sdr_grabber_spectrum"); return r > 0; }
+  sdr_grabber_t *handle() { return h_; }
 
  private:
   static void check(int rc, const char *what) {

@@ -189,6 +189,11 @@ int sdr_grabber_import_state(sdr_grabber_t *h, const uint32_t *channel_ids, uint
 int sdr_grabber_spectrum(sdr_grabber_t *h, const uint32_t *channels, uint32_t n, float *power);
 int sdr_grabber_spectrum_device(sdr_grabber_t *h, const uint32_t *d_channels, uint32_t n, float *d_power, void *cuda_stream);
 
+/* The channel count and device a handle was created with (for code that drives handles it did not create, e.g. sdr_graph.h) */
+int sdr_preproc_get_info(const sdr_preproc_t *h, uint32_t *n_channels, int *device);
+int sdr_iqgen_get_info(const sdr_iqgen_t *h, uint32_t *n_channels, int *device);
+int sdr_grabber_get_info(const sdr_grabber_t *h, uint32_t *n_channels, int *device);
+
 const char *sdr_aux_last_error(void);
 const char *sdr_aux_version(void);
 

@@ -260,6 +260,12 @@ int sdr_batch_import_state(sdr_batch_t *h, const uint32_t *channel_ids, uint32_t
  * groups[cls] = CTA launches counted. */
 int sdr_batch_get_role_profile(sdr_batch_t *h, uint64_t *busy28, uint64_t *total2, uint64_t *groups2);
 
+/* The descriptor the handle was created with (for code that drives a handle it did not create, e.g. sdr_graph.h). */
+int sdr_batch_get_desc(const sdr_batch_t *h, sdr_batch_desc *out);
+/* The handle orders its next call, its getters and its destruction after the last stream it was given; call this before
+ * destroying a stream the handle may have run on: if it was that stream, its work is waited for and the handle forgets it. */
+int sdr_batch_release_stream(sdr_batch_t *h, void *cuda_stream);
+
 /* Kernels this handle has launched so far (for the benchmark's gpu_launches claim). */
 uint64_t sdr_batch_launch_count(const sdr_batch_t *h);
 const char *sdr_batch_last_error(void);
