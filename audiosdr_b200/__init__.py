@@ -13,7 +13,7 @@ from .api import (AGC_FAST, AGC_MEDIUM, AGC_OFF, AGC_SLOW, AM, AUDIO_2100, AUDIO
                   BS_AGC_GAIN, BS_AM_CARRIER, BS_FIELDS, BS_NAMES, BS_NB_AVERAGE, BS_NB_DETECTED, BS_SAM_FREQUENCY,
                   BS_SAM_LOCKED, CW_LSB, CW_USB, FMT_F32, FMT_I16, LSB, SAM, SETTERS, USB, WSPR, ChannelStatus, SdrBatch,
                   SdrError, block_status_fields, lib_path, load_library)
-from .aux import AuxError, GrabberBatch, IQGeneratorBatch, PreProcessorBatch
+from .aux import AuxError, GrabberBatch, IQGeneratorBatch, PreProcessorBatch, WaterfallBatch
 from .build import build_aux_library, build_graph_library, build_library
 from .graph import GraphBatch, GraphError
 

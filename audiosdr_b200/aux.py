@@ -4,6 +4,7 @@ include/sdr_aux.h (audiosdr_b200/libsdr_aux.so; CUDA only, no CPU fallback):
   PreProcessorBatch  <-  class AudioSDRpreProcessor    (AudioSDRpreProcessor.h:49-73): same method names, channel selector first
   IQGeneratorBatch   <-  class AudioIQgenerator        (AudioIQgenerator.h:49-107)
   GrabberBatch       <-  class AudioGrabberComplex256  (AudioGrabberComplex256.h:46-64)
+  WaterfallBatch     averaged waterfall lines per channel over the grabber's per-pair spectra (sdr_waterfall_*)
 
 Channel selector: None = every channel, an int, or a sequence of ints.  Planes are int16 [n_channels, >= 128*n_blocks].
 
@@ -31,7 +32,11 @@ EXPORTS = ["sdr_preproc_create", "sdr_preproc_destroy", "sdr_preproc_set", "sdr_
            "sdr_iqgen_export_state", "sdr_iqgen_import_state", "sdr_grabber_process_device_subset", "sdr_grabber_state_bytes",
            "sdr_grabber_export_state", "sdr_grabber_import_state", "sdr_grabber_process_device_snapshots",
            "sdr_preproc_process_device_status", "sdr_preproc_process_host_status",
-           "sdr_preproc_get_info", "sdr_iqgen_get_info", "sdr_grabber_get_info"]
+           "sdr_preproc_get_info", "sdr_iqgen_get_info", "sdr_grabber_get_info", "sdr_grabber_process_device_waterfall",
+           "sdr_grabber_process_device_waterfall_at"]
+# the waterfall handle's own functions (sdr_waterfall_*)
+WATERFALL_EXPORTS = ["sdr_waterfall_create", "sdr_waterfall_destroy", "sdr_waterfall_get_info", "sdr_waterfall_state_bytes",
+                     "sdr_waterfall_export_state", "sdr_waterfall_import_state"]
 # per-block status records of the pre-processor (include/sdr_aux.h, SDR_PP_BS_*): int32 [n_blocks, PP_BS_FIELDS, rows], the
 # fields in the order of sdr_preproc_status
 (PP_BS_AUTO_DETECT, PP_BS_CORRECTION, PP_BS_FAILURE_COUNT, PP_BS_SUCCESS_COUNT, PP_BS_SAVED_SAMPLE, PP_BS_SWAP,
@@ -101,6 +106,15 @@ def load_library(path=None):
     if hasattr(L, "sdr_preproc_process_device_status"):
         L.sdr_preproc_process_device_status.argtypes = [vp, vp, u32, vp, vp, sz, vp, vp, sz, u32, vp, vp]
         L.sdr_preproc_process_host_status.argtypes = [vp, vp, u32, vp, vp, sz, vp, vp, sz, u32, vp]
+    if hasattr(L, "sdr_waterfall_create"):
+        L.sdr_waterfall_create.argtypes = [C.POINTER(vp), u32, C.c_int, u32]
+        L.sdr_waterfall_destroy.argtypes = [vp]; L.sdr_waterfall_destroy.restype = None
+        L.sdr_waterfall_get_info.argtypes = [vp, vp, vp, vp]
+        L.sdr_waterfall_state_bytes.argtypes = []; L.sdr_waterfall_state_bytes.restype = sz
+        L.sdr_waterfall_export_state.argtypes = [vp, vp, u32, vp]
+        L.sdr_waterfall_import_state.argtypes = [vp, vp, u32, vp]
+        L.sdr_grabber_process_device_waterfall.argtypes = [vp, vp, vp, u32, vp, vp, sz, u32, vp, vp, vp]
+        L.sdr_grabber_process_device_waterfall_at.argtypes = [vp, vp, vp, u32, vp, vp, sz, u32, vp, sz, vp, vp, vp]
     L.sdr_aux_last_error.restype = C.c_char_p
     L.sdr_aux_version.restype = C.c_char_p
     if path is None:
@@ -315,16 +329,28 @@ class GrabberBatch(_Base):
 
     __del__ = close
 
-    def process(self, I, Q, n_blocks=None, stream=None, channels=None, snapshots=None, power=None):
+    def process(self, I, Q, n_blocks=None, stream=None, channels=None, snapshots=None, power=None, waterfall=None, lines=None):
         """update() x n_blocks on every channel (or the listed ones).  snapshots (CUDA int16 [rows, S, 512]) and/or power
         (CUDA float32 [rows, S, 256]), S = (n_blocks + 1) // 2: every snapshot the call publishes and its spectrum, slot k of
         row i = the k-th pair the call completes for that row's channel (sdr_grabber_process_device_snapshots).  Then returns
-        counts, numpy uint32 [rows]: the slots written per row."""
+        counts, numpy uint32 [rows]: the slots written per row.
+        waterfall (a WaterfallBatch) with lines (CUDA float32 [rows, waterfall.line_slots(n_blocks), 256]): the call also
+        advances the waterfall and writes the lines it completes (sdr_grabber_process_device_waterfall); counts are then the
+        lines written per row.  Not combined with snapshots / power."""
         n_blocks = int(n_blocks if n_blocks is not None else I.shape[1] // N_BLOCK)
         p, n, keep, rows = _ids(channels, self.n_channels)
         _check_dev(rows, I, Q)
         assert I.stride(0) == Q.stride(0)
         sp = C.c_void_p(stream.cuda_stream) if stream is not None else None
+        if waterfall is not None:
+            assert snapshots is None and power is None, "waterfall lines and per-slot outputs are separate calls"
+            t = lines
+            assert t is not None and t.is_cuda and str(t.dtype) == "torch.float32" and t.is_contiguous() and \
+                tuple(t.shape) == (rows, waterfall.line_slots(n_blocks), 256), "lines: a contiguous CUDA float32 tensor [rows, Lmax, 256]"
+            counts = np.zeros(rows, np.uint32)
+            self._check(self.L.sdr_grabber_process_device_waterfall(self.h, waterfall.h, p, rows, I.data_ptr(), Q.data_ptr(), I.stride(0),
+                                                                    n_blocks, t.data_ptr(), counts.ctypes.data, sp))
+            return counts
         if snapshots is not None or power is not None:
             S = (n_blocks + 1) // 2
             for t, dt, w in ((snapshots, "torch.int16", 512), (power, "torch.float32", 256)):
@@ -381,3 +407,27 @@ class GrabberBatch(_Base):
         if r < 0:
             self._check(r)
         return out if r > 0 else None
+
+
+class WaterfallBatch(_Base):
+    """Averaged waterfall lines per channel (include/sdr_aux.h, sdr_waterfall_*): the grabber's per-pair power spectra
+    averaged K at a time in pair order, across calls, bit for bit the same however the stream is cut into calls.  Driven by
+    GrabberBatch.process(..., waterfall=, lines=) and GraphBatch(..., waterfall=)."""
+    _kind = "waterfall"
+
+    def __init__(self, n_channels, K, device=0, _lib=None):
+        self.L = _lib or load_library()
+        self.n_channels, self.K = int(n_channels), int(K)
+        self.h = C.c_void_p()
+        self._check(self.L.sdr_waterfall_create(C.byref(self.h), self.n_channels, int(device), self.K))
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.sdr_waterfall_destroy(self.h)
+            self.h = None
+
+    __del__ = close
+
+    def line_slots(self, n_blocks):
+        """Lmax: the line slots per row of a call of n_blocks blocks."""
+        return (self.K - 1 + (int(n_blocks) + 1) // 2) // self.K

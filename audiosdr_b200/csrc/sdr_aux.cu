@@ -417,9 +417,12 @@ __device__ __forceinline__ void fft_bfly(float &ar, float &ai, float &br, float 
     _Pragma("unroll") for (int r = 0; r < 8; r++) { xr[r] = sr[fft_swz(IDX_R)]; xi[r] = si[fft_swz(IDX_R)]; } \
   } while (0)
 
-/* w[i]: point 8 l + i as (re | im << 16), layout L0.  power[256] of the snapshot (natural bin order) to `out`.  sm: the
- * warp's FFT_WARP_WORDS words of shared memory. */
-__device__ __forceinline__ void fft256_power(const uint32_t w[8], float *sm, const FftTw &t, int l, float *out) {
+/* the bin of register r of lane l after fft256_pow: brev3(r) * 32 + brev5(l) */
+__device__ __forceinline__ int fft_bin(int r, int l) { return (((r & 1) << 2) | (r & 2) | (r >> 2)) * 32 + (int)(__brev((unsigned)l) >> 27); }
+
+/* w[i]: point 8 l + i as (re | im << 16), layout L0.  pw[r] <- the power of bin fft_bin(r, l).  sm: the warp's
+ * FFT_WARP_WORDS words of shared memory. */
+__device__ __forceinline__ void fft256_pow(const uint32_t w[8], float *sm, const FftTw &t, int l, float pw[8]) {
   float *sr = sm, *si = sm + 256;
   float xr[8], xi[8];
 #pragma unroll
@@ -443,12 +446,22 @@ __device__ __forceinline__ void fft256_power(const uint32_t w[8], float *sm, con
   for (int r = 0; r < 8; r++) if (!(r & 2)) fft_bfly(xr[r], xi[r], xr[r + 2], xi[r + 2], fft_tw(64 * (r & 1))); /* j = b0, step 64 */
 #pragma unroll
   for (int r = 0; r < 8; r += 2) fft_bfly(xr[r], xi[r], xr[r + 1], xi[r + 1], fft_tw(0));
+#pragma unroll
+  for (int r = 0; r < 8; r++) {
+    const float a = xr[r] * xr[r], b = xi[r] * xi[r];
+    pw[r] = a + b;
+  }
+}
+
+/* power[256] of the snapshot (natural bin order) to `out` */
+__device__ __forceinline__ void fft256_power(const uint32_t w[8], float *sm, const FftTw &t, int l, float *out) {
+  float pw[8];
+  fft256_pow(w, sm, t, l, pw);
   const int col = (int)(__brev((unsigned)l) >> 27);
 #pragma unroll
   for (int r = 0; r < 8; r++) {
     const int row = ((r & 1) << 2) | (r & 2) | (r >> 2); /* brev3 */
-    const float a = xr[r] * xr[r], b = xi[r] * xi[r];
-    out[row * 32 + col] = a + b;
+    out[row * 32 + col] = pw[r];
   }
 }
 
@@ -458,6 +471,20 @@ __device__ __forceinline__ void grab_interleave8(const int16_t *I, const int16_t
   const uint32_t ai[4] = {a.x, a.y, a.z, a.w}, bi[4] = {b.x, b.y, b.z, b.w};
 #pragma unroll
   for (int i = 0; i < 4; i++) { w[2 * i] = __byte_perm(ai[i], bi[i], 0x5410); w[2 * i + 1] = __byte_perm(ai[i], bi[i], 0x7632); }
+}
+
+/* lane l's 8 points of slot k of row r (channel ch, pair phase p before the call): the pair the call's block e = 2k + 1 - p
+ * completes, blocks e - 1 and e, block -1 being the carried half.  Lanes 0-15 hold the first block, lanes 16-31 the second. */
+__device__ __forceinline__ void grab_slot_points(const GrabLaunch &L, uint32_t r, uint32_t ch, int p, uint32_t k, int l, uint32_t w[8]) {
+  const int e = 2 * (int)k + 1 - p, blk = l < 16 ? e - 1 : e, s8 = 8 * (l & 15);
+  if (blk < 0) {
+    const uint4 *c = reinterpret_cast<const uint4 *>(L.half + (size_t)ch * 256 + 2 * s8);
+    const uint4 u = c[0], v = c[1];
+    w[0] = u.x; w[1] = u.y; w[2] = u.z; w[3] = u.w; w[4] = v.x; w[5] = v.y; w[6] = v.z; w[7] = v.w;
+  } else {
+    const size_t off = (size_t)r * L.pitch + (size_t)blk * 128 + s8;
+    grab_interleave8(L.I + off, L.Q + off, w);
+  }
 }
 
 #define FFT_THREADS 256
@@ -479,16 +506,8 @@ __global__ void __launch_bounds__(FFT_THREADS) grab_snapshots_kernel(const GrabL
     const uint32_t ch = L.ids ? __ldg(L.ids + r) : r;
     const int p = (int)L.phase[ch];
     if (k >= (p + L.n_blocks) / 2) continue; /* uniform over the warp */
-    const int e = 2 * (int)k + 1 - p, blk = l < 16 ? e - 1 : e, s8 = 8 * (l & 15);
     uint32_t w[8];
-    if (blk < 0) {
-      const uint4 *c = reinterpret_cast<const uint4 *>(L.half + (size_t)ch * 256 + 2 * s8);
-      const uint4 u = c[0], v = c[1];
-      w[0] = u.x; w[1] = u.y; w[2] = u.z; w[3] = u.w; w[4] = v.x; w[5] = v.y; w[6] = v.z; w[7] = v.w;
-    } else {
-      const size_t off = (size_t)r * L.pitch + (size_t)blk * 128 + s8;
-      grab_interleave8(L.I + off, L.Q + off, w);
-    }
+    grab_slot_points(L, r, ch, p, k, l, w);
     if (snaps) {
       uint4 *d = reinterpret_cast<uint4 *>(snaps + it * 512 + 16 * l);
       d[0] = make_uint4(w[0], w[1], w[2], w[3]);
@@ -496,6 +515,84 @@ __global__ void __launch_bounds__(FFT_THREADS) grab_snapshots_kernel(const GrabL
     }
     if (power) fft256_power(w, sm[wib], t, l, power + it * 256);
   }
+}
+
+/* Averaged waterfall lines (sdr_grabber_process_device_waterfall), launched before grab_update_kernel on the call's stream:
+ * it reads the pair phases and carried halves as grab_snapshots_kernel does and averages the same slots' power K at a time.
+ * A channel holds h < K pairs summed in acc[sel] (st = h << 1 | sel).  Number the pairs v = h + k for the call's slot k,
+ * v < h standing for the held sum: with C = (p + n_blocks) / 2 slots the row completes nl = (h + C) / K lines, line m
+ * summing v = mK .. mK + K - 1 in order, one rounding per add, then one IEEE division by K per bin.  Item (row, m), m <= Lmax,
+ * one warp each, grid-stride: m < nl writes line m to lines[r * line_pitch + first[r] + m]; m == nl with (h + C) % K != 0
+ * sums the trailing partial into acc[sel ^ 1].  Line 0 (or, when nl == 0, the partial) reads acc[sel], so reader and
+ * writer never share a buffer; wf_advance_kernel then flips sel and stores the new h for the listed rows only, because the
+ * other channels' sums stay where they are.  Lane l accumulates bins fft_bin(0..7, l) in registers. */
+struct WfLaunch {
+  float *acc;                    /* [2][n_channels][256] */
+  uint32_t *st;                  /* [n_channels]: pairs held << 1 | accumulator buffer */
+  float *lines;                  /* [n_rows][line_pitch][256] */
+  const uint32_t *first;         /* device [n_rows]: row r's first line slot, NULL: 0 */
+  unsigned long long line_pitch; /* in lines */
+  uint32_t n_channels, K, Lmax;
+};
+__global__ void __launch_bounds__(FFT_THREADS) grab_waterfall_kernel(const GrabLaunch L, const WfLaunch W) {
+  __shared__ float sm[FFT_THREADS / 32][FFT_WARP_WORDS];
+  const int l = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  FftTw t;
+  fft_load_tw(t, l);
+  /* opaque to the compiler from here: kept in registers, instead of reloaded in every FFT of the loop below from constant
+   * memory at per-lane addresses, which serialises */
+  float *tf = reinterpret_cast<float *>(&t);
+#pragma unroll
+  for (int i = 0; i < (int)(sizeof(FftTw) / 4); i++) asm volatile("" : "+f"(tf[i]));
+  const uint32_t per = W.Lmax + 1;
+  const unsigned long long items = (unsigned long long)L.n_rows * per, nw = (unsigned long long)gridDim.x * (FFT_THREADS / 32);
+  for (unsigned long long it = (unsigned long long)blockIdx.x * (FFT_THREADS / 32) + wib; it < items; it += nw) {
+    const uint32_t r = (uint32_t)(it / per), m = (uint32_t)(it - (unsigned long long)r * per);
+    const uint32_t ch = L.ids ? __ldg(L.ids + r) : r;
+    const int p = (int)L.phase[ch];
+    const uint32_t s = W.st[ch], h = s >> 1, sel = s & 1;
+    const uint32_t T = h + (p + L.n_blocks) / 2, nl = T / W.K;
+    if (m > nl || (m == nl && T % W.K == 0)) continue; /* uniform over the warp */
+    uint32_t v = m * W.K;
+    const uint32_t v1 = min(v + W.K, T);
+    float acc[8];
+    if (v < h) { /* line 0 (or the partial) continues the held sum */
+      const float *a = W.acc + ((size_t)sel * W.n_channels + ch) * 256;
+#pragma unroll
+      for (int j = 0; j < 8; j++) acc[j] = a[fft_bin(j, l)];
+      v = h;
+    } else {
+#pragma unroll
+      for (int j = 0; j < 8; j++) acc[j] = 0.0f;
+    }
+    for (; v < v1; v++) {
+      uint32_t w[8];
+      float pw[8];
+      grab_slot_points(L, r, ch, p, v - h, l, w);
+      fft256_pow(w, sm[wib], t, l, pw);
+#pragma unroll
+      for (int j = 0; j < 8; j++) acc[j] = acc[j] + pw[j];
+    }
+    if (m < nl) {
+      float *o = W.lines + ((size_t)r * W.line_pitch + (W.first ? __ldg(W.first + r) : 0u) + m) * 256;
+      const float k = (float)W.K;
+#pragma unroll
+      for (int j = 0; j < 8; j++) o[fft_bin(j, l)] = __fdiv_rn(acc[j], k);
+    } else {
+      float *a = W.acc + ((size_t)(sel ^ 1) * W.n_channels + ch) * 256;
+#pragma unroll
+      for (int j = 0; j < 8; j++) a[fft_bin(j, l)] = acc[j];
+    }
+  }
+}
+
+/* after grab_waterfall_kernel, before grab_update_kernel moves the phases on: the listed rows' new held count and buffer */
+__global__ void wf_advance_kernel(const GrabLaunch L, uint32_t *st, uint32_t K) {
+  const uint32_t r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= L.n_rows) return;
+  const uint32_t ch = L.ids ? __ldg(L.ids + r) : r;
+  const uint32_t s = st[ch];
+  st[ch] = ((((s >> 1) + (L.phase[ch] + L.n_blocks) / 2) % K) << 1) | ((s & 1) ^ 1);
 }
 
 /* Spectrum tap on the snapshots (SURVEY 8f row 3: the panadapter that consumes grab(); sdr_grabber_spectrum[_device]): power
@@ -1064,32 +1161,137 @@ static unsigned fft_grid(const sdr_grabber *h, unsigned long long items) {
   return (unsigned)std::max(1ull, std::min(need, cap));
 }
 
-extern "C" int sdr_grabber_process_device_snapshots(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I,
-                                                    const int16_t *Q, size_t pitch, uint32_t n_blocks, int16_t *snapshots, float *power,
-                                                    uint32_t *counts, void *cuda_stream) {
+/* ------------------------------------------------------------------ waterfall ---- */
+/* Per channel: the pairs held (< K) and which of its two accumulator buffers holds their sum.  The device words st[] are
+ * what the kernels read and advance; the host mirrors them (held, sel) for the line counts and the checkpoints, as the
+ * grabber mirrors its pair phases. */
+struct sdr_waterfall {
+  uint32_t n = 0; int device = 0; uint32_t K = 1;
+  float *acc = nullptr;   /* [2][n][256] */
+  uint32_t *d_st = nullptr;
+  std::vector<uint32_t> held;
+  std::vector<uint8_t> sel;
+  int ctas = 1;           /* resident CTAs of grab_waterfall_kernel on the whole device: its grid */
+  IdList first;           /* device copy of a call's first line slots per row */
+};
+
+static uint32_t wf_lmax(uint32_t K, uint32_t n_blocks) { return (uint32_t)(((unsigned long long)K - 1 + (n_blocks + 1) / 2) / K); }
+
+/* The grabber's process call with its optional outputs: snapshots / power per slot (grab_snapshots_kernel) and waterfall
+ * lines (wf != NULL: grab_waterfall_kernel; counts then receive the lines per row, else the slots per row).  Every check
+ * comes before anything is queued. */
+static int grab_process(sdr_grabber *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I, const int16_t *Q, size_t pitch,
+                        uint32_t n_blocks, int16_t *snapshots, float *power, uint32_t *counts, sdr_waterfall *wf, float *lines,
+                        size_t line_pitch, const uint32_t *first_line, cudaStream_t st) {
   if (!h || !I || !Q || n_blocks == 0) return fail(SDR_AUX_EINVAL, "bad arguments");
   if (int rc = check_ids(channel_ids, n_ids, h->n, h->mark)) return rc;
   if ((pitch & 7) || pitch < (size_t)n_blocks * 128 || (((uintptr_t)I | (uintptr_t)Q) & 15)) return fail(SDR_AUX_EINVAL, "planes must be 16-byte aligned, pitch a multiple of 8 and >= 128*n_blocks");
   if (((uintptr_t)snapshots | (uintptr_t)power) & 15) return fail(SDR_AUX_EINVAL, "snapshots and power must be 16-byte aligned");
+  if (wf) {
+    if (wf->n != h->n || wf->device != h->device) return fail(SDR_AUX_EINVAL, "the waterfall must have the grabber's device and channel count");
+    if (!lines || ((uintptr_t)lines & 15)) return fail(SDR_AUX_EINVAL, "lines must be non-NULL and 16-byte aligned");
+    for (uint32_t i = 0; i < n_ids; i++) {
+      const uint32_t c = channel_ids ? channel_ids[i] : i;
+      const unsigned long long nl = (wf->held[c] + (h->phase[c] + n_blocks) / 2) / wf->K;
+      if ((first_line ? first_line[i] : 0ull) + nl > line_pitch) return fail(SDR_AUX_EINVAL, "a row's lines run past line_pitch");
+    }
+  }
   CK(cudaSetDevice(h->device));
-  cudaStream_t st = (cudaStream_t)cuda_stream;
   if (channel_ids) { if (int rc = h->ids.upload(channel_ids, n_ids, st)) return rc; }
+  if (wf && first_line) { if (int rc = wf->first.upload(first_line, n_ids, st)) return rc; }
   GrabLaunch L = {I, Q, pitch, h->half, h->outb, h->d_phase, h->d_valid, channel_ids ? h->ids.d : nullptr, n_ids, n_blocks};
   if (snapshots || power) { /* reads the phases and carried halves before grab_update_kernel moves them on */
     grab_snapshots_kernel<<<fft_grid(h, (unsigned long long)n_ids * ((n_blocks + 1) / 2)), FFT_THREADS, 0, st>>>(L, snapshots, power);
     CK(cudaGetLastError());
   }
+  if (wf) { /* the same, then the waterfall's words move on, then the phases */
+    const uint32_t Lmax = wf_lmax(wf->K, n_blocks);
+    const WfLaunch W = {wf->acc, wf->d_st, lines, first_line ? wf->first.d : nullptr, line_pitch, wf->n, wf->K, Lmax};
+    const unsigned long long need = ((unsigned long long)n_ids * (Lmax + 1) + FFT_THREADS / 32 - 1) / (FFT_THREADS / 32);
+    grab_waterfall_kernel<<<(unsigned)std::max(1ull, std::min(need, (unsigned long long)wf->ctas)), FFT_THREADS, 0, st>>>(L, W);
+    CK(cudaGetLastError());
+    wf_advance_kernel<<<(n_ids + 255) / 256, 256, 0, st>>>(L, wf->d_st, wf->K);
+    CK(cudaGetLastError());
+    if (first_line) { if (int rc = wf->first.done(st)) return rc; }
+  }
   const unsigned long long threads = (unsigned long long)n_ids * 64;
   grab_update_kernel<<<(unsigned)((threads + GRAB_THREADS - 1) / GRAB_THREADS), GRAB_THREADS, 0, st>>>(L);
   CK(cudaGetLastError());
   if (channel_ids) { if (int rc = h->ids.done(st)) return rc; }
-  for (uint32_t i = 0; i < n_ids; i++) { /* the host mirror of what the kernel does to phase and valid */
+  for (uint32_t i = 0; i < n_ids; i++) { /* the host mirror of what the kernels do to phase, valid and the waterfall's words */
     const uint32_t c = channel_ids ? channel_ids[i] : i;
     const bool completed = h->phase[c] + n_blocks >= 2; /* some block of this call completes a pair */
-    if (counts) counts[i] = (h->phase[c] + n_blocks) / 2;
+    const uint32_t slots = (h->phase[c] + n_blocks) / 2;
+    if (wf) {
+      const uint32_t T = wf->held[c] + slots;
+      if (counts) counts[i] = T / wf->K;
+      wf->held[c] = T % wf->K;
+      wf->sel[c] ^= 1;
+    } else if (counts) {
+      counts[i] = slots;
+    }
     h->phase[c] = (uint8_t)((h->phase[c] + n_blocks) & 1);
     if (completed) { h->n_valid += !h->valid[c]; h->valid[c] = 1; h->fresh[c] = 1; }
   }
+  return 0;
+}
+
+extern "C" int sdr_grabber_process_device_snapshots(sdr_grabber_t *h, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I,
+                                                    const int16_t *Q, size_t pitch, uint32_t n_blocks, int16_t *snapshots, float *power,
+                                                    uint32_t *counts, void *cuda_stream) {
+  return grab_process(h, channel_ids, n_ids, I, Q, pitch, n_blocks, snapshots, power, counts, nullptr, nullptr, 0, nullptr, (cudaStream_t)cuda_stream);
+}
+
+extern "C" int sdr_grabber_process_device_waterfall_at(sdr_grabber_t *gr, sdr_waterfall_t *wf, const uint32_t *channel_ids, uint32_t n_ids,
+                                                       const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, float *lines,
+                                                       size_t line_pitch, const uint32_t *first_line, uint32_t *counts, void *cuda_stream) {
+  if (!wf) return fail(SDR_AUX_EINVAL, "null waterfall");
+  return grab_process(gr, channel_ids, n_ids, I, Q, pitch, n_blocks, nullptr, nullptr, counts, wf, lines, line_pitch, first_line,
+                      (cudaStream_t)cuda_stream);
+}
+
+extern "C" int sdr_grabber_process_device_waterfall(sdr_grabber_t *gr, sdr_waterfall_t *wf, const uint32_t *channel_ids, uint32_t n_ids,
+                                                    const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, float *lines,
+                                                    uint32_t *counts, void *cuda_stream) {
+  if (!wf || n_blocks == 0) return fail(SDR_AUX_EINVAL, "bad arguments");
+  return sdr_grabber_process_device_waterfall_at(gr, wf, channel_ids, n_ids, I, Q, pitch, n_blocks, lines, wf_lmax(wf->K, n_blocks), nullptr,
+                                                 counts, cuda_stream);
+}
+
+extern "C" int sdr_waterfall_create(sdr_waterfall_t **out, uint32_t n_channels, int device, uint32_t K) {
+  if (!out || n_channels == 0 || K == 0) return fail(SDR_AUX_EINVAL, "sdr_waterfall_create: bad arguments (n_channels >= 1, K >= 1)");
+  CK(cudaSetDevice(device));
+  if (int rc = upload_tables()) return rc;
+  sdr_waterfall *w = new sdr_waterfall();
+  w->n = n_channels; w->device = device; w->K = K;
+  w->held.assign(n_channels, 0); w->sel.assign(n_channels, 0);
+  int sms = 0, per_sm = 0;
+  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess ||
+      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, grab_waterfall_kernel, FFT_THREADS, 0) != cudaSuccess) {
+    delete w; return fail(SDR_AUX_ECUDA, "cannot query the device's multiprocessors");
+  }
+  w->ctas = std::max(1, sms * per_sm);
+  if (cudaMalloc(&w->acc, 2 * 1024 * (size_t)n_channels) != cudaSuccess || cudaMalloc(&w->d_st, 4 * (size_t)n_channels) != cudaSuccess) {
+    sdr_waterfall_destroy(w); return fail(SDR_AUX_ENOMEM, "cudaMalloc failed");
+  }
+  if (int rc = w->first.init(n_channels)) { sdr_waterfall_destroy(w); return rc; }
+  CK(cudaMemset(w->acc, 0, 2 * 1024 * (size_t)n_channels));
+  CK(cudaMemset(w->d_st, 0, 4 * (size_t)n_channels));
+  *out = w;
+  return 0;
+}
+
+extern "C" void sdr_waterfall_destroy(sdr_waterfall_t *w) {
+  if (!w) return;
+  cudaSetDevice(w->device);
+  cudaFree(w->acc); cudaFree(w->d_st);
+  w->first.release();
+  delete w;
+}
+
+extern "C" int sdr_waterfall_get_info(const sdr_waterfall_t *w, uint32_t *n_channels, int *device, uint32_t *K) {
+  if (!w || !n_channels || !device || !K) return fail(SDR_AUX_EINVAL, "get_info: bad arguments");
+  *n_channels = w->n; *device = w->device; *K = w->K;
   return 0;
 }
 
@@ -1250,6 +1452,54 @@ extern "C" int sdr_grabber_import_state(sdr_grabber_t *h, const uint32_t *channe
   }
   CK(cudaMemcpy(h->d_phase, h->phase.data(), h->n, cudaMemcpyHostToDevice));
   CK(cudaMemcpy(h->d_valid, h->valid.data(), h->n, cudaMemcpyHostToDevice));
+  return 0;
+}
+
+/* the waterfall's blob: K (a sum of pairs is a part of a line only for the same K), the pairs held and their sum */
+enum : uint32_t { BLOB_WF = 0x57465358u };
+struct WfBlob { uint32_t tag, version, K, held; float acc[256]; };
+
+extern "C" size_t sdr_waterfall_state_bytes(void) { return sizeof(WfBlob); }
+
+extern "C" int sdr_waterfall_export_state(sdr_waterfall_t *w, const uint32_t *channel_ids, uint32_t n, void *blobs) {
+  if (!w || !blobs) return fail(SDR_AUX_EINVAL, "export_state: bad arguments");
+  if (int rc = check_blob_ids(channel_ids, n, w->n)) return rc;
+  if (n == 0) return 0;
+  CK(cudaSetDevice(w->device));
+  CK(cudaDeviceSynchronize());
+  for (uint32_t i = 0; i < n; i++) {
+    const uint32_t c = channel_ids ? channel_ids[i] : i;
+    WfBlob b;
+    b.tag = BLOB_WF; b.version = BLOB_VERSION; b.K = w->K; b.held = w->held[c];
+    memset(b.acc, 0, sizeof b.acc); /* with no pair held the buffer is never read, and holds whatever sum it last received */
+    if (b.held) CK(cudaMemcpy(b.acc, w->acc + ((size_t)w->sel[c] * w->n + c) * 256, sizeof b.acc, cudaMemcpyDeviceToHost));
+    memcpy((char *)blobs + i * sizeof b, &b, sizeof b);
+  }
+  return 0;
+}
+
+extern "C" int sdr_waterfall_import_state(sdr_waterfall_t *w, const uint32_t *channel_ids, uint32_t n, const void *blobs) {
+  if (!w || !blobs) return fail(SDR_AUX_EINVAL, "import_state: bad arguments");
+  if (int rc = check_blob_ids(channel_ids, n, w->n)) return rc;
+  if (int rc = check_blobs<WfBlob>(blobs, n, BLOB_WF)) return rc;
+  for (uint32_t i = 0; i < n; i++) {
+    WfBlob b;
+    memcpy(&b, (const char *)blobs + i * sizeof b, sizeof b);
+    if (b.K != w->K || b.held >= w->K) return fail(SDR_AUX_EINVAL, "import_state: the blob is of a waterfall with another K");
+  }
+  if (n == 0) return 0;
+  CK(cudaSetDevice(w->device));
+  CK(cudaDeviceSynchronize());
+  for (uint32_t i = 0; i < n; i++) {
+    const uint32_t c = channel_ids ? channel_ids[i] : i;
+    WfBlob b;
+    memcpy(&b, (const char *)blobs + i * sizeof b, sizeof b);
+    CK(cudaMemcpy(w->acc + ((size_t)w->sel[c] * w->n + c) * 256, b.acc, sizeof b.acc, cudaMemcpyHostToDevice));
+    w->held[c] = b.held;
+  }
+  std::vector<uint32_t> st(w->n);
+  for (uint32_t c = 0; c < w->n; c++) st[c] = w->held[c] << 1 | w->sel[c];
+  CK(cudaMemcpy(w->d_st, st.data(), 4 * (size_t)w->n, cudaMemcpyHostToDevice));
   return 0;
 }
 

@@ -70,6 +70,9 @@ struct sdr_graph {
   uint64_t calls;   /* calls queued since create (= the latest ticket) */
   std::vector<uint8_t> mark;
   std::vector<uint32_t> counts, chunk_counts;
+  sdr_waterfall_t *wf; /* attached waterfall or NULL */
+  Buf wf_lines[2];     /* a whole call's lines [rows][Lmax][256], by call parity */
+  std::vector<uint32_t> line_first; /* per row: lines of the call so far = the next chunk's first slot */
 };
 
 static int check_ids(sdr_graph *g, const uint32_t *ids, uint32_t n_ids) {
@@ -100,7 +103,7 @@ extern "C" void sdr_graph_destroy(sdr_graph_t *g) {
     for (cudaEvent_t e : {g->ev_h2d[k], g->ev_comp[k], g->ev_d2h[k]}) if (e) cudaEventDestroy(e);
   }
   for (cudaEvent_t e : g->ev_call) if (e) cudaEventDestroy(e);
-  g->mid_i.release(); g->mid_q.release();
+  g->mid_i.release(); g->mid_q.release(); g->wf_lines[0].release(); g->wf_lines[1].release();
   for (cudaStream_t s : {g->s_h2d, g->s_comp, g->s_d2h}) if (s) cudaStreamDestroy(s);
   delete g;
 }
@@ -129,6 +132,7 @@ extern "C" int sdr_graph_create(sdr_graph_t **out, const sdr_graph_desc *desc) {
   for (int k = 0; k < 2; k++) g->ev_h2d[k] = g->ev_comp[k] = g->ev_d2h[k] = nullptr;
   for (auto &e : g->ev_call) e = nullptr;
   g->seq = g->calls = 0;
+  g->wf = nullptr;
   g->mark.assign(g->n_ch, 0);
   int rc = 0;
   auto stream = [&](cudaStream_t *s) { if (!rc && cudaStreamCreateWithFlags(s, cudaStreamNonBlocking) != cudaSuccess) rc = fail(SDR_ERR_CUDA, "cudaStreamCreate failed"); };
@@ -175,10 +179,35 @@ static uint32_t chunk_blocks(const sdr_graph *g, uint32_t n_blocks, bool streame
   return c < n_blocks ? c : n_blocks;
 }
 
+extern "C" int sdr_graph_attach_waterfall(sdr_graph_t *g, sdr_waterfall_t *wf) {
+  if (!g) return fail(SDR_ERR_ARG, "attach_waterfall: bad arguments");
+  if (wf) {
+    if (!g->d.grabber) return fail(SDR_ERR_ARG, "attach_waterfall: the graph has no grabber");
+    uint32_t n = 0, K = 0; int dev = 0;
+    if (int rc = from_aux(sdr_waterfall_get_info(wf, &n, &dev, &K), "waterfall")) return rc;
+    if (n != g->n_ch || dev != g->device) return fail(SDR_ERR_ARG, "attach_waterfall: the waterfall must have the graph's device and channel count");
+  }
+  CU(cudaSetDevice(g->device));
+  if (int rc = drain(g)) return rc; /* calls in flight use the waterfall attached before */
+  g->wf = wf;
+  return SDR_OK;
+}
+
 static int graph_call(sdr_graph *g, const uint32_t *ids, uint32_t n_ids, const int16_t *I, const int16_t *Q, size_t in_pitch,
-                      void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o, bool streamed) {
+                      void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o, bool streamed,
+                      bool with_lines, float *lines, uint32_t *line_counts) {
   /* ---- every argument, before anything is queued */
   if (!g || !I || !audio) return fail(SDR_ERR_ARG, "submit_host: bad arguments");
+  if (with_lines != (g->wf != nullptr))
+    return fail(SDR_ERR_ARG, g->wf ? "a graph with a waterfall takes the _waterfall calls" : "the _waterfall calls need an attached waterfall");
+  uint32_t K = 1, Lmax = 0;
+  if (g->wf) {
+    uint32_t n = 0; int dev = 0;
+    if (int rc = from_aux(sdr_waterfall_get_info(g->wf, &n, &dev, &K), "waterfall")) return rc;
+    if (!lines || ((uintptr_t)lines & 15)) return fail(SDR_ERR_ARG, "lines must be non-NULL and 16-byte aligned");
+    if (o && (o->power || o->snapshots || o->counts)) return fail(SDR_ERR_ARG, "power, snapshots and counts are not available with a waterfall");
+    if (n_blocks) Lmax = (uint32_t)(((unsigned long long)K - 1 + (n_blocks + 1) / 2) / K);
+  }
   if (int rc = check_ids(g, ids, n_ids)) return rc;
   if (n_blocks == 0) return fail(SDR_ERR_ARG, "n_blocks == 0");
   if (n_blocks > (1u << 24)) return fail(SDR_ERR_ARG, "n_blocks too large (at most 2^24 blocks per call)");
@@ -202,8 +231,8 @@ static int graph_call(sdr_graph *g, const uint32_t *ids, uint32_t n_ids, const i
   const size_t need[7] = {cs * 2 * rows, Q ? cs * 2 * rows : 0, cs * oes * rows, out.rx_status ? (size_t)chunk * SDR_BS_FIELDS * rows * 4 : 0,
                           out.pp_status ? (size_t)chunk * SDR_PP_BS_FIELDS * rows * 4 : 0, out.power ? cslots * 1024 * rows : 0,
                           out.snapshots ? cslots * 1024 * rows : 0};
-  const size_t mid = g->d.pp || g->d.gen ? cs * 2 * rows : 0;
-  bool grow = mid > g->mid_i.cap;
+  const size_t mid = g->d.pp || g->d.gen ? cs * 2 * rows : 0, lines_bytes = g->wf ? (size_t)(Lmax ? Lmax : 1) * 1024 * rows : 0;
+  bool grow = mid > g->mid_i.cap || lines_bytes > g->wf_lines[0].cap;
   for (int k = 0; k < 2; k++) {
     const Buf *b[7] = {&g->in_a[k], &g->in_b[k], &g->audio[k], &g->rx_rec[k], &g->pp_rec[k], &g->power[k], &g->snaps[k]};
     for (int j = 0; j < 7; j++) grow |= need[j] > b[j]->cap;
@@ -216,6 +245,7 @@ static int graph_call(sdr_graph *g, const uint32_t *ids, uint32_t n_ids, const i
     }
     if (int rc = g->mid_i.ensure(mid)) return rc;
     if (int rc = g->mid_q.ensure(mid)) return rc;
+    for (Buf &b : g->wf_lines) if (int rc = b.ensure(lines_bytes)) return rc;
   }
 
   /* ---- the chunks */
@@ -224,7 +254,23 @@ static int graph_call(sdr_graph *g, const uint32_t *ids, uint32_t n_ids, const i
   int err = 0;
 #define GR_TRY(expr) if ((err = (expr)) != 0) break
 #define GR_CU(call) if ((call) != cudaSuccess) { err = fail(SDR_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(cudaGetLastError())); break; }
-  for (uint32_t done = 0; done < n_blocks;) {
+  /* Waterfall: each chunk's grabber call puts row r's lines at slot line_first[r] of the call's device buffer wl, where the
+   * uncut call would put them.  After a chunk every row has completed the slots below the least line_first, and no later
+   * chunk writes them: they come down in one copy.  A row's final count is at least Lmax - 1 (rows differ in their held
+   * pairs, < K, and by at most one pair of their phase), so only slot Lmax - 1 may be left unwritten by some rows: it is
+   * loaded with the caller's lines first, and the last chunk copies it down whole. */
+  float *wl = g->wf ? (float *)g->wf_lines[(g->calls + 1) & 1].p : nullptr;
+  const size_t lp = (size_t)Lmax * 1024; /* bytes per row of wl and of the caller's lines */
+  uint32_t copied = 0;
+  if (g->wf) {
+    g->line_first.assign(rows, 0);
+    do {
+      /* wl was last read by the final copy of the call two before this one */
+      if (g->calls >= 2) GR_CU(cudaStreamWaitEvent(g->s_h2d, g->ev_call[(g->calls - 1) % GRAPH_TICKETS], 0));
+      if (Lmax) GR_CU(cudaMemcpy2DAsync(wl + (size_t)(Lmax - 1) * 256, lp, lines + (size_t)(Lmax - 1) * 256, lp, 1024, rows, cudaMemcpyHostToDevice, g->s_h2d));
+    } while (0);
+  }
+  for (uint32_t done = 0; done < n_blocks && !err;) {
     const uint32_t nb = n_blocks - done < chunk ? n_blocks - done : chunk;
     const size_t w = (size_t)nb * 128;
     const int b = (int)(g->seq & 1);
@@ -247,7 +293,10 @@ static int graph_call(sdr_graph *g, const uint32_t *ids, uint32_t n_ids, const i
                       "I/Q generator"));
       ri = (const int16_t *)g->mid_i.p; rq = (const int16_t *)g->mid_q.p;
     }
-    if (g->d.grabber) {
+    if (g->wf) {
+      GR_TRY(from_aux(sdr_grabber_process_device_waterfall_at(g->d.grabber, g->wf, ids, n_ids, ri, rq, cs, nb, wl, Lmax, g->line_first.data(),
+                                                              g->chunk_counts.data(), g->s_comp), "grabber"));
+    } else if (g->d.grabber) {
       GR_TRY(from_aux(sdr_grabber_process_device_snapshots(g->d.grabber, ids, n_ids, ri, rq, cs, nb, out.snapshots ? (int16_t *)g->snaps[b].p : nullptr,
                                                            out.power ? (float *)g->power[b].p : nullptr, g->chunk_counts.data(), g->s_comp),
                       "grabber"));
@@ -267,7 +316,14 @@ static int graph_call(sdr_graph *g, const uint32_t *ids, uint32_t n_ids, const i
       const size_t rec = (size_t)SDR_PP_BS_FIELDS * rows * 4;
       GR_CU(cudaMemcpyAsync((char *)out.pp_status + (size_t)done * rec, g->pp_rec[b].p, nb * rec, cudaMemcpyDeviceToHost, g->s_d2h));
     }
-    if (g->d.grabber) {
+    if (g->wf) {
+      uint32_t lo = UINT32_MAX;
+      for (uint32_t r = 0; r < rows; r++) { g->line_first[r] += g->chunk_counts[r]; lo = g->line_first[r] < lo ? g->line_first[r] : lo; }
+      const uint32_t hi = done + nb == n_blocks ? Lmax : lo;
+      if (hi > copied)
+        GR_CU(cudaMemcpy2DAsync(lines + (size_t)copied * 256, lp, wl + (size_t)copied * 256, lp, (size_t)(hi - copied) * 1024, rows, cudaMemcpyDeviceToHost, g->s_d2h));
+      copied = hi;
+    } else if (g->d.grabber) {
       /* rows in runs of equal slot counts: a row writes (phase + nb) / 2 slots of the chunk, and the slot a row does not
        * write (an odd last chunk and phase 0) must keep what the caller's buffer holds */
       for (uint32_t r0 = 0; r0 < rows && !err;) {
@@ -298,6 +354,7 @@ static int graph_call(sdr_graph *g, const uint32_t *ids, uint32_t n_ids, const i
    * the call */
   if (err) { drain(g); return err; }
   if (out.counts) memcpy(out.counts, g->counts.data(), 4 * (size_t)rows);
+  if (line_counts) memcpy(line_counts, g->line_first.data(), 4 * (size_t)rows);
   /* the call's ticket: its last copy-out is the last thing in the D2H stream */
   g->calls++;
   CU(cudaEventRecord(g->ev_call[g->calls % GRAPH_TICKETS], g->s_d2h));
@@ -306,12 +363,25 @@ static int graph_call(sdr_graph *g, const uint32_t *ids, uint32_t n_ids, const i
 
 extern "C" int sdr_graph_submit_host(sdr_graph_t *g, const uint32_t *ids, uint32_t n_ids, const int16_t *I_or_X, const int16_t *Q, size_t in_pitch,
                                      void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o) {
-  return graph_call(g, ids, n_ids, I_or_X, Q, in_pitch, audio, out_pitch, out_fmt, n_blocks, o, true);
+  return graph_call(g, ids, n_ids, I_or_X, Q, in_pitch, audio, out_pitch, out_fmt, n_blocks, o, true, false, nullptr, nullptr);
 }
 
 extern "C" int sdr_graph_process_host(sdr_graph_t *g, const uint32_t *ids, uint32_t n_ids, const int16_t *I_or_X, const int16_t *Q, size_t in_pitch,
                                       void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o) {
-  if (int rc = graph_call(g, ids, n_ids, I_or_X, Q, in_pitch, audio, out_pitch, out_fmt, n_blocks, o, false)) return rc;
+  if (int rc = graph_call(g, ids, n_ids, I_or_X, Q, in_pitch, audio, out_pitch, out_fmt, n_blocks, o, false, false, nullptr, nullptr)) return rc;
+  return sdr_graph_wait_host_ticket(g, g->calls);
+}
+
+extern "C" int sdr_graph_submit_host_waterfall(sdr_graph_t *g, const uint32_t *ids, uint32_t n_ids, const int16_t *I_or_X, const int16_t *Q,
+                                               size_t in_pitch, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks,
+                                               const sdr_graph_outputs *o, float *lines, uint32_t *line_counts) {
+  return graph_call(g, ids, n_ids, I_or_X, Q, in_pitch, audio, out_pitch, out_fmt, n_blocks, o, true, true, lines, line_counts);
+}
+
+extern "C" int sdr_graph_process_host_waterfall(sdr_graph_t *g, const uint32_t *ids, uint32_t n_ids, const int16_t *I_or_X, const int16_t *Q,
+                                                size_t in_pitch, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks,
+                                                const sdr_graph_outputs *o, float *lines, uint32_t *line_counts) {
+  if (int rc = graph_call(g, ids, n_ids, I_or_X, Q, in_pitch, audio, out_pitch, out_fmt, n_blocks, o, false, true, lines, line_counts)) return rc;
   return sdr_graph_wait_host_ticket(g, g->calls);
 }
 

@@ -148,6 +148,37 @@ class IQGeneratorBatch {
   sdr_iqgen_t *h_;
 };
 
+/* averaged waterfall lines per channel, K pairs per line (sdr_waterfall_*); driven through GrabberBatch::process */
+class WaterfallBatch {
+ public:
+  WaterfallBatch(uint32_t n_channels, uint32_t K, int device = 0) : h_(nullptr), K_(K) {
+    check(sdr_waterfall_create(&h_, n_channels, device, K), "sdr_waterfall_create");
+  }
+  ~WaterfallBatch() { sdr_waterfall_destroy(h_); }
+  WaterfallBatch(const WaterfallBatch &) = delete;
+  WaterfallBatch &operator=(const WaterfallBatch &) = delete;
+  /* Lmax: line slots per row of a call of n_blocks blocks */
+  uint32_t line_slots(uint32_t n_blocks) const { return (uint32_t)(((uint64_t)K_ - 1 + (n_blocks + 1) / 2) / K_); }
+  static size_t state_bytes() { return sdr_waterfall_state_bytes(); }
+  std::vector<uint8_t> export_state(const std::vector<uint32_t> &ids) {
+    std::vector<uint8_t> b(ids.size() * state_bytes());
+    check(sdr_waterfall_export_state(h_, ids.data(), (uint32_t)ids.size(), b.data()), "sdr_waterfall_export_state");
+    return b;
+  }
+  void import_state(const std::vector<uint32_t> &ids, const std::vector<uint8_t> &blobs) {
+    if (blobs.size() != ids.size() * state_bytes()) throw std::runtime_error("import_state: one blob per channel");
+    check(sdr_waterfall_import_state(h_, ids.data(), (uint32_t)ids.size(), blobs.data()), "sdr_waterfall_import_state");
+  }
+  sdr_waterfall_t *handle() { return h_; }
+
+ private:
+  static void check(int rc, const char *what) {
+    if (rc != SDR_AUX_OK) throw std::runtime_error(std::string(what) + ": " + sdr_aux_last_error());
+  }
+  sdr_waterfall_t *h_;
+  uint32_t K_;
+};
+
 /* AudioGrabberComplex256 (AudioGrabberComplex256.h:46-64) for n channels */
 class GrabberBatch {
  public:
@@ -176,6 +207,15 @@ class GrabberBatch {
                float *power, uint32_t *counts, void *cuda_stream = nullptr) {
     check(sdr_grabber_process_device_snapshots(h_, ids.data(), (uint32_t)ids.size(), I, Q, pitch, n_blocks, snapshots, power, counts, cuda_stream),
           "sdr_grabber_process_device_snapshots");
+  }
+  /* ... advancing the waterfall wf and writing the lines the call completes (device [rows][wf.line_slots(n_blocks)][256]
+   * float) and the lines per row (host, rows entries, may be null); sdr_grabber_process_device_waterfall.  ids empty:
+   * every channel */
+  void process(WaterfallBatch &wf, const std::vector<uint32_t> &ids, const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks,
+               float *lines, uint32_t *counts, void *cuda_stream = nullptr) {
+    check(sdr_grabber_process_device_waterfall(h_, wf.handle(), ids.empty() ? nullptr : ids.data(), ids.empty() ? n_channels_ : (uint32_t)ids.size(),
+                                               I, Q, pitch, n_blocks, lines, counts, cuda_stream),
+          "sdr_grabber_process_device_waterfall");
   }
   static size_t state_bytes() { return sdr_grabber_state_bytes(); }
   std::vector<uint8_t> export_state(const std::vector<uint32_t> &ids) {

@@ -55,6 +55,22 @@ class SdrGraph {
     check(sdr_graph_process_host(g_, ids.data(), (uint32_t)ids.size(), I_or_X, Q, in_pitch, audio, out_pitch, out_fmt, n_blocks, o),
           "sdr_graph_process_host");
   }
+  /* waterfall lines from the grabber tap (sdr_graph_attach_waterfall); the calls are then the _waterfall ones below */
+  void attach_waterfall(WaterfallBatch *wf) { check(sdr_graph_attach_waterfall(g_, wf ? wf->handle() : nullptr), "sdr_graph_attach_waterfall"); }
+  /* host lines [rows][wf.line_slots(n_blocks)][256] float, line_counts [rows] (may be null); ids empty: every channel */
+  uint64_t submit_host(const std::vector<uint32_t> &ids, const int16_t *I_or_X, const int16_t *Q, size_t in_pitch, void *audio, size_t out_pitch,
+                       int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o, float *lines, uint32_t *line_counts) {
+    check(sdr_graph_submit_host_waterfall(g_, ids.empty() ? nullptr : ids.data(), ids.empty() ? n_ : (uint32_t)ids.size(), I_or_X, Q, in_pitch, audio,
+                                          out_pitch, out_fmt, n_blocks, o, lines, line_counts),
+          "sdr_graph_submit_host_waterfall");
+    return sdr_graph_host_ticket(g_);
+  }
+  void process_host(const std::vector<uint32_t> &ids, const int16_t *I_or_X, const int16_t *Q, size_t in_pitch, void *audio, size_t out_pitch,
+                    int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o, float *lines, uint32_t *line_counts) {
+    check(sdr_graph_process_host_waterfall(g_, ids.empty() ? nullptr : ids.data(), ids.empty() ? n_ : (uint32_t)ids.size(), I_or_X, Q, in_pitch, audio,
+                                           out_pitch, out_fmt, n_blocks, o, lines, line_counts),
+          "sdr_graph_process_host_waterfall");
+  }
   void wait_host() { check(sdr_graph_wait_host(g_), "sdr_graph_wait_host"); }
   void wait_host(uint64_t ticket) { check(sdr_graph_wait_host_ticket(g_, ticket), "sdr_graph_wait_host_ticket"); }
   sdr_graph_t *handle() { return g_; }

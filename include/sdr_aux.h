@@ -189,6 +189,41 @@ int sdr_grabber_import_state(sdr_grabber_t *h, const uint32_t *channel_ids, uint
 int sdr_grabber_spectrum(sdr_grabber_t *h, const uint32_t *channels, uint32_t n, float *power);
 int sdr_grabber_spectrum_device(sdr_grabber_t *h, const uint32_t *d_channels, uint32_t n, float *d_power, void *cuda_stream);
 
+/* ---------------------------------------------------------------- waterfall ---- */
+/* Averaged waterfall lines per channel: the grabber's per-pair power spectra (sdr_grabber_process_device_snapshots' `power`,
+ * bit for bit) averaged K at a time, in pair order, across calls.  Number the pairs a channel's grabber completes 0, 1, 2, ...
+ * since the waterfall was created (or since the channel's blob was imported); line m of the channel is, per bin,
+ *     acc = 0.0f;  for j in mK .. mK+K-1:  acc = acc + P_j     (float32, one rounding per add, in j order)
+ *     line_m = acc / (float)K                                  (one IEEE division)
+ * so with K == 1 the lines are the spectra themselves.  A channel's lines do not depend on how its blocks are cut into calls
+ * or subsets, nor on a migration through export_state / import_state.  The waterfall holds each channel's partial sum (the
+ * pairs held, < K) between calls; it is driven only through the grabber calls below. */
+typedef struct sdr_waterfall sdr_waterfall_t;
+
+int sdr_waterfall_create(sdr_waterfall_t **out, uint32_t n_channels, int device, uint32_t K); /* K >= 1 */
+void sdr_waterfall_destroy(sdr_waterfall_t *w);
+int sdr_waterfall_get_info(const sdr_waterfall_t *w, uint32_t *n_channels, int *device, uint32_t *K);
+/* Blob: K, the pairs held and their partial sum (256 floats).  Imports only into a waterfall with the same K. */
+size_t sdr_waterfall_state_bytes(void);
+int sdr_waterfall_export_state(sdr_waterfall_t *w, const uint32_t *channel_ids, uint32_t n, void *blobs);
+int sdr_waterfall_import_state(sdr_waterfall_t *w, const uint32_t *channel_ids, uint32_t n, const void *blobs);
+/* sdr_grabber_process_device_subset on the listed channels (same ids, planes, checks and resulting grabber state), also
+ * advancing the waterfall `wf` (same device and channel count as the grabber, else SDR_AUX_EINVAL) over the pairs it completes.
+ *   Lmax = (K - 1 + (n_blocks + 1) / 2) / K line slots per row.
+ *   lines   device, float [n_ids][Lmax][256], 16-byte aligned: row i's counts[i] lines completed by this call, oldest first,
+ *           natural bin order.  Slots past counts[i] are not written.
+ *   counts  host, uint32 [n_ids] or NULL: filled before the call returns, without synchronising.
+ * A bad argument queues nothing: no state changes, nothing is written. */
+int sdr_grabber_process_device_waterfall(sdr_grabber_t *gr, sdr_waterfall_t *wf, const uint32_t *channel_ids, uint32_t n_ids, const int16_t *I,
+                                         const int16_t *Q, size_t pitch, uint32_t n_blocks, float *lines, uint32_t *counts, void *cuda_stream);
+/* The same with row i's lines at slots first_line[i] .. first_line[i] + counts[i] - 1 of a row of line_pitch slots:
+ * lines[((size_t)i * line_pitch + first_line[i] + m) * 256 + bin].  first_line: host, uint32 [n_ids] or NULL (zeros); a row
+ * whose lines would run past line_pitch is SDR_AUX_EINVAL.  Lets a caller that cuts one call into several (sdr_graph.h)
+ * gather each row's lines where the uncut call would have put them. */
+int sdr_grabber_process_device_waterfall_at(sdr_grabber_t *gr, sdr_waterfall_t *wf, const uint32_t *channel_ids, uint32_t n_ids,
+                                            const int16_t *I, const int16_t *Q, size_t pitch, uint32_t n_blocks, float *lines,
+                                            size_t line_pitch, const uint32_t *first_line, uint32_t *counts, void *cuda_stream);
+
 /* The channel count and device a handle was created with (for code that drives handles it did not create, e.g. sdr_graph.h) */
 int sdr_preproc_get_info(const sdr_preproc_t *h, uint32_t *n_channels, int *device);
 int sdr_iqgen_get_info(const sdr_iqgen_t *h, uint32_t *n_channels, int *device);

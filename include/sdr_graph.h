@@ -79,6 +79,22 @@ int sdr_graph_submit_host(sdr_graph_t *g, const uint32_t *ids, uint32_t n_ids, c
                           size_t in_pitch, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o);
 int sdr_graph_process_host(sdr_graph_t *g, const uint32_t *ids, uint32_t n_ids, const int16_t *I_or_X, const int16_t *Q,
                            size_t in_pitch, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o);
+/* Waterfall lines from the grabber tap (sdr_waterfall_*, sdr_aux.h).  attach_waterfall gives a graph with a grabber a
+ * waterfall handle on the same device with the same channel count (NULL detaches it; not while calls are in flight that
+ * use it: attach waits for them).  While one is attached, the graph's calls are the _waterfall forms, which equal, bit for
+ * bit, one sdr_grabber_process_device_waterfall over the whole call in place of the grabber's device call:
+ *   lines        host, float [n_ids][Lmax][256], 16-byte aligned, Lmax = (K - 1 + (n_blocks + 1) / 2) / K: row i's lines of
+ *                the call in slots 0 .. line_counts[i] - 1; later slots keep what they held.
+ *   line_counts  host, uint32 [n_ids] or NULL, filled before submit returns.
+ * The lines are gathered on the device and each chunk's completed line slots come down in one copy.  o->power, o->snapshots
+ * and o->counts are not available with a waterfall (SDR_ERR_ARG); the plain calls are SDR_ERR_ARG while one is attached. */
+int sdr_graph_attach_waterfall(sdr_graph_t *g, sdr_waterfall_t *wf);
+int sdr_graph_submit_host_waterfall(sdr_graph_t *g, const uint32_t *ids, uint32_t n_ids, const int16_t *I_or_X, const int16_t *Q,
+                                    size_t in_pitch, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o,
+                                    float *lines, uint32_t *line_counts);
+int sdr_graph_process_host_waterfall(sdr_graph_t *g, const uint32_t *ids, uint32_t n_ids, const int16_t *I_or_X, const int16_t *Q,
+                                     size_t in_pitch, void *audio, size_t out_pitch, int out_fmt, uint32_t n_blocks, const sdr_graph_outputs *o,
+                                     float *lines, uint32_t *line_counts);
 /* The latest call's ticket (1, 2, ...; 0 before the first).  Calls complete in order. */
 uint64_t sdr_graph_host_ticket(const sdr_graph_t *g);
 /* Returns when everything submitted so far has landed / when call `ticket` has landed (later calls stay in flight). */
